@@ -2,6 +2,7 @@
 """bench.py -- headline measurement of the plane-sweep hot path (contract: see the task brief / DESIGN.md §5).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|cfg1|cfg4] [--no-graph]
+                    [--dump-outputs DIR]
 
 Own arm: one "step" = one MVSNet train step (forward + loss + backward + gradient all-reduce + Adam) on one synthetic
 DTU-shaped batch (BASELINE.json configs[1]: bf16, batch 4, 3 views, 640x512 input => 160x128x32 features, D = 192), replayed as
@@ -183,6 +184,22 @@ def _pin_rank_to_cores(local_rank, local_world):
         return os.cpu_count() or 1
 
 
+def dump_outputs(out_dir, last, params):
+    """What the last timed step handed its caller, as float32 DIR/<name>.npy: the loss, the initial and refined depth maps and,
+    for a train step, the gradients (every parameter's, flattened and concatenated in model.parameters() order); at most a few
+    MB at every workload.  The weights after the optimiser step are not written: Adam's first step moves each weight by about
+    lr * sign(gradient), so float noise in a gradient near zero moves a weight by up to 2 lr."""
+    import numpy as np
+    import torch
+    loss, initial, refined = last
+    arrays = {"loss": loss.reshape(1), "initial_depth": initial, "refined_depth": refined}
+    if params is not None:
+        arrays["grads"] = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_b200(args, rank, world, local_rank, workload=None, light=False):
     """One workload on this rank.  light: an extra measurement riding on the default line (no per-kernel event pass, no clocks,
     no isolated K1 launches, fewer steps)."""
@@ -236,6 +253,20 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
             dist.broadcast(t.data, 0)
         slab = DepthSlabMVSNet(model, graph=not args.no_graph)
 
+    # --dump-outputs: the seeded starting state of the training run, restored before the last timed step.  The float atomics of
+    # the kernels make every step differ from run to run in the last bits, and the steps before would carry that into the
+    # weights; from this state the last step's outputs are the same in every run up to that last-bit noise.
+    start = [t.detach().clone() for t in params + list(model.buffers())] if args.dump_outputs and train and not light else None
+
+    def restart():
+        with torch.no_grad():
+            for t, s in zip(params + list(model.buffers()), start):
+                t.copy_(s)
+            for st in opt.state.values():                 # in place: a captured graph holds these tensors
+                for v in st.values():
+                    if torch.is_tensor(v):
+                        v.zero_()
+
     gstep = ginf = None
     if graphed:
         from mvs_b200.harness import GraphedTrainStep
@@ -245,11 +276,12 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
         ginf = GraphedInference(model, B, V, H, W, dev)
 
     def step(img, gt):
+        """-> (loss, initial depth map, refined depth map) of this step."""
         if gstep is not None:                              # forward + loss + backward + all-reduce + Adam: one CUDA graph
-            return gstep.run(img, gt, K, R, T, d_min, d_int)
+            return (gstep.run(img, gt, K, R, T, d_min, d_int), *gstep.depth)
         if slab is not None:
             initial, refined = slab.forward(img, K, R, T, d_min, d_int, V)
-            return loss_fcn(gt, initial, refined)[0]
+            return loss_fcn(gt, initial, refined)[0], initial, refined
         if train:
             if reducer is not None and reducer.attached:
                 reducer.bucket.zero_()
@@ -261,13 +293,13 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
             if reducer:
                 reducer.reduce()
             opt.step()
-            return loss.detach()
+            return loss.detach(), initial.detach(), refined.detach()
         with torch.no_grad():
             if ginf is not None:                           # inference forward replayed as one CUDA graph
                 initial, refined = ginf.run(img, K, R, T, d_min, d_int)
             else:
                 initial, refined = model(img, K, R, T, d_min, d_int, B, V)
-            return loss_fcn(gt, initial, refined)[0]
+            return loss_fcn(gt, initial, refined)[0], initial, refined
 
     def step_resident():
         return step(img_dev, gt_dev)
@@ -308,7 +340,7 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
             prefetch(cur)
             feed["primed"] = True
         torch.cuda.current_stream().wait_event(ready[cur])
-        loss = step(stage[cur][0], stage[cur][1])
+        loss = step(stage[cur][0], stage[cur][1])[0]
         consumed[cur].record()
         # the next step's 47 MB H2D copy is issued AFTER this step's launches: the step's own small H2D copies (sweep geometry,
         # on the compute stream) share the host-to-device copy engine with it and would otherwise queue behind it -- the whole
@@ -329,13 +361,14 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
         return loss_host
 
     def timed(fn, n):
+        """-> (ms for n calls of fn, what the last call returned)"""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(n):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize()
         if world > 1:
@@ -343,7 +376,7 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     graph_note = None
     if gstep is not None:
@@ -366,7 +399,15 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
     if gstep is None and ginf is None and not light:
         ops.EVENTS = {}
     n0 = mvs_b200.launch_count()
-    ms = timed(step_resident, steps)
+    if start is None:
+        ms, last = timed(step_resident, steps)
+    else:                                                  # two timed windows; the restart between them is not timed
+        ms = timed(step_resident, steps - 1)[0] if steps > 1 else 0.0
+        restart()
+        ms_last, last = timed(step_resident, 1)
+        ms += ms_last
+    if args.dump_outputs and rank == 0 and not light:
+        dump_outputs(args.dump_outputs, last, params if train else None)
     launches = ((gstep.launches * steps) if gstep is not None else
                 (ginf.launches * steps) if ginf is not None else
                 (slab.launches * steps) if slab is not None and getattr(slab, "launches", 0) else mvs_b200.launch_count() - n0)
@@ -374,7 +415,7 @@ def run_b200(args, rank, world, local_rank, workload=None, light=False):
     clocks = sampler.stop() if (rank == 0 and not light) else None
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, steps)
+    ms_e2e, _ = timed(step_e2e, steps)
     maps = B * (1 if slab is not None else world) * steps
     value, e2e_value = maps / (ms * 1e-3), maps / (ms_e2e * 1e-3)
 
@@ -614,7 +655,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg4 depth-slab / cfg3 measurements riding on the default line")
     ap.add_argument("--no-graph", action="store_true", help="issue the train step eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (loss, depth maps, gradients) as DIR/<name>.npy; a train "
+                         "step's last timed step then starts from the seeded initial weights")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
 

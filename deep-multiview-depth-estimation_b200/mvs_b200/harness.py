@@ -138,7 +138,7 @@ class GraphedTrainStep:
         self.d_int = torch.ones(batch_size, 1, 1, 1, device=device)
         self.sweep = None
         self.dims = (h, w)
-        self.graph, self.loss, self.launches = None, None, 0
+        self.graph, self.loss, self.depth, self.launches = None, None, None, 0
         self.warmup, self._lib = warmup, _lib
         self.params = [p for p in model.parameters() if p.requires_grad]
         self.reducer, self.optimizer = reducer, optimizer
@@ -183,7 +183,7 @@ class GraphedTrainStep:
             self.reducer.reduce_attached()                 # all-reduce + average of the flat bucket, in place
         if self.optimizer is not None:
             self.optimizer.step()
-        return loss.detach()
+        return loss.detach(), (initial.detach(), refined.detach())
 
     def _optimizer_state_tensors(self):
         out = []
@@ -193,7 +193,8 @@ class GraphedTrainStep:
         return out
 
     def run(self, img, gt, K, R, T, d_min, d_int):
-        """-> loss (device scalar, valid after the current stream reaches this point); gradients in .grad."""
+        """-> loss (device scalar, valid after the current stream reaches this point); gradients in .grad, the step's
+        (initial, refined) depth maps in .depth."""
         self._load(img, gt, K, R, T, d_min, d_int)
         if self.graph is None:
             buffers = list(self.model.buffers())
@@ -221,7 +222,7 @@ class GraphedTrainStep:
             n0 = self._lib.launch_count()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                self.loss = self._fwd_bwd()
+                self.loss, self.depth = self._fwd_bwd()
             self.launches = self._lib.launch_count() - n0   # libmvs_b200.so launches recorded in the graph
             self.graph = g
         self.graph.replay()
@@ -229,7 +230,7 @@ class GraphedTrainStep:
 
     def release(self):
         """Drop the captured graph (with a reducer it holds NCCL work: do this before destroy_process_group())."""
-        self.graph, self.loss = None, None
+        self.graph, self.loss, self.depth = None, None, None
         torch.cuda.synchronize()
 
 

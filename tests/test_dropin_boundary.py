@@ -2,7 +2,6 @@
 names and signatures (scripts/homography.py:6-14, costvolume.py:3, depthmap.py:4) and read the host application's `config`
 at call time, as `model.py:5-7` expects.  CPU: names, signatures, refusal to run without CUDA.  GPU: the call sequence of
 MVSNet.forward (model.py:177-187) through the drop-in modules on the golden inputs of the unmodified reference."""
-import ast
 import importlib
 import inspect
 import os
@@ -15,7 +14,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DROPIN = os.path.join(ROOT, "deep-multiview-depth-estimation_b200", "dropin")
-REFERENCE = {   # as written in the reference (SURVEY §8b); re-read from /root/reference when it is present (this container only)
+REFERENCE = {   # as written in the reference (SURVEY §8b)
     "homography": ("homography_warping", ["K_batch", "R_batch", "T_batch", "d_min", "d_int", "feature_maps", "batch_size",
                                           "n_views", "d_num"]),
     "costvolume": ("assemble_cost_volume", ["warped_feature_maps", "n_views"]),
@@ -44,11 +43,6 @@ def test_names_and_signatures_match_the_reference():
     for mod, (fn, params) in REFERENCE.items():
         f = getattr(mods[mod], fn)
         assert list(inspect.signature(f).parameters) == params, (mod, fn)
-        ref_py = os.path.join("/root/reference/scripts", mod + ".py")
-        if os.path.exists(ref_py):                  # the real thing, when the reference tree is mounted
-            tree = ast.parse(open(ref_py).read())
-            node = next(n for n in tree.body if isinstance(n, ast.FunctionDef) and n.name == fn)
-            assert [a.arg for a in node.args.args] == params
     import mvs_b200
     sd = mvs_b200.CostVolumeReg(device="cpu").state_dict()
     assert {"conv_0_0.weight", "deconv_3_0.weight", "conv_out.weight", "BN_3.running_var", "BN_0.num_batches_tracked"} <= set(sd)
@@ -93,54 +87,3 @@ def test_mvsnet_forward_sequence_through_the_dropins(golden_dir, name, monkeypat
     assert np.abs(depth.detach().cpu().numpy()[:, 0] - g["depth"][:, 0])[ok].max() < 0.005 * step
     depth.sum().backward()
     assert feat.grad is not None and bool(torch.isfinite(feat.grad).all())
-
-
-_REAL_MODEL_SCRIPT = r"""
-import sys, os
-ROOT, REF = sys.argv[1], sys.argv[2]
-PKG = os.path.join(ROOT, "deep-multiview-depth-estimation_b200")
-sys.path.insert(0, REF)                                   # the reference's scripts/ (config, utils, model, ...)
-# ---- the swap of INTEGRATION.md section 2: drop-in modules shadow homography / costvolume / depthmap
-sys.path.insert(0, os.path.join(PKG, "dropin"))
-sys.path.insert(0, PKG)
-import torch
-import model                                             # the reference's UNMODIFIED scripts/model.py
-import mvs_b200
-model.CostVolumeReg = mvs_b200.CostVolumeReg             # the one rebinding (model.py:161 then builds the native regulariser)
-dropin = os.path.join(PKG, "dropin")
-for fn in (model.homography_warping, model.assemble_cost_volume, model.extract_depth_map):
-    assert os.path.dirname(os.path.abspath(sys.modules[fn.__module__].__file__)) == dropin, fn
-assert "kornia" not in sys.modules                       # the reference's own homography.py was never imported
-torch.manual_seed(0)
-net = model.MVSNet()                                     # exactly as train.py:159 / test.py:199 build it
-assert type(net.cost_volume_reg) is mvs_b200.CostVolumeReg
-assert net.cost_volume_reg.conv_0_0.weight.device.type == model.DEVICE.type     # reference default device=DEVICE (model.py:70)
-assert sum(p.numel() for p in net.parameters) == 382016  # MVSNet.parameters is a LIST (model.py:164-166); report Table 1
-B, V = 1, 3
-img = torch.randn(B * V, 3, 512, 640)
-K = torch.eye(3).repeat(B * V, 1, 1); R = torch.eye(3).repeat(B * V, 1, 1); T = torch.zeros(B * V, 3, 1)
-d_min, d_int = torch.full((B, 1, 1, 1), 425.0), torch.ones(B, 1, 1, 1)
-try:
-    with torch.no_grad():
-        net(img.to(model.DEVICE), K, R, T, d_min, d_int, B, V)
-except mvs_b200.MvsB200Error as e:
-    print("REACHED_NATIVE_PATH_NO_CUDA:", str(e)[:80])
-else:
-    print("FORWARD_RAN_ON", model.DEVICE)
-"""
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/scripts"), reason="the reference tree is only mounted in the authoring container")
-def test_real_reference_model_binds_the_dropins():
-    """The reference's UNMODIFIED scripts/model.py, imported with dropin/ ahead of scripts/ on sys.path and the one
-    CostVolumeReg rebinding of INTEGRATION.md: `model.homography_warping` & co. are the drop-ins, `MVSNet()` builds the native
-    regulariser with the reference's default device, and `MVSNet.forward` reaches the native path (here, without a GPU, its
-    refusal to compute on the CPU; on a CUDA machine the forward runs)."""
-    import subprocess
-    r = subprocess.run([sys.executable, "-c", _REAL_MODEL_SCRIPT, ROOT, "/root/reference/scripts"], capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0, r.stderr[-3000:]
-    if torch.cuda.is_available():
-        assert "FORWARD_RAN_ON" in r.stdout, r.stdout
-    else:
-        assert "REACHED_NATIVE_PATH_NO_CUDA" in r.stdout, r.stdout

@@ -1,9 +1,8 @@
 """SURVEY §8 row f4: the DTU on-disk formats and the checkpoint dictionary (mvs_b200/dtu.py) against what the UNMODIFIED reference
 reads from the same files (tests/golden/dtu/ + tests/golden/dtu_formats.npz, written by oracle/make_golden_dtu.py) -- bit-exact,
-the reference's quirks included; against the live reference when /root/reference is mounted (this container only)."""
+the reference's quirks included."""
 import os
 import random
-import sys
 
 import numpy as np
 import pytest
@@ -110,19 +109,14 @@ def test_native_regulariser_loads_a_reference_shaped_checkpoint():
     assert torch.equal(other.conv_2_1.weight, reg.conv_2_1.weight + 1)
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/scripts/data.py"), reason="the reference tree is only in the build container")
-def test_against_the_live_reference():
-    sys.path.insert(0, "/root/reference/scripts")
-    try:
-        import data as ref
-    except Exception as e:                                            # cv2 / torchvision of the reference's imports absent
-        pytest.skip(f"reference data.py does not import here: {e}")
-    finally:
-        sys.path.remove("/root/reference/scripts")
-    c = ref.Cameras(BASE, [0, 1, 2, 3])
+def test_against_the_recorded_reference():
+    """What the reference's data.py (`Cameras`, `load_depth`) returned for tests/golden/dtu, as oracle/make_golden_dtu.py recorded
+    it in dtu_formats.npz: the same per-camera arrays, pairs and depth map, element for element."""
     mine = dtu.read_cameras(BASE, [0, 1, 2, 3])
     for key in ("K", "R", "T", "d", "d_int"):
-        assert all(np.array_equal(a, b) for a, b in zip(getattr(c, key), mine[key]))
-    assert all(np.array_equal(a, b) for a, b in zip(c.pairs, mine["pairs"]))
+        want = GOLD[f"all_{key}"]
+        assert len(mine[key]) == len(want) and all(np.array_equal(a, b) for a, b in zip(want, mine[key])), key
+    assert len(mine["pairs"]) == int(GOLD["all_n_pairs"])
+    assert all(np.array_equal(GOLD[f"all_pair{k}"], p) for k, p in enumerate(mine["pairs"]))
     p = os.path.join(BASE, "Depths", "scan1_train", "depth_map_0000.pfm")
-    assert np.array_equal(ref.load_depth(p), dtu.load_pfm(p))
+    assert np.array_equal(GOLD["pfm_depth_map_0000.pfm"], dtu.load_pfm(p))
