@@ -1101,9 +1101,14 @@ struct KdnParams {
     int planar;                     // 1: the planes are independent maps (2D convolution, mvsb200_conv2d_rows_fwd): only the middle
                                     // depth slice of the filter exists -- MMAs of N = Cout on its row block, one slab per output
                                     // plane (no halo planes), the accumulator IS the output plane (no running partial sums)
+    const float* scale;             // AFF: y = relu(acc * scale[c] + shift[c]) per stored channel c of the launch's row block
+    const float* shift;             // (fp32 [cout] vectors, offset to the block's first row), then ONE rounding to bf16
 };
 
-template <int CIN, int NOUT, int MB>
+// AFF (eval-mode BatchNorm + ReLU folded into the epilogue): scale / shift are read from global memory (L1-resident, 2 x cout
+// floats) per 8-channel store, after the TMEM load of the slab -- never held across the epilogue, whose volume mode already runs
+// near the register limit on its running partial sums.
+template <int CIN, int NOUT, int MB, bool AFF = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
 conv3d_s1_kdn_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                      const __grid_constant__ KdnParams kp) {
@@ -1290,6 +1295,11 @@ conv3d_s1_kdn_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
 #pragma unroll
                             for (int i = 0; i < 16; i += 8) {
                                 if (c0 + i < p.cout) {
+                                    if constexpr (AFF) {
+#pragma unroll
+                                        for (int j = 0; j < 8; ++j)
+                                            o[i + j] = fmaxf(fmaf(o[i + j], kp.scale[c0 + i + j], kp.shift[c0 + i + j]), 0.f);
+                                    }
                                     const uint4 u = make_uint4(pack_bf16x2(o[i], o[i + 1]), pack_bf16x2(o[i + 2], o[i + 3]),
                                                                pack_bf16x2(o[i + 4], o[i + 5]), pack_bf16x2(o[i + 6], o[i + 7]));
                                     *reinterpret_cast<uint4*>(row + c0 + i) = u;
@@ -1317,10 +1327,10 @@ TilePlan plan_tiles_mb(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_
 
 static thread_local int g_kdn_planar = 0;        // set by mvsb200_conv2d_rows_fwd around its call of the kdn dispatch
 
-template <int CIN, int NOUT, int MB>
+template <int CIN, int NOUT, int MB, bool AFF = false>
 int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
                        int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, const TilePlan& tp, int slots,
-                       cudaStream_t st, int cin_real = CIN) {
+                       cudaStream_t st, int cin_real = CIN, const float* scale = nullptr, const float* shift = nullptr) {
     // cin_real < CIN: voxel rows of x hold cin_real channels; the TMA box is CIN wide, the channels beyond the tensor's extent
     // arrive as zeros (out-of-bounds fill) -- an 8-channel volume feeds the K = 16 MMA without a widened copy
     constexpr int ROWB = CIN * 2;
@@ -1362,6 +1372,8 @@ int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
     kp.slots = slots;
     kp.planar = g_kdn_planar;
+    kp.scale = AFF ? scale + y_coff : nullptr;
+    kp.shift = AFF ? shift + y_coff : nullptr;
     const int halo = kp.planar ? 0 : 2;
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
     int sms = 148;
@@ -1383,15 +1395,16 @@ int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int
     p.n_items = (int)(tiles * p.nchunks * B);
     const dim3 grid((unsigned)(p.n_items < sms ? p.n_items : sms), 1, 1);
     const size_t smem = 1024 + W_BYTES_AL + (size_t)slots * tp.slab_bytes + 256;
-    MVS_CUDA(cudaFuncSetAttribute(conv3d_s1_kdn_kernel<CIN, NOUT, MB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    conv3d_s1_kdn_kernel<CIN, NOUT, MB><<<grid, kTcThreads, smem, st>>>(tm_x, tm_w, kp);
+    MVS_CUDA(cudaFuncSetAttribute(conv3d_s1_kdn_kernel<CIN, NOUT, MB, AFF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    conv3d_s1_kdn_kernel<CIN, NOUT, MB, AFF><<<grid, kTcThreads, smem, st>>>(tm_x, tm_w, kp);
     MVS_CHECK_LAUNCH("conv3d_s1_kdn");
     return MVSB200_OK;
 }
 
-template <int CIN, int NOUT>
+template <int CIN, int NOUT, bool AFF = false>
 int launch_conv_kdn(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
-                    int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, cudaStream_t st, int cin_real = CIN) {
+                    int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, cudaStream_t st, int cin_real = CIN,
+                    const float* scale = nullptr, const float* shift = nullptr) {
     constexpr int ROWB = CIN * 2;
     constexpr size_t W_BYTES_AL = ((size_t)27 * NOUT * ROWB + 1023) / 1024 * 1024;
     constexpr int MBMAX = 512 / (2 * 3 * NOUT) >= 4 ? 4 : (512 / (2 * 3 * NOUT) >= 2 ? 2 : 1);
@@ -1422,7 +1435,7 @@ int launch_conv_kdn(const void* x, const void* w, void* y, int B, int Di, int Hi
         }
     }
     MVS_REQUIRE(best.score > 0, "conv3d_s1_kdn: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
-#define MVS_KDN(M) return launch_conv_kdn_mb<CIN, NOUT, M>(x, w, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, y_coff, n_rows, w_row0, off_d, off_h, off_w, best, best_slots, st, cin_real)
+#define MVS_KDN(M) return launch_conv_kdn_mb<CIN, NOUT, M, AFF>(x, w, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, y_coff, n_rows, w_row0, off_d, off_h, off_w, best, best_slots, st, cin_real, scale, shift)
     if (best.MB == 1) MVS_KDN(1);
     if constexpr (MBMAX >= 2) { if (best.MB == 2) MVS_KDN(2); }
     if constexpr (MBMAX >= 4) { if (best.MB == 4) MVS_KDN(4); }
@@ -1457,9 +1470,22 @@ struct DeconvParams {
     __nv_bfloat16* y;
     float* stats;                   // null, or [gridDim.x][2][cout]: per-CTA sums of the stored values and of their squares (the
                                     // train-mode BatchNorm that follows takes its statistics from here: no pass over the canvas)
+    // EPI only (see deconv3d_s2_tc_kernel): the output window and the eval-mode BatchNorm + ReLU + skip-add epilogue
+    int lo_d, lo_h, lo_w;           // canvas voxel at the window's origin; Do / Ho / Wo above are then the window's END
+    int j0_d, j0_h, j0_w;           // first voxel octet that meets the window: lo / 2 (Jd / Jh / Jw count the octets from there)
+    const float* scale;             // fp32 [cout]
+    const float* shift;             // fp32 [cout]
+    const __nv_bfloat16* add;       // null, or bf16 rows in the window's frame with y's strides
 };
 
-template <int CIN, int NOUT>
+// EPI: eval-mode form.  y = relu(acc * scale[c] + shift[c]) (+ add[voxel][c]), rounded once to bf16, written only on an
+// axis-aligned WINDOW [lo, Do) x [lo_h, Ho) x [lo_w, Wo) of the canvas, in the window's frame (voxel lo -> row 0 of y / add).
+// Geometry: the kernel's work unit is the voxel octet J (outputs 2J + par, par in {0,1}^3).  The octets issued are those that
+// meet the window, J = j0 + j with j0 = floor(lo / 2) and j < Jd = floor((Do - 1) / 2) - j0 + 1 per axis; the input slabs are
+// fetched j0 further along.  An odd lo means the first octet's parity-0 voxels lie before the window: like the voxels past
+// Do they are computed and not stored.  The MMA schedule (one MMA per input shift) and the 32-byte stores are those of the
+// dense form, so the window of a full-canvas launch and a windowed launch store bit-identical values.
+template <int CIN, int NOUT, bool EPI = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
 deconv3d_s2_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_w,
                       const __grid_constant__ DeconvParams p) {
@@ -1536,7 +1562,11 @@ deconv3d_s2_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
                 if (gs >= kSlots3) mbar_wait(empty + slot, ((gs / kSlots3) - 1) & 1);
                 if (elect_one()) {
                     mbar_expect_tx(full + slot, box_bytes);
-                    tma_load_5d(slab_smem + (size_t)slot * p.slab_bytes, &tm_x, full + slot, 0, x0 - 1, y0 - 1, d_begin - 1 + s, b);
+                    if constexpr (EPI)
+                        tma_load_5d(slab_smem + (size_t)slot * p.slab_bytes, &tm_x, full + slot, 0, p.j0_w + x0 - 1, p.j0_h + y0 - 1,
+                                    p.j0_d + d_begin - 1 + s, b);
+                    else
+                        tma_load_5d(slab_smem + (size_t)slot * p.slab_bytes, &tm_x, full + slot, 0, x0 - 1, y0 - 1, d_begin - 1 + s, b);
                 }
                 __syncwarp();
             }
@@ -1603,11 +1633,21 @@ deconv3d_s2_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
             tj[mb] = m / p.BW; ti[mb] = m - tj[mb] * p.BW;
             in_tile[mb] = ti[mb] < p.BW - 2 && tj[mb] < p.L;
         }
+        // EPI: the BatchNorm vectors in registers for the whole epilogue (at most 2 x 32 floats; this kernel has the room, and
+        // per-voxel loads of them cost more epilogue issue slots than the stores)
+        float e_sc[EPI ? NOUT : 1], e_sh[EPI ? NOUT : 1];
+        if constexpr (EPI) {
+#pragma unroll
+            for (int ch = 0; ch < NOUT; ++ch) {
+                e_sc[ch] = ch < p.cout ? p.scale[ch] : 0.f;
+                e_sh[ch] = ch < p.cout ? p.shift[ch] : 0.f;
+            }
+        }
         // per-channel sums of what this thread stores, for the BatchNorm that follows
         float st_s[NOUT], st_q[NOUT];
 #pragma unroll
         for (int ch = 0; ch < NOUT; ++ch) { st_s[ch] = 0.f; st_q[ch] = 0.f; }
-        const bool want_stats = p.stats != nullptr;
+        const bool want_stats = !EPI && p.stats != nullptr;
         int gp = 0;
         for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
             int b, d_begin, nd, x0, y0;
@@ -1625,6 +1665,48 @@ deconv3d_s2_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
                         tmem_ld<NOUT>(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(((stage * MB + mb) * 8 + c) * NOUT), v);
                         tmem_ld_wait();
                         const int cl = p.g.cls_of_pos[c];                  // accumulator block c holds output-parity class cl
+                        if constexpr (EPI) {
+                            const int z = 2 * p.j0_d + oz + (cl >> 2), yy = 2 * p.j0_h + oy + (cl >> 1 & 1), xx = 2 * p.j0_w + ox + (cl & 1);
+                            if (in_tile[mb] && z >= p.lo_d && yy >= p.lo_h && xx >= p.lo_w && z < p.Do && yy < p.Ho && xx < p.Wo) {
+                                const long long off = (long long)b * p.y_sb + (long long)(z - p.lo_d) * p.y_sd +
+                                                      (long long)(yy - p.lo_h) * p.y_sh + (long long)(xx - p.lo_w) * p.y_sw;
+                                // 8 channels ch .. ch + 7: affine, ReLU, skip addition in fp32, one rounding
+                                auto epi8 = [&](int ch) {
+                                    float a[8];
+#pragma unroll
+                                    for (int i = 0; i < 8; ++i) a[i] = fmaxf(fmaf(__uint_as_float(v[ch + i]), e_sc[ch + i], e_sh[ch + i]), 0.f);
+                                    if (p.add != nullptr) {
+                                        const uint4 r = *reinterpret_cast<const uint4*>(p.add + off + ch);
+                                        const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+                                        for (int i = 0; i < 4; ++i) {
+                                            a[2 * i] += __uint_as_float(rw[i] << 16);
+                                            a[2 * i + 1] += __uint_as_float(rw[i] & 0xffff0000u);
+                                        }
+                                    }
+                                    return make_uint4(pack_bf16x2(a[0], a[1]), pack_bf16x2(a[2], a[3]), pack_bf16x2(a[4], a[5]),
+                                                      pack_bf16x2(a[6], a[7]));
+                                };
+                                __nv_bfloat16* row = p.y + off;
+                                if (p.wide_io) {
+#pragma unroll
+                                    for (int ch = 0; ch < NOUT; ch += 16) {
+                                        if (ch < p.cout) {
+                                            const uint4 lo = epi8(ch), hi = epi8(ch + 8);
+                                            U8 o;
+                                            o.v[0] = lo.x; o.v[1] = lo.y; o.v[2] = lo.z; o.v[3] = lo.w;
+                                            o.v[4] = hi.x; o.v[5] = hi.y; o.v[6] = hi.z; o.v[7] = hi.w;
+                                            st_u8(row + ch, o);
+                                        }
+                                    }
+                                } else {
+#pragma unroll
+                                    for (int ch = 0; ch < NOUT; ch += 8)
+                                        if (ch < p.cout) *reinterpret_cast<uint4*>(row + ch) = epi8(ch);
+                                }
+                            }
+                            continue;
+                        }
                         const int z = oz + (cl >> 2), yy = oy + (cl >> 1 & 1), xx = ox + (cl & 1);
                         if (in_tile[mb] && z < p.Do && yy < p.Ho && xx < p.Wo) {
                             if (want_stats) {
@@ -1720,17 +1802,25 @@ TilePlan plan_tiles_mb(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_
     return best;
 }
 
-template <int CIN, int NOUT>
+// EPI: win (host int[6]: lo_d, lo_h, lo_w, n_d, n_h, n_w) is the window of the Do x Ho x Wo canvas that is written, y / add
+// point at its origin; scale / shift / add as in DeconvParams.
+template <int CIN, int NOUT, bool EPI = false>
 int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
                      int n_rows, int pad_d, int pad_h, int pad_w, const long long* y_strides4, cudaStream_t st,
-                     float* stats = nullptr, int* n_blocks_out = nullptr) {
+                     float* stats = nullptr, int* n_blocks_out = nullptr, const int* win = nullptr, const float* scale = nullptr,
+                     const float* shift = nullptr, const void* add = nullptr) {
     constexpr int ROWB = CIN * 2;
     constexpr int MB = 512 / (16 * NOUT);
     constexpr size_t W_BYTES_AL = ((size_t)kDeconvSlots * NOUT * ROWB + 1023) / 1024 * 1024;
     EncodeTiledFn enc = encode_fn();
     MVS_REQUIRE(enc != nullptr, "deconv3d_s2: cuTensorMapEncodeTiled is not available from the driver");
     const size_t smem_budget = 227 * 1024 - 1024 - 1024;      // - the epilogue's statistics rows
-    const int Jd = (Do + 1) / 2, Jh = (Ho + 1) / 2, Jw = (Wo + 1) / 2;
+    int Jd = (Do + 1) / 2, Jh = (Ho + 1) / 2, Jw = (Wo + 1) / 2;
+    if (EPI) {
+        Jd = (win[0] + win[3] - 1) / 2 - win[0] / 2 + 1;
+        Jh = (win[1] + win[4] - 1) / 2 - win[1] / 2 + 1;
+        Jw = (win[2] + win[5] - 1) / 2 - win[2] / 2 + 1;
+    }
     const TilePlan tp = plan_tiles_mb(Jh, Jw, ROWB, W_BYTES_AL, smem_budget, MB);
     MVS_REQUIRE(tp.score > 0, "deconv3d_s2: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
 
@@ -1759,6 +1849,13 @@ int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int H
 
     DeconvParams p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.Jd = Jd; p.Jh = Jh; p.Jw = Jw;
+    p.lo_d = p.lo_h = p.lo_w = p.j0_d = p.j0_h = p.j0_w = 0;
+    p.scale = scale; p.shift = shift; p.add = reinterpret_cast<const __nv_bfloat16*>(add);
+    if (EPI) {
+        p.lo_d = win[0]; p.lo_h = win[1]; p.lo_w = win[2];
+        p.j0_d = win[0] / 2; p.j0_h = win[1] / 2; p.j0_w = win[2] / 2;
+        p.Do = win[0] + win[3]; p.Ho = win[1] + win[4]; p.Wo = win[2] + win[5];
+    }
     p.BW = tp.BW; p.L = tp.L; p.MB = MB; p.tiles_x = tp.tiles_x; p.tiles_y = tp.tiles_y;
     p.cout = cout; p.n_rows = n_rows; p.slab_bytes = tp.slab_bytes;
     { const int rc = build_deconv_wide(pad_d, pad_h, pad_w, NOUT, p.g); if (rc != MVSB200_OK) return rc; }
@@ -1789,8 +1886,8 @@ int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int H
     const size_t smem = 1024 + W_BYTES_AL + (size_t)kSlots3 * tp.slab_bytes + 256 + 1024;
     p.stats = stats;
     if (n_blocks_out) *n_blocks_out = (int)grid.x;
-    MVS_CUDA(cudaFuncSetAttribute(deconv3d_s2_tc_kernel<CIN, NOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    deconv3d_s2_tc_kernel<CIN, NOUT><<<grid, kTcThreads, smem, st>>>(tm_x, tm_w, p);
+    MVS_CUDA(cudaFuncSetAttribute(deconv3d_s2_tc_kernel<CIN, NOUT, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    deconv3d_s2_tc_kernel<CIN, NOUT, EPI><<<grid, kTcThreads, smem, st>>>(tm_x, tm_w, p);
     MVS_CHECK_LAUNCH("deconv3d_s2_tc");
     return MVSB200_OK;
 }
@@ -2019,12 +2116,48 @@ extern "C" int mvsb200_deconv3d_s2_fwd(const void* x, const void* w_packed, void
                                          nullptr, nullptr, stream);
 }
 
+/* Eval-mode form of mvsb200_deconv3d_s2_fwd (include/mvs_b200.h): y = relu(acc * scale + shift) (+ add) on a window of the canvas
+ * (deconv3d_s2_tc_kernel<.., EPI = true>). */
+extern "C" int mvsb200_deconv3d_s2_fwd_affine(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                              int Do, int Ho, int Wo, int cout, int n_rows, int pad_d, int pad_h, int pad_w,
+                                              const int* window6_host, const int64_t* y_strides4, const float* scale, const float* shift,
+                                              const void* add, void* stream) {
+    const char* name = "deconv3d_s2_fwd_affine";
+    MVS_REQUIRE(x && w_packed && y && y_strides4 && window6_host && scale && shift, "%s: null pointer", name);
+    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y) && (add == nullptr || aligned16(add)),
+                "%s: pointers must be 16-byte aligned", name);
+    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
+    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && (n_rows == 16 || n_rows == 32),
+                "%s: cout must be a multiple of 8 and n_rows 16 or 32 (cout=%d n_rows=%d)", name, cout, n_rows);
+    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
+    const int* wn = window6_host;
+    const int ext[3] = {Do, Ho, Wo};
+    for (int a = 0; a < 3; ++a)
+        MVS_REQUIRE(wn[a] >= 0 && wn[3 + a] >= 1 && wn[a] + wn[3 + a] <= ext[a], "%s: window [%d, %d) outside the canvas extent %d (axis %d)",
+                    name, wn[a], wn[a] + wn[3 + a], ext[a], a);
+    const long long ys[4] = {(long long)y_strides4[0], (long long)y_strides4[1], (long long)y_strides4[2], (long long)y_strides4[3]};
+    for (int i = 0; i < 4; ++i) MVS_REQUIRE(ys[i] % 8 == 0, "%s: output strides must be multiples of 8 elements", name);
+    cudaStream_t st = (cudaStream_t)stream;
+    int rc = MVSB200_E_UNSUPPORTED;
+#define MVS_DC(CI, NO) rc = launch_deconv_s2<CI, NO, true>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, n_rows, pad_d, pad_h, pad_w, ys, st, \
+                                                          nullptr, nullptr, wn, scale, shift, add)
+    if (Cin == 16 && n_rows == 16) MVS_DC(16, 16);
+    else if (Cin == 16 && n_rows == 32) MVS_DC(16, 32);
+    else if (Cin == 32 && n_rows == 16) MVS_DC(32, 16);
+    else if (Cin == 32 && n_rows == 32) MVS_DC(32, 32);
+    else if (Cin == 64 && n_rows == 16) MVS_DC(64, 16);
+    else if (Cin == 64 && n_rows == 32) MVS_DC(64, 32);
+    else MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
+#undef MVS_DC
+    return rc;
+}
+
 /* Same convolution as mvsb200_conv3d_s1_fwd with the depth tap folded into the MMA N extent (conv3d_s1_kdn_kernel).
  * w_packed: [9 (kh,kw)][3 (kd)][n_rows][Cin] bf16. */
-extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
-                                         int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
-                                         void* stream) {
-    const char* name = "conv3d_s1_fwd_kdn";
+template <bool AFF>
+static int kdn_dispatch(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin, int Do, int Ho, int Wo,
+                        int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w, void* stream, const char* name,
+                        const float* scale = nullptr, const float* shift = nullptr) {
     MVS_REQUIRE(x && w_packed && y, "%s: null pointer", name);
     MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "%s: pointers must be 16-byte aligned", name);
     MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
@@ -2036,9 +2169,9 @@ extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, vo
         const int nout = n_rows - row0 < 32 ? n_rows - row0 : 32;
         const int c_here = cout - row0 < nout ? cout - row0 : nout;
         int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_CONV(CI, NO) rc = launch_conv_kdn<CI, NO>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st)
-        if (Cin == 8 && nout == 16) rc = launch_conv_kdn<16, 16>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8);
-        else if (Cin == 8 && nout == 32) rc = launch_conv_kdn<16, 32>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8);
+#define MVS_CONV(CI, NO) rc = launch_conv_kdn<CI, NO, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, CI, scale, shift)
+        if (Cin == 8 && nout == 16) rc = launch_conv_kdn<16, 16, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8, scale, shift);
+        else if (Cin == 8 && nout == 32) rc = launch_conv_kdn<16, 32, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8, scale, shift);
         else if (Cin == 16 && nout == 16) MVS_CONV(16, 16);
         else if (Cin == 16 && nout == 32) MVS_CONV(16, 32);
         else if (Cin == 32 && nout == 16) MVS_CONV(32, 16);
@@ -2050,6 +2183,28 @@ extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, vo
         if (rc != MVSB200_OK) return rc;
     }
     return MVSB200_OK;
+}
+
+extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                         int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
+                                         void* stream) {
+    return kdn_dispatch<false>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, stream,
+                               "conv3d_s1_fwd_kdn");
+}
+
+/* mvsb200_conv3d_s1_fwd_kdn (planar = 0) or mvsb200_conv2d_rows_fwd (planar = 1, B = 1, Di = Do = maps) with eval-mode BatchNorm +
+ * ReLU in the epilogue: y = relu(acc * scale[c] + shift[c]), scale / shift fp32 [cout] device vectors. */
+extern "C" int mvsb200_conv3d_s1_fwd_kdn_affine(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                                int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
+                                                int planar, const float* scale, const float* shift, void* stream) {
+    const char* name = "conv3d_s1_fwd_kdn_affine";
+    MVS_REQUIRE(scale && shift, "%s: null scale / shift", name);
+    MVS_REQUIRE(planar == 0 || (planar == 1 && B == 1 && Di == Do && off_d == 0), "%s: planar mode takes B = 1, Di = Do, off_d = 0", name);
+    g_kdn_planar = planar;
+    const int rc = kdn_dispatch<true>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, stream, name,
+                                      scale, shift);
+    g_kdn_planar = 0;
+    return rc;
 }
 
 /* Weight gradient of the STRIDE-2 layers on the same kernel:  gw[k][cb][cs] = sum_o big(2o - pad + k)[cb] * small(o)[cs]

@@ -35,6 +35,7 @@ _SIGNATURES = {
     "mvsb200_variance_views_bwd": (_I, [_P, _P, _P, _I, _I, _c.c_int64, _P]),
     "mvsb200_conv3d_s1_fwd": (_I, [_P, _P, _P] + [_I] * 14 + [_P]),
     "mvsb200_conv3d_s1_fwd_kdn": (_I, [_P, _P, _P] + [_I] * 14 + [_P]),
+    "mvsb200_conv3d_s1_fwd_kdn_affine": (_I, [_P, _P, _P] + [_I] * 15 + [_P, _P, _P]),
     "mvsb200_conv3d_s1_fwd_ex": (_I, [_P, _P, _P] + [_I] * 13 + [_c.c_uint, _P, _P]),
     "mvsb200_conv3d_s2_fwd": (_I, [_P, _P, _P] + [_I] * 14 + [_P]),
     "mvsb200_conv3d_s2_fwd_stats": (_I, [_P, _P, _P] + [_I] * 14 + [_P, _P, _P]),
@@ -42,6 +43,7 @@ _SIGNATURES = {
     "mvsb200_conv3d_s2_wgrad_lines": (_I, [_P, _P, _P] + [_I] * 12 + [_P, _P]),
     "mvsb200_deconv3d_s2_fwd": (_I, [_P, _P, _P] + [_I] * 13 + [_P, _P]),
     "mvsb200_deconv3d_s2_fwd_stats": (_I, [_P, _P, _P] + [_I] * 13 + [_P, _P, _P, _P]),
+    "mvsb200_deconv3d_s2_fwd_affine": (_I, [_P, _P, _P] + [_I] * 13 + [_P, _P, _P, _P, _P, _P]),
     "mvsb200_deconv3d_s2_kc_fwd": (_I, [_P, _I, _P, _P, _P, _I, _P] + [_I] * 12 + [_P, _I, _P]),
     "mvsb200_conv3d_s1_wgrad": (_I, [_P, _P, _P] + [_I] * 12 + [_P]),
     "mvsb200_conv3d_s1_wgrad_ex": (_I, [_P, _P, _P] + [_I] * 12 + [_c.c_uint, _P]),

@@ -37,15 +37,16 @@ def _n_rows(c):
     return 16 if c <= 16 else (32 if c <= 32 else 64)
 
 
-def _pack2d(w, role, n_rows, n_cols):
+def _pack2d(w, role, n_rows, n_cols, out=None):
     """Conv2d weight [co, ci, 3, 3] (dense fp32) -> the bf16 [(kh, kw)][kd][row][col] filter operand of the kdn kernel in one
     launch: middle depth slice = the 3x3 filter, the other slices and the padded rows / columns zero.  role "fwd": rows = co,
-    columns = ci; "dgrad": taps flipped, rows = ci, columns = co."""
+    columns = ci; "dgrad": taps flipped, rows = ci, columns = co.  out: the buffer to write (the filter is re-packed in place)."""
     from .conv3d_sm100 import _FLIP, _NAT, _kdn_order
     co, ci = w.shape[:2]
     taps = [t - 9 if 9 <= t < 18 else -1 for t in _kdn_order(_NAT if role == "fwd" else _FLIP)]
     rows_real, cols_real, sr, sc = (co, ci, 9 * ci, 9) if role == "fwd" else (ci, co, 9, 9 * ci)
-    out = torch.empty((27, n_rows, n_cols), dtype=torch.bfloat16, device=w.device)
+    if out is None:
+        out = torch.empty((27, n_rows, n_cols), dtype=torch.bfloat16, device=w.device)
     _lib.call("mvsb200_pack_filter", w.data_ptr(), out.data_ptr(), 27, n_rows, n_cols, rows_real, cols_real, 0, sr, sc,
               (ctypes.c_int * 27)(*taps), _stream())
     return out
@@ -177,20 +178,31 @@ def _bn_relu(y, bn, s2d=False):
 _ENC_LAYERS = ((3, 8, 3, 1), (8, 8, 3, 1), (8, 16, 5, 2), (16, 16, 3, 1), (16, 16, 3, 1), (16, 32, 5, 2), (32, 32, 3, 1), (32, 32, 3, 1))
 
 
+def encoder_layout_error(module):
+    """None when FeatureEncoder `module` has the reference's layout (eight bias-free fp32 Conv2d of _ENC_LAYERS, seven
+    BatchNorm2d), else what differs."""
+    convs = [m for m in getattr(module, "model", ()) if isinstance(m, torch.nn.Conv2d)]
+    bns = [m for m in getattr(module, "model", ()) if isinstance(m, torch.nn.BatchNorm2d)]
+    if len(convs) != 8 or len(bns) != 7:
+        return f"feature encoder: {len(convs)} Conv2d / {len(bns)} BatchNorm2d layers, the reference has 8 / 7"
+    for i, (c, (ci, co, k, s)) in enumerate(zip(convs, _ENC_LAYERS)):
+        if (c.in_channels, c.out_channels, c.kernel_size, c.stride, c.padding) != (ci, co, (k, k), (s, s), (k // 2, k // 2)) \
+                or c.bias is not None or c.weight.dtype != torch.float32:
+            return f"feature encoder: convolution {i} is not the reference's {ci} -> {co}, {k}x{k}, stride {s}, bias-free fp32 layer"
+    for i, (b, (_, co, _, _)) in enumerate(zip(bns, _ENC_LAYERS)):
+        if b.num_features != co:
+            return f"feature encoder: BatchNorm {i} has {b.num_features} channels, the reference {co}"
+    return None
+
+
 def encoder_ok(module, images) -> bool:
     """Whether FeatureEncoder `module` can run on the library's kernels: the reference's eight layers, train-mode BatchNorm, fp32
     images on the GPU whose sides are multiples of 4."""
     from . import conv3d_sm100
-    convs = [m for m in module.model if isinstance(m, torch.nn.Conv2d)]
-    bns = [m for m in module.model if isinstance(m, torch.nn.BatchNorm2d)]
-    if not (images.is_cuda and images.dtype == torch.float32 and images.dim() == 4 and module.training and len(convs) == 8
-            and len(bns) == 7 and images.shape[2] % 4 == 0 and images.shape[3] % 4 == 0 and min(images.shape[2:]) >= 12):
+    if not (images.is_cuda and images.dtype == torch.float32 and images.dim() == 4 and module.training
+            and images.shape[2] % 4 == 0 and images.shape[3] % 4 == 0 and min(images.shape[2:]) >= 12):
         return False
-    for c, (ci, co, k, s) in zip(convs, _ENC_LAYERS):
-        if (c.in_channels, c.out_channels, c.kernel_size, c.stride, c.padding) != (ci, co, (k, k), (s, s), (k // 2, k // 2)) \
-                or c.bias is not None or c.weight.dtype != torch.float32:
-            return False
-    return conv3d_sm100.available()
+    return encoder_layout_error(module) is None and conv3d_sm100.available()
 
 
 def encode_native(module, images):

@@ -116,13 +116,18 @@ def refine_output(res_rows, norm, d_min, span):
     return _RefineOutput.apply(res_rows, norm, _per_sample(d_min, B, "d_min"), _per_sample(span, B, "depth span"))
 
 
+def layout_ok(module) -> bool:
+    """Whether DepthRefinement `module` has the reference's layers: four bias-free 3x3 Conv2d 4 -> 32 -> 32 -> 32 -> 1."""
+    convs = [m for m in getattr(module, "model", ()) if isinstance(m, torch.nn.Conv2d)]
+    return (len(convs) == 4 and convs[0].in_channels == 4 and convs[-1].out_channels == 1
+            and all(c.kernel_size == (3, 3) and c.stride == (1, 1) and c.padding == (1, 1) and c.bias is None for c in convs)
+            and all(c.out_channels == 32 for c in convs[:3]))
+
+
 def native_ok(module, x_like) -> bool:
     """Whether DepthRefinement `module` can run on the library's kernels: train-mode BatchNorm, CUDA, the reference's widths."""
     from . import conv3d_sm100
-    convs = [m for m in module.model if isinstance(m, torch.nn.Conv2d)]
-    return (x_like.is_cuda and module.training and len(convs) == 4 and convs[0].in_channels == 4 and convs[-1].out_channels == 1
-            and all(c.kernel_size == (3, 3) and c.stride == (1, 1) and c.padding == (1, 1) and c.bias is None for c in convs)
-            and all(c.out_channels == 32 for c in convs[:3]) and conv3d_sm100.available())
+    return x_like.is_cuda and module.training and layout_ok(module) and conv3d_sm100.available()
 
 
 def refine_native(module, initial, images, n_views, d_min, span):

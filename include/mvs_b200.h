@@ -146,6 +146,13 @@ int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, void* y, int 
                               int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
                               void* stream);
 
+/* mvsb200_conv3d_s1_fwd_kdn with eval-mode BatchNorm + ReLU in the epilogue: y = relu(acc * scale[c] + shift[c]) rounded once to
+ * bf16, scale / shift fp32 [cout] device vectors (the filter stays unscaled: the same packed operand as the train path).
+ * planar = 1: the 2D form of mvsb200_conv2d_rows_fwd (B = 1, Di = Do = number of maps, off_d = 0). */
+int mvsb200_conv3d_s1_fwd_kdn_affine(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                     int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
+                                     int planar, const float* scale, const float* shift, void* stream);
+
 /* Same kernel with a subset of the 27 taps (bit (kd*3+kh)*3+kw of tap_mask) and a strided output: the voxel row of
  * output (b,z,y,x) starts at y + b*ys[0] + z*ys[1] + y*ys[2] + x*ys[3] elements (y_strides4: HOST int64).  This is one
  * output-parity class of a stride-2 TRANSPOSED convolution (ConvTranspose3d, scripts/model.py:229-234, used at :115-121):
@@ -198,6 +205,18 @@ int mvsb200_deconv3d_s2_fwd_stats(const void* x, const void* w_packed, void* y, 
  * replacing aten::convolution_backward's data gradient.  out[2J + par] = sum_k W[k] . x[J + (par + pad - k)/2] as above.
  * x: [B, Di, Hi, Wi, x_cs] bf16 dense; w_packed: chunk after chunk, each [28, n_rows, kc_n[c]] bf16 with a 28th all-zero tap (rows = output channels);
  * kc_off / kc_n: HOST int arrays; y as in mvsb200_deconv3d_s2_fwd, cout <= n_rows <= 64; accumulate = 1 adds to y. */
+/* Eval-mode form of mvsb200_deconv3d_s2_fwd: the BatchNorm (running statistics) + ReLU that follows the transposed convolution and
+ * the skip addition after it (scripts/model.py:117-123, relu(BN(deconv(x))) + enc) in the epilogue, on a WINDOW of the canvas:
+ *   y[v] = relu(acc[v] * scale[c] + shift[c]) + add[v][c]      (fp32, one rounding to bf16)
+ * for the voxels v of the box window6_host = {lo_d, lo_h, lo_w, n_d, n_h, n_w} (HOST ints) of the Do x Ho x Wo canvas, written in the
+ * window's frame: y and add (NULL: no addition; else bf16 rows with y's strides) point at the window's origin voxel.  Only the
+ * voxel octets that meet the window are computed.  scale / shift: fp32 [cout] device vectors.  Other arguments as
+ * mvsb200_deconv3d_s2_fwd; stored values are bit-identical to that window of relu(acc * scale + shift) (+ add) on the full canvas. */
+int mvsb200_deconv3d_s2_fwd_affine(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                   int Do, int Ho, int Wo, int cout, int n_rows, int pad_d, int pad_h, int pad_w,
+                                   const int* window6_host, const int64_t* y_strides4_host, const float* scale, const float* shift,
+                                   const void* add, void* stream);
+
 int mvsb200_deconv3d_s2_kc_fwd(const void* x, int x_cs, const void* w_packed, const int* kc_off_host, const int* kc_n_host, int n_kc,
                                void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout, int n_rows,
                                int pad_d, int pad_h, int pad_w, const int64_t* y_strides4_host, int accumulate, void* stream);
