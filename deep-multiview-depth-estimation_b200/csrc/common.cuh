@@ -96,4 +96,19 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     return *reinterpret_cast<uint32_t*>(&h);
 }
 
+// one axis of torch's upsample_bilinear2d with align_corners = False (refine_input, the colours of the fused point cloud):
+// src = (o + 0.5) * scale - 0.5 clamped at 0, taps i0 and i0 + step (clamped at the border), weights l0 and l1
+struct Tap { int i0, step; float l0, l1; };
+
+__device__ __forceinline__ Tap tap_of(int o, float scale, int n_in) {
+    float src = scale * ((float)o + 0.5f) - 0.5f;
+    src = src < 0.f ? 0.f : src;
+    Tap t;
+    t.i0 = min((int)src, n_in - 1);
+    t.step = t.i0 < n_in - 1 ? 1 : 0;
+    t.l1 = src - (float)t.i0;
+    t.l0 = 1.f - t.l1;
+    return t;
+}
+
 }  // namespace mvsb200

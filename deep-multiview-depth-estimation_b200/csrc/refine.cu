@@ -20,19 +20,6 @@ namespace {
 
 constexpr int kRefThreads = 128;
 
-struct Tap { int i0, step; float l0, l1; };
-
-__device__ __forceinline__ Tap tap_of(int o, float scale, int n_in) {
-    float src = scale * ((float)o + 0.5f) - 0.5f;
-    src = src < 0.f ? 0.f : src;
-    Tap t;
-    t.i0 = min((int)src, n_in - 1);
-    t.step = t.i0 < n_in - 1 ? 1 : 0;
-    t.l1 = src - (float)t.i0;
-    t.l0 = 1.f - t.l1;
-    return t;
-}
-
 template <int CP>
 __global__ void __launch_bounds__(kRefThreads) refine_input_fwd_kernel(
         const float* __restrict__ initial, const float* __restrict__ images, long long s_n, long long s_c, long long s_h, long long s_w,

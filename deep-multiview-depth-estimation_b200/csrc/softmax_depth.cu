@@ -21,10 +21,30 @@ constexpr int kPix = 32;       // pixels per CTA (one warp-width of x)
 constexpr int kSlices = 8;     // warps per CTA, each owning planes d = slice (mod 8)
 constexpr int kMaxKeep = 8;
 
+// MVSNet's photometric confidence: the probability mass of the (up to) four planes around the estimate.  t = (depth - d_0) /
+// (d_1 - d_0), k0 = floor(t); conf = sum of P[k] over k in {k0-1 .. k0+2} and [0, D-1], added in ascending k in fp32.  D == 1
+// gives 1; a non-finite depth, index or summed probability gives NaN.  `p(k)` reads plane k of this pixel.
+template <class ProbAt>
+__device__ __forceinline__ float confidence_of(float dep, const float* __restrict__ dv, int D, ProbAt p) {
+    if (!isfinite(dep)) return __int_as_float(0x7fc00000);
+    if (D == 1) return 1.f;
+    const float t = (dep - dv[0]) / (dv[1] - dv[0]);
+    if (!isfinite(t)) return __int_as_float(0x7fc00000);
+    const float k0f = floorf(t);
+    if (k0f < -3.f || k0f > (float)D + 1.f) return 0.f;      // the window misses [0, D-1]
+    const int k0 = (int)k0f;
+    float s = 0.f;
+    for (int k = max(k0 - 1, 0); k <= min(k0 + 2, D - 1); ++k) s += p(k);
+    return isfinite(s) ? s : __int_as_float(0x7fc00000);
+}
+
+// CONF: also write the confidence of every pixel (conf != nullptr, depth required); the plain form keeps its code unchanged
+template <bool CONF>
 __global__ void __launch_bounds__(kPix * kSlices) softmax_depth_fwd_kernel(const float* __restrict__ in, int apply_softmax,
                                                                         const float* __restrict__ depths,
                                                                         float* __restrict__ prob, int32_t* __restrict__ ranks,
-                                                                        float* __restrict__ depth, int D, int hw, int n_keep) {
+                                                                        float* __restrict__ depth, float* __restrict__ conf,
+                                                                        int D, int hw, int n_keep) {
     extern __shared__ float smem[];
     float* tile = smem;                          // [D][kPix]
     float* red = smem + (size_t)D * kPix;        // [kSlices][kPix]
@@ -99,7 +119,18 @@ __global__ void __launch_bounds__(kPix * kSlices) softmax_depth_fwd_kernel(const
             }
         }
         if (depth) depth[(size_t)b * hw + pix] = num / den;
+        if constexpr (CONF)
+            conf[(size_t)b * hw + pix] = confidence_of(num / den, depths + (size_t)b * D, D, [&](int k) { return tile[k * kPix + lane]; });
     }
+}
+
+__global__ void depth_confidence_kernel(const float* __restrict__ prob, const float* __restrict__ depth, const float* __restrict__ depths,
+                                        float* __restrict__ conf, int D, int hw) {
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
+    if (pix >= hw) return;
+    const float* col = prob + (size_t)b * D * hw + pix;
+    conf[(size_t)b * hw + pix] = confidence_of(depth[(size_t)b * hw + pix], depths + (size_t)b * D, D,
+                                               [&](int k) { return col[(size_t)k * hw]; });
 }
 
 __global__ void depth_from_ranks_kernel(const float* __restrict__ prob, const int32_t* __restrict__ ranks,
@@ -166,21 +197,47 @@ __global__ void __launch_bounds__(kPix * kSlices) softmax_bwd_kernel(const float
 
 }  // namespace
 
-extern "C" int mvsb200_softmax_depth_fwd(const float* in, int apply_softmax, const float* depths, float* prob,
-                                         int32_t* ranks, float* depth, int B, int D, int h, int w, int n_est, void* stream) {
-    MVS_REQUIRE(in, "softmax_depth_fwd: null input");
-    MVS_REQUIRE(!apply_softmax || prob, "softmax_depth_fwd: prob output required with apply_softmax");
-    MVS_REQUIRE((depth != nullptr) == (depths != nullptr), "softmax_depth_fwd: depth and depths go together");
-    MVS_REQUIRE(B >= 1 && B <= 65535 && D >= 1 && D <= 1024 && h >= 1 && w >= 1, "softmax_depth_fwd: bad shape");
-    MVS_REQUIRE(n_est >= 1 && n_est <= kMaxKeep, "softmax_depth_fwd: 1 <= n_est <= %d", kMaxKeep);
+template <bool CONF>
+static int softmax_depth_launch(const char* name, const float* in, int apply_softmax, const float* depths, float* prob,
+                                int32_t* ranks, float* depth, float* conf, int B, int D, int h, int w, int n_est, void* stream) {
+    MVS_REQUIRE(in, "%s: null input", name);
+    MVS_REQUIRE(!apply_softmax || prob, "%s: prob output required with apply_softmax", name);
+    MVS_REQUIRE((depth != nullptr) == (depths != nullptr), "%s: depth and depths go together", name);
+    MVS_REQUIRE(!CONF || (conf && depth), "%s: conf and depth outputs required", name);
+    MVS_REQUIRE(B >= 1 && B <= 65535 && D >= 1 && D <= 1024 && h >= 1 && w >= 1, "%s: bad shape", name);
+    MVS_REQUIRE(n_est >= 1 && n_est <= kMaxKeep, "%s: 1 <= n_est <= %d", name, kMaxKeep);
     const int hw = h * w, n_keep = n_est < D ? n_est : D;
     const size_t smem = ((size_t)D * kPix + kSlices * kPix) * sizeof(float) + kMaxKeep * kPix * sizeof(int);
     if (smem > 48 * 1024)   // per-device attribute; cheap, so set whenever the opt-in range is needed
-        MVS_CUDA(cudaFuncSetAttribute(softmax_depth_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        MVS_CUDA(cudaFuncSetAttribute(softmax_depth_fwd_kernel<CONF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid((hw + kPix - 1) / kPix, B);
-    softmax_depth_fwd_kernel<<<grid, kPix * kSlices, smem, (cudaStream_t)stream>>>(in, apply_softmax, depths, prob, ranks,
-                                                                                  depth, D, hw, n_keep);
-    MVS_CHECK_LAUNCH("softmax_depth_fwd");
+    softmax_depth_fwd_kernel<CONF><<<grid, kPix * kSlices, smem, (cudaStream_t)stream>>>(in, apply_softmax, depths, prob, ranks,
+                                                                                        depth, conf, D, hw, n_keep);
+    MVS_CHECK_LAUNCH(name);
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_softmax_depth_fwd(const float* in, int apply_softmax, const float* depths, float* prob,
+                                         int32_t* ranks, float* depth, int B, int D, int h, int w, int n_est, void* stream) {
+    return softmax_depth_launch<false>("softmax_depth_fwd", in, apply_softmax, depths, prob, ranks, depth, nullptr, B, D, h, w,
+                                       n_est, stream);
+}
+
+extern "C" int mvsb200_softmax_depth_conf_fwd(const float* in, int apply_softmax, const float* depths, float* prob,
+                                              int32_t* ranks, float* depth, float* conf, int B, int D, int h, int w, int n_est,
+                                              void* stream) {
+    return softmax_depth_launch<true>("softmax_depth_conf_fwd", in, apply_softmax, depths, prob, ranks, depth, conf, B, D, h, w,
+                                      n_est, stream);
+}
+
+extern "C" int mvsb200_depth_confidence(const float* prob, const float* depth, const float* depths, float* conf, int B, int D,
+                                        int h, int w, void* stream) {
+    MVS_REQUIRE(prob && depth && depths && conf, "depth_confidence: null pointer");
+    MVS_REQUIRE(B >= 1 && B <= 65535 && D >= 1 && h >= 1 && w >= 1, "depth_confidence: bad shape");
+    const int hw = h * w;
+    dim3 grid((hw + 127) / 128, B);
+    depth_confidence_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(prob, depth, depths, conf, D, hw);
+    MVS_CHECK_LAUNCH("depth_confidence");
     return MVSB200_OK;
 }
 

@@ -14,7 +14,10 @@ from . import conv3d_sm100  # noqa: F401  (registers the tcgen05 convolution bac
 from .refine import refine_depth  # noqa: F401
 from .nets2d import encode_features  # noqa: F401
 from .frozen import FrozenMVSNet  # noqa: F401
+from .ops import depth_confidence  # noqa: F401
+from .fusion import fuse_depth_maps, infer_scene, write_ply  # noqa: F401
 
 __all__ = ["homography_warping", "assemble_cost_volume", "extract_depth_map", "CostVolumeReg",
            "WarpedFeatureVolumes", "PlaneSweep", "warp_variance", "warp_materialize", "softmax_depth",
-           "softmax_over_depth", "depth_from_prob", "refine_depth", "encode_features", "FrozenMVSNet", "MvsB200Error", "launch_count", "load_library"]
+           "softmax_over_depth", "depth_from_prob", "refine_depth", "encode_features", "FrozenMVSNet", "depth_confidence",
+           "fuse_depth_maps", "infer_scene", "write_ply", "MvsB200Error", "launch_count", "load_library"]

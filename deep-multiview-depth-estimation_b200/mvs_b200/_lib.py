@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("MVSB200_LIB") or os.path.normpath(os.path.join(_HERE,
 ABI_VERSION = 1
 F32, BF16 = 0, 1
 VIEW_PARAM_FLOATS = 16
+FUSION_CAM_FLOATS, FUSION_BLOCK_PIXELS, FUSION_MAX_SOURCES = 32, 128, 16     # MVSB200_FUSION_* of include/mvs_b200.h
 
 _c = ctypes
 _P, _I = _c.c_void_p, _c.c_int
@@ -28,6 +29,8 @@ _SIGNATURES = {
     "mvsb200_warp_variance_bwd": (_I, [_P, _P, _P, _P, _I, _P, _I, _I, _I, _I, _I, _I, _P]),
     "mvsb200_warp_materialize": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "mvsb200_softmax_depth_fwd": (_I, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "mvsb200_softmax_depth_conf_fwd": (_I, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "mvsb200_depth_confidence": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "mvsb200_depth_from_ranks": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "mvsb200_depth_bwd": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "mvsb200_softmax_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P]),
@@ -84,6 +87,9 @@ _SIGNATURES = {
     "mvsb200_bn_relu_add_apply": (_I, [_P, _I, _P, _P, _P, _P, _I, _c.c_int64, _I, _P, _P]),
     "mvsb200_bn_relu_bwd_crop": (_I, [_P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _c.c_int64, _I, _P, _P]),
     "mvsb200_bn_relu_bwd": (_I, [_P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _c.c_int64, _I, _P]),
+    "mvsb200_fusion_check": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _c.c_float, _c.c_float, _c.c_float, _I, _P, _P, _P, _P, _P]),
+    "mvsb200_fusion_emit": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
+    "mvsb200_resize_rgb": (_I, [_P, _I, _I, _I, _I, _I, _P, _P]),
 }
 
 _lib = None

@@ -147,9 +147,11 @@ class FrozenMVSNet:
         return self.forward(*args, **kwargs)
 
     @torch.no_grad()
-    def forward(self, nn_input, K_batch, R_batch, T_batch, d_min, d_int, batch_size, n_views, sweep=None):
+    def forward(self, nn_input, K_batch, R_batch, T_batch, d_min, d_int, batch_size, n_views, sweep=None, return_confidence=False):
         """MVSNet.forward (model.py:168-207) -> (initial, refined) depth maps fp32 [B, 1, H/4, W/4].  sweep: an ops.PlaneSweep
-        already holding this batch's geometry on the device, as in harness.MVSNet.forward."""
+        already holding this batch's geometry on the device, as in harness.MVSNet.forward.  return_confidence: also return
+        the photometric confidence of the initial depth map (ops.depth_confidence) -> (initial, refined, confidence); the
+        depth-axis softmax, depth and confidence then run as one launch, and initial and refined stay bit-identical."""
         if not nn_input.is_cuda:
             _fail(f"the input images live on {nn_input.device}; mvs_b200 has no CPU path")
         if nn_input.dtype != torch.float32 or nn_input.dim() != 4 or nn_input.shape[1] != 3:
@@ -163,10 +165,15 @@ class FrozenMVSNet:
             ev.record()
         warped, d_batch, _ = api.homography_warping(K_batch, R_batch, T_batch, d_min, d_int, feats, batch_size, n_views, self.d_num,
                                                     self.d_scale, sweep=sweep)
-        prob = self.regularise(api.assemble_cost_volume(warped, n_views, torch.bfloat16))
-        initial = api.extract_depth_map(prob, d_batch, self.n_depth_est)
+        cost = api.assemble_cost_volume(warped, n_views, torch.bfloat16)
+        conf = None
+        if return_confidence:
+            _, _, initial, conf = ops.softmax_depth_confidence(self.logits(cost), d_batch, self.n_depth_est)
+        else:
+            initial = api.extract_depth_map(self.regularise(cost), d_batch, self.n_depth_est)
         dev = initial.device
-        return initial, self.refine(initial, nn_input, n_views, d_min.to(dev), d_int.to(dev) * self.d_num * self.d_scale)
+        refined = self.refine(initial, nn_input, n_views, d_min.to(dev), d_int.to(dev) * self.d_num * self.d_scale)
+        return (initial, refined) if conf is None else (initial, refined, conf)
 
     # ------------------------------------------------------------------------------------------------------------------
     def _conv2d(self, x, wname, cy, bn=None):

@@ -294,6 +294,38 @@ def softmax_depth(logits: torch.Tensor, d_batch: torch.Tensor, n_est: int = 5):
     return prob.view(B, 1, D, h, w), depth.view(B, 1, h, w)
 
 
+def softmax_depth_confidence(logits: torch.Tensor, d_batch: torch.Tensor, n_est: int = 5):
+    """Fused forward (one launch): logits [B,1,D,h,w] -> (prob, ranks, depth, conf).  prob, ranks and depth are bit-identical to
+    softmax_over_depth + depth_from_prob; conf [B,1,h,w] is the confidence of depth_confidence.  Inference only; no autograd."""
+    _need_cuda(logits, "logits")
+    x, (B, D, h, w) = _as_bdhw(logits.detach().float())
+    depths = d_batch.detach().to(device=x.device, dtype=torch.float32).reshape(B, D).contiguous()
+    prob = torch.empty_like(x)
+    ranks = torch.empty((B, min(int(n_est), D), h, w), dtype=torch.int32, device=x.device)
+    depth = torch.empty((B, h, w), dtype=torch.float32, device=x.device)
+    conf = torch.empty_like(depth)
+    with _timed("softmax_depth_conf_fwd"):
+        _lib.call("mvsb200_softmax_depth_conf_fwd", x.data_ptr(), 1, depths.data_ptr(), prob.data_ptr(), ranks.data_ptr(),
+                  depth.data_ptr(), conf.data_ptr(), B, D, h, w, int(n_est), _stream())
+    return prob.view(B, 1, D, h, w), ranks, depth.view(B, 1, h, w), conf.view(B, 1, h, w)
+
+
+def depth_confidence(prob: torch.Tensor, depth: torch.Tensor, d_batch: torch.Tensor) -> torch.Tensor:
+    """MVSNet's photometric confidence of an existing probability volume prob [B,1,D,h,w] and depth map [B,1,h,w]: the
+    probability mass of the planes k0-1 .. k0+2 (clipped to the sweep) with k0 = floor((depth - d_0) / (d_1 - d_0)), summed in
+    ascending order in fp32 -> [B,1,h,w].  1 when D = 1; NaN where the depth or a summed probability is not finite.  No autograd."""
+    _need_cuda(prob, "prob_volume")
+    p, (B, D, h, w) = _as_bdhw(prob.detach().float())
+    if depth.shape != (B, 1, h, w):
+        raise _lib.MvsB200Error(f"depth_confidence: depth map [{B}, 1, {h}, {w}] expected, got {tuple(depth.shape)}")
+    dep = depth.detach().to(device=p.device, dtype=torch.float32).contiguous()
+    depths = d_batch.detach().to(device=p.device, dtype=torch.float32).reshape(B, D).contiguous()
+    conf = torch.empty((B, 1, h, w), dtype=torch.float32, device=p.device)
+    with _timed("depth_confidence"):
+        _lib.call("mvsb200_depth_confidence", p.data_ptr(), dep.data_ptr(), depths.data_ptr(), conf.data_ptr(), B, D, h, w, _stream())
+    return conf
+
+
 # --------------------------------------------------------------------------------------------------
 # K3b: train-mode BatchNorm3d + ReLU on channel-last volumes
 # --------------------------------------------------------------------------------------------------

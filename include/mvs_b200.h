@@ -100,6 +100,19 @@ int mvsb200_softmax_depth_fwd(const float* in, int apply_softmax, const float* d
                               float* prob, int32_t* ranks, float* depth,
                               int B, int D, int h, int w, int n_est, void* stream);
 
+/* mvsb200_softmax_depth_fwd that also writes conf [B, h, w] (required, as are depths and depth): MVSNet's photometric
+ * confidence, the probability mass of the planes k0-1 .. k0+2 (clipped to [0, D-1]) where k0 = floor((depth - d_0) / (d_1 - d_0)),
+ * summed in ascending k in fp32; 1 when D == 1; NaN for a non-finite depth or summed probability.  prob, ranks and depth are
+ * bit-identical to mvsb200_softmax_depth_fwd. */
+int mvsb200_softmax_depth_conf_fwd(const float* in, int apply_softmax, const float* depths,
+                                   float* prob, int32_t* ranks, float* depth, float* conf,
+                                   int B, int D, int h, int w, int n_est, void* stream);
+
+/* the same confidence from a probability volume prob [B, D, h, w] and depth map [B, h, w] that already exist; bit-identical to the
+ * conf of mvsb200_softmax_depth_conf_fwd on the same values */
+int mvsb200_depth_confidence(const float* prob, const float* depth, const float* depths, float* conf,
+                             int B, int D, int h, int w, void* stream);
+
 /* depth from precomputed ranks (the cheap second half when softmax ran earlier, in CostVolumeReg) */
 int mvsb200_depth_from_ranks(const float* prob, const int32_t* ranks, const float* depths, float* depth,
                              int B, int D, int h, int w, int n_keep, void* stream);
@@ -425,6 +438,30 @@ int mvsb200_image_to_rows8(const float* images, const int64_t* strides4_host, in
 int mvsb200_s2d_rows_bf16(const void* src, void* dst, int N, int h, int w, int C, int inverse, void* stream);
 int mvsb200_conv3d_s1_wgrad_ex(const void* x, const void* gy, float* gw, int B, int Di, int Hi, int Wi, int Cin, int Do, int Ho,
                                int Wo, int cout, int off_d, int off_h, int off_w, unsigned kd_mask, void* stream);
+
+/* ---- K7: multi-view consistency filter and point-cloud fusion (MVSNet §4.2) -----------------------------------------------------
+ * N depth maps [N, h, w] of one scene, their confidences, and a camera table cams [N, MVSB200_FUSION_CAM_FLOATS] fp32 per view:
+ *   [0:12] P = K [R | T] (3x4, row-major)  [12:21] R^T K^-1  [21:24] C = -R^T T  [24:27] n, the depth normal  [27:32] unused.
+ * Depth d at pixel (x, y) is the point X = C + d / (n^T r) r with r = R^T K^-1 (x, y, 1); the depth of X in view j is n_j^T (X - C_j).
+ * sources [N, S] int32 (S <= 16, -1 = padding).  A pixel is valid when conf >= conf_min and d is finite and > 0; a source s is
+ * consistent when X projects into s with z > 0 inside [0, w-1] x [0, h-1], the four bilinear taps of d_s there are finite and > 0,
+ * and the point X_s (the sampled depth unprojected in s) projects back to p' with |p' - p| < reproj_px and
+ * |n_ref^T (X_s - C_ref) - d| / d < rel_depth.  mask = valid && count >= min_views, fused = (d + sum of reprojected depths) /
+ * (1 + count).  block_counts [N * ceil(h w / MVSB200_FUSION_BLOCK_PIXELS)]: the masked pixels of each block (view-major). */
+#define MVSB200_FUSION_CAM_FLOATS 32
+#define MVSB200_FUSION_BLOCK_PIXELS 128
+#define MVSB200_FUSION_MAX_SOURCES 16
+int mvsb200_fusion_check(const float* depth, const float* conf, const float* cams, const int32_t* sources, int N, int S,
+                         int h, int w, float conf_min, float reproj_px, float rel_depth, int min_views,
+                         uint8_t* mask, int32_t* count, float* fused, int32_t* block_counts, void* stream);
+
+/* compaction: offsets [N * blocks] int64, the exclusive scan of block_counts.  Writes xyz [M, 3] (the fused depth unprojected at the
+ * reference pixel) and rgb [M, 3] (colours [N, 3, h, w] at that pixel) in view-major, row-major order; deterministic, no atomics. */
+int mvsb200_fusion_emit(const uint8_t* mask, const float* fused, const float* colours, const float* cams, const int64_t* offsets,
+                        int N, int h, int w, float* xyz, float* rgb, void* stream);
+
+/* images [N, 3, H, W] fp32 contiguous -> out [N, 3, h, w]: torch's bilinear resize with align_corners = False (as refine_input) */
+int mvsb200_resize_rgb(const float* images, int N, int H, int W, int h, int w, float* out, void* stream);
 
 #ifdef __cplusplus
 }
