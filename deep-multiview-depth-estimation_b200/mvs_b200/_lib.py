@@ -13,6 +13,7 @@ ABI_VERSION = 1
 F32, BF16 = 0, 1
 VIEW_PARAM_FLOATS = 16
 FUSION_CAM_FLOATS, FUSION_BLOCK_PIXELS, FUSION_MAX_SOURCES = 32, 128, 16     # MVSB200_FUSION_* of include/mvs_b200.h
+PC_MAX_CELLS = 1 << 28                                                       # MVSB200_PC_MAX_CELLS
 
 _c = ctypes
 _P, _I = _c.c_void_p, _c.c_int
@@ -90,6 +91,11 @@ _SIGNATURES = {
     "mvsb200_fusion_check": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _c.c_float, _c.c_float, _c.c_float, _I, _P, _P, _P, _P, _P]),
     "mvsb200_fusion_emit": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "mvsb200_resize_rgb": (_I, [_P, _I, _I, _I, _I, _I, _P, _P]),
+    "mvsb200_pc_grid_keys": (_I, [_P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _P, _P]),
+    "mvsb200_pc_grid_cells": (_I, [_P, _P, _P, _I, _P, _P, _P, _P]),
+    "mvsb200_pc_nearest": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _P, _P]),
+    "mvsb200_pc_thin_neighbours": (_I, [_P, _P, _P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_double, _P, _P, _P, _P]),
+    "mvsb200_pc_thin_round": (_I, [_P, _P, _P, _P, _I, _P, _P]),
 }
 
 _lib = None

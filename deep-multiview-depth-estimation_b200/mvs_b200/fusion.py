@@ -221,3 +221,71 @@ def write_ply(path, xyz, rgb=None):
     with open(path, "wb") as f:
         f.write(header.encode("ascii"))
         f.write(rec.tobytes())
+
+
+_PLY_TYPES = {"char": "i1", "int8": "i1", "uchar": "u1", "uint8": "u1", "short": "i2", "int16": "i2", "ushort": "u2", "uint16": "u2",
+              "int": "i4", "int32": "i4", "uint": "u4", "uint32": "u4", "float": "f4", "float32": "f4", "double": "f8", "float64": "f8"}
+
+
+def read_ply(path):
+    """The vertex element of a PLY file (binary little-endian or ASCII) -> (xyz fp32 [n, 3], rgb uint8 [n, 3] or None), CPU tensors.
+    Scalar properties of any PLY type are read; x, y, z become fp32 and red, green, blue uint8 (as stored by write_ply, whose output
+    reads back bit for bit); other scalar properties are skipped.  Refused with MvsB200Error: big-endian files, list properties in
+    the vertex element (or in an element before it), and a missing x, y or z."""
+    with open(path, "rb") as f:
+        raw = f.read()
+    end = raw.find(b"end_header")
+    if not raw.startswith(b"ply") or end < 0:
+        _fail(f"read_ply: {path} is not a PLY file")
+    body_at = raw.index(b"\n", end) + 1
+    fmt, elements = None, []
+    for line in raw[:end].decode("ascii", errors="replace").splitlines()[1:]:
+        tok = line.split()
+        if not tok or tok[0] in ("comment", "obj_info"):
+            continue
+        if tok[0] == "format":
+            fmt = tok[1]
+        elif tok[0] == "element":
+            elements.append((tok[1], int(tok[2]), []))
+        elif tok[0] == "property":
+            if not elements:
+                _fail(f"read_ply: {path}: property before any element")
+            if tok[1] == "list":
+                elements[-1][2].append((tok[-1], None))
+            elif tok[1] in _PLY_TYPES:
+                elements[-1][2].append((tok[2], _PLY_TYPES[tok[1]]))
+            else:
+                _fail(f"read_ply: {path}: unknown property type {tok[1]!r}")
+    if fmt == "binary_big_endian":
+        _fail(f"read_ply: {path}: big-endian PLY files are not supported")
+    if fmt not in ("binary_little_endian", "ascii"):
+        _fail(f"read_ply: {path}: unknown format {fmt!r}")
+    names = [e[0] for e in elements]
+    if "vertex" not in names:
+        _fail(f"read_ply: {path} has no vertex element")
+    vi = names.index("vertex")
+    for name, count, props in elements[:vi + 1]:
+        if any(t is None for _, t in props):
+            _fail(f"read_ply: {path}: list property in the element {name!r} (only scalar properties can be read)")
+    _, n, props = elements[vi]
+    pnames = [p for p, _ in props]
+    for c in "xyz":
+        if c not in pnames:
+            _fail(f"read_ply: {path}: the vertex element has no property {c!r}")
+    if fmt == "ascii":
+        lines = raw[body_at:].decode("ascii").splitlines()
+        skip = sum(c for _, c, _ in elements[:vi])
+        rows = [l.split() for l in lines[skip:skip + n]]
+        if len(rows) != n or any(len(r) != len(props) for r in rows):
+            _fail(f"read_ply: {path}: {n} vertex lines of {len(props)} values expected")
+        cols = {p: np.array([r[k] for r in rows], dtype=np.float64 if t[0] == "f" else np.int64).astype(t)
+                for k, (p, t) in enumerate(props)}
+    else:
+        at = body_at + sum(c * sum(np.dtype("<" + t).itemsize for _, t in pr) for _, c, pr in elements[:vi])
+        rec = np.frombuffer(raw, dtype=[(p, "<" + t) for p, t in props], count=n, offset=at)
+        cols = {p: rec[p] for p in pnames}
+    xyz = torch.from_numpy(np.stack([cols[c] for c in "xyz"], 1).astype(np.float32))
+    rgb = None
+    if all(c in cols for c in ("red", "green", "blue")):
+        rgb = torch.from_numpy(np.stack([cols[c] for c in ("red", "green", "blue")], 1).astype(np.uint8))
+    return xyz, rgb

@@ -463,6 +463,41 @@ int mvsb200_fusion_emit(const uint8_t* mask, const float* fused, const float* co
 /* images [N, 3, H, W] fp32 contiguous -> out [N, 3, h, w]: torch's bilinear resize with align_corners = False (as refine_input) */
 int mvsb200_resize_rgb(const float* images, int N, int H, int W, int h, int w, float* out, void* stream);
 
+/* ---- K8: point-cloud evaluation (the DTU protocol: accuracy / completeness) -----------------------------------------------------
+ * Uniform grid over a cloud of m points [m, 3] fp32: fine cells of edge `cell` from the origin (ox, oy, oz), grouped in coarse
+ * blocks of 8 x 8 x 8 cells, nbx x nby x nbz blocks (8 nb fine cells per axis, at most MVSB200_PC_MAX_CELLS cells in all).  The
+ * cell of a point is floor((x - o) / cell) per axis in fp64, clamped to the grid; its key is block-major,
+ *   key = ((bz nby + by) nbx + bx) 512 + (lz 8 + ly) 8 + lx,   (bx, lx) = (ix / 8, ix % 8), ...
+ * grid_keys writes keys [m] int32.  After a stable sort of the keys (sorted_keys, perm [m] int64), grid_cells writes pts [m, 4]
+ * fp32 (x, y, z, the original index as int32 bits), cells [8^3 nbx nby nbz][2] and blocks [nbx nby nbz][2] int32 {begin, end} into
+ * pts: cells and blocks must be ZEROED by the caller (an untouched entry is empty).  Every entry is written by one thread. */
+#define MVSB200_PC_MAX_CELLS (1 << 28)
+int mvsb200_pc_grid_keys(const float* xyz, int n, float ox, float oy, float oz, float cell, int nbx, int nby, int nbz,
+                         int32_t* keys, void* stream);
+int mvsb200_pc_grid_cells(const float* xyz, const int32_t* sorted_keys, const int64_t* perm, int n, float* pts,
+                          int32_t* cells, int32_t* blocks, void* stream);
+
+/* Exact nearest distance, capped: dist[i] = min_j |query_i - pts_j| (fp32) when that is < max_dist, +inf otherwise, for n queries
+ * [n, 3] against a grid built as above.  Search: shells of fine cells, then shells of coarse blocks (empty ones skipped) while a
+ * lower bound on the distance to the rest, minus `slack`, is below the best distance so far and below max_dist.  slack: at least
+ * the fp32 rounding of the grid's cell faces (the host passes 1e-5 cell + 2.4e-7 max |coordinate|).  Deterministic. */
+int mvsb200_pc_nearest(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
+                       float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, float* dist,
+                       void* stream);
+
+/* Greedy minimum-distance thinning (reducePts_haa for a given visiting order) as parallel rounds, on a grid with cell >= dst built
+ * over the cloud itself.  rank_sorted [m] int32: the position in the visiting order of each sorted point.  offsets == NULL: counts
+ * [m] = the number of points of lower rank within dst (|p - q| <= dst in fp64 on the fp32 coordinates); otherwise list[offsets[s]
+ * ...] = their sorted positions (offsets [m + 1] int64, the exclusive scan of counts), in a fixed scan order. */
+int mvsb200_pc_thin_neighbours(const float* pts, const int32_t* cells, const int32_t* rank_sorted, int n, float ox, float oy,
+                               float oz, float cell, int nbx, int nby, int nbz, double dst, const int64_t* offsets,
+                               int32_t* counts, int32_t* list, void* stream);
+/* One round.  state: 0 undecided, 1 kept, 2 removed (per sorted point).  An undecided point becomes kept when every neighbour in
+ * its list is removed, removed when one is kept; decided points are copied.  Reads state_in, writes state_out (distinct buffers)
+ * and ADDS the number of points still undecided to *undecided.  The fixed point is the sequential greedy set of that order. */
+int mvsb200_pc_thin_round(const int64_t* offsets, const int32_t* list, const uint8_t* state_in, uint8_t* state_out, int n,
+                          int32_t* undecided, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
