@@ -8,6 +8,9 @@
 //   fusion_check_kernel   one thread per reference pixel, grid row = reference view: the photometric test, then every source
 //                         in table order (project, bilinear depth sample, unproject there, project back), the consistent count
 //                         and fused depth; also the number of kept pixels of its block (one __syncthreads_count)
+//     <VIS = true>        visibility fusion: one launch per reference view `ref`, in the caller's view order.  A pixel already
+//                         marked in used[ref] is no reference (mask 0, count 0, fused = d, as an invalid pixel); a kept pixel
+//                         marks, in every consistent source j, the pixel nearest its projection there: used[j, round(v), round(u)]
 //   fusion_emit_kernel    same grid: the block's offset (exclusive scan of the block counts, computed on the host side with
 //                         torch.cumsum) plus the rank of the pixel among the kept pixels of the block (ballots) -> xyz, rgb.
 //                         View-major, row-major output; no atomics, so two runs write the same point cloud bit for bit.
@@ -50,14 +53,20 @@ __device__ __forceinline__ float depth_in(const float* c, F3 X) {
 
 __device__ __forceinline__ bool usable(float d) { return isfinite(d) && d > 0.f; }
 
+template <bool VIS>
 __global__ void __launch_bounds__(kBlk) fusion_check_kernel(const float* __restrict__ depth, const float* __restrict__ conf,
                                                            const float* __restrict__ cams, const int32_t* __restrict__ sources,
                                                            int S, int h, int w, float conf_min, float reproj_px, float rel_depth,
                                                            int min_views, uint8_t* __restrict__ mask, int32_t* __restrict__ count,
-                                                           float* __restrict__ fused, int32_t* __restrict__ block_counts) {
+                                                           float* __restrict__ fused, int32_t* __restrict__ block_counts,
+                                                           int vis_ref, uint8_t* __restrict__ used) {
     __shared__ float cam_s[(1 + kMaxSrc) * kCam];   // [0]: the reference view, [1 + s]: source s
     __shared__ int src_s[kMaxSrc];
-    const int ref = blockIdx.y, hw = h * w, pix = blockIdx.x * kBlk + threadIdx.x;
+    // VIS: per source, the index of the source pixel nearest to where the test projected this thread's pixel.  Staged here from
+    // the same fp32 (u, v) the test used, so the mark can never disagree with the decision (a recomputed projection could be
+    // contracted differently by the compiler).
+    __shared__ int mark_s[VIS ? kMaxSrc * kBlk : 1];
+    const int ref = VIS ? vis_ref : (int)blockIdx.y, hw = h * w, pix = blockIdx.x * kBlk + threadIdx.x;
     if (threadIdx.x < S) src_s[threadIdx.x] = sources[(size_t)ref * S + threadIdx.x];
     __syncthreads();
     for (int i = threadIdx.x; i < (1 + S) * kCam; i += kBlk) {
@@ -71,8 +80,10 @@ __global__ void __launch_bounds__(kBlk) fusion_check_kernel(const float* __restr
         const size_t at = (size_t)ref * hw + pix;
         const float d = depth[at];
         const float fx = (float)(pix % w), fy = (float)(pix / w);
-        const bool valid = conf[at] >= conf_min && usable(d);     // a NaN confidence fails the comparison
+        bool valid = conf[at] >= conf_min && usable(d);           // a NaN confidence fails the comparison
+        if constexpr (VIS) valid = valid && !used[at];           // another view's point has absorbed this pixel
         int cnt = 0;
+        unsigned consistent = 0;                                 // VIS: bit s = source s was consistent
         float sum = d;
         if (valid) {
             const F3 X = unproject(cam_s, fx, fy, d);
@@ -99,6 +110,12 @@ __global__ void __launch_bounds__(kBlk) fusion_check_kernel(const float* __restr
                 if (ex * ex + ey * ey < reproj_px * reproj_px && fabsf(dr - d) < rel_depth * d) {
                     ++cnt;
                     sum += dr;
+                    if constexpr (VIS) {
+                        // floor(u + 1/2) = x0 + (u - x0 >= 1/2), and u - x0 is exact in fp32 (Sterbenz): this rounds the test's own
+                        // u with no further rounding.  x0 = w - 1 implies u = w - 1, so the index stays inside the map
+                        consistent |= 1u << s;
+                        mark_s[s * kBlk + threadIdx.x] = (y0 + (ay >= 0.5f)) * w + x0 + (ax >= 0.5f);
+                    }
                 }
             }
         }
@@ -106,6 +123,15 @@ __global__ void __launch_bounds__(kBlk) fusion_check_kernel(const float* __restr
         mask[at] = keep;
         count[at] = cnt;
         fused[at] = sum / (float)(1 + cnt);
+        if constexpr (VIS) {
+            // several threads may store the same 1 to one byte; no launch writes the used[] slice it reads (the host refuses a
+            // view among its own sources), and launches of successive views are ordered on the stream
+            if (keep)
+                for (unsigned b = consistent; b; b &= b - 1) {
+                    const int s = __ffs(b) - 1;
+                    used[(size_t)src_s[s] * hw + mark_s[s * kBlk + threadIdx.x]] = 1;
+                }
+        }
     }
     const int kept = __syncthreads_count(keep);
     if (threadIdx.x == 0) block_counts[(size_t)ref * gridDim.x + blockIdx.x] = kept;
@@ -157,9 +183,27 @@ extern "C" int mvsb200_fusion_check(const float* depth, const float* conf, const
     MVS_REQUIRE(N >= 1 && N <= 65535 && h >= 1 && w >= 1 && (long long)h * w < (1LL << 30), "fusion_check: bad shape");
     MVS_REQUIRE(S >= 0 && S <= kMaxSrc, "fusion_check: 0 <= S <= %d sources per view", kMaxSrc);
     dim3 grid((h * w + kBlk - 1) / kBlk, N);
-    fusion_check_kernel<<<grid, kBlk, 0, (cudaStream_t)stream>>>(depth, conf, cams, sources, S, h, w, conf_min, reproj_px, rel_depth,
-                                                                 min_views, mask, count, fused, block_counts);
+    fusion_check_kernel<false><<<grid, kBlk, 0, (cudaStream_t)stream>>>(depth, conf, cams, sources, S, h, w, conf_min, reproj_px,
+                                                                        rel_depth, min_views, mask, count, fused, block_counts, 0,
+                                                                        nullptr);
     MVS_CHECK_LAUNCH("fusion_check");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_fusion_visibility(const float* depth, const float* conf, const float* cams, const int32_t* sources, int N,
+                                         int S, int h, int w, float conf_min, float reproj_px, float rel_depth, int min_views, int ref,
+                                         uint8_t* used, uint8_t* mask, int32_t* count, float* fused, int32_t* block_counts,
+                                         void* stream) {
+    MVS_REQUIRE(depth && conf && cams && used && mask && count && fused && block_counts, "fusion_visibility: null pointer");
+    MVS_REQUIRE(S == 0 || sources, "fusion_visibility: null source table");
+    MVS_REQUIRE(N >= 1 && N <= 65535 && h >= 1 && w >= 1 && (long long)h * w < (1LL << 30), "fusion_visibility: bad shape");
+    MVS_REQUIRE(S >= 0 && S <= kMaxSrc, "fusion_visibility: 0 <= S <= %d sources per view", kMaxSrc);
+    MVS_REQUIRE(ref >= 0 && ref < N, "fusion_visibility: reference view %d outside [0, %d)", ref, N);
+    dim3 grid((h * w + kBlk - 1) / kBlk, 1);
+    fusion_check_kernel<true><<<grid, kBlk, 0, (cudaStream_t)stream>>>(depth, conf, cams, sources, S, h, w, conf_min, reproj_px,
+                                                                       rel_depth, min_views, mask, count, fused, block_counts, ref,
+                                                                       used);
+    MVS_CHECK_LAUNCH("fusion_visibility");
     return MVSB200_OK;
 }
 

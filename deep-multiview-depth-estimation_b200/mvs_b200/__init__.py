@@ -15,11 +15,11 @@ from .refine import refine_depth  # noqa: F401
 from .nets2d import encode_features  # noqa: F401
 from .frozen import FrozenMVSNet  # noqa: F401
 from .ops import depth_confidence  # noqa: F401
-from .fusion import fuse_depth_maps, infer_scene, write_ply, read_ply  # noqa: F401
+from .fusion import fuse_depth_maps, visibility_fusion, infer_scene, write_ply, read_ply  # noqa: F401
 from .evaluation import thin_points, nearest_distance, evaluate_point_cloud, load_dtu_eval  # noqa: F401
 
 __all__ = ["homography_warping", "assemble_cost_volume", "extract_depth_map", "CostVolumeReg",
            "WarpedFeatureVolumes", "PlaneSweep", "warp_variance", "warp_materialize", "softmax_depth",
            "softmax_over_depth", "depth_from_prob", "refine_depth", "encode_features", "FrozenMVSNet", "depth_confidence",
-           "fuse_depth_maps", "infer_scene", "write_ply", "read_ply", "thin_points", "nearest_distance",
+           "fuse_depth_maps", "visibility_fusion", "infer_scene", "write_ply", "read_ply", "thin_points", "nearest_distance",
            "evaluate_point_cloud", "load_dtu_eval", "MvsB200Error", "launch_count", "load_library"]

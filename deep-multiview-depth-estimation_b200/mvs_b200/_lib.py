@@ -89,6 +89,8 @@ _SIGNATURES = {
     "mvsb200_bn_relu_bwd_crop": (_I, [_P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _c.c_int64, _I, _P, _P]),
     "mvsb200_bn_relu_bwd": (_I, [_P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _c.c_int64, _I, _P]),
     "mvsb200_fusion_check": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _c.c_float, _c.c_float, _c.c_float, _I, _P, _P, _P, _P, _P]),
+    "mvsb200_fusion_visibility": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _c.c_float, _c.c_float, _c.c_float, _I, _I, _P, _P, _P, _P, _P,
+                                       _P]),
     "mvsb200_fusion_emit": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
     "mvsb200_resize_rgb": (_I, [_P, _I, _I, _I, _I, _I, _P, _P]),
     "mvsb200_pc_grid_keys": (_I, [_P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _P, _P]),

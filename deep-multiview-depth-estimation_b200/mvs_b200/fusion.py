@@ -2,7 +2,7 @@
 (MVSNet, Yao et al. 2018, §4.2) on the library's kernels (csrc/fusion.cu, the confidence in csrc/softmax_depth.cu).
 
     depth, conf, colours = infer_scene(FrozenMVSNet(model), images, K, R, T, d_min, d_int, pairs)
-    xyz, rgb, masks = fuse_depth_maps(depth, conf, colours, K, R, T, sources)
+    xyz, rgb, masks = fuse_depth_maps(depth, conf, colours, K, R, T, sources)      # or visibility_fusion: each point once
     write_ply("scene.ply", xyz, rgb)
 
 What a depth means.  The network sweeps the planes n^T (X - C_ref) = d with n = R_ref[:, 2], the third COLUMN of R (geometry.py,
@@ -78,7 +78,8 @@ def _maps(t, N, c, h, w, what):
     return t.detach().float().contiguous()
 
 
-def _check(depth, conf, K, R, T, sources, normal, conf_min, reproj_px, rel_depth, min_views):
+def _prepare(depth, conf, K, R, T, sources, normal):
+    """The inputs of the check on the device and its outputs (uninitialised): d, c, cams, source table, mask, count, fused, blocks."""
     if not isinstance(depth, torch.Tensor) or not depth.is_cuda:
         _fail("depth must be a CUDA tensor; mvs_b200 has no CPU path")
     if depth.dim() != 4 or depth.shape[1] != 1:
@@ -97,11 +98,32 @@ def _check(depth, conf, K, R, T, sources, normal, conf_min, reproj_px, rel_depth
     count = torch.empty((N, 1, h, w), dtype=torch.int32, device=dev)
     fused = torch.empty((N, 1, h, w), dtype=torch.float32, device=dev)
     blocks = torch.empty((N * -(-h * w // _lib.FUSION_BLOCK_PIXELS),), dtype=torch.int32, device=dev)
+    return d, c, cams, src, mask, count, fused, blocks
+
+
+def _check(depth, conf, K, R, T, sources, normal, conf_min, reproj_px, rel_depth, min_views):
+    d, c, cams, src, mask, count, fused, blocks = _prepare(depth, conf, K, R, T, sources, normal)
+    N, _, h, w = depth.shape
     with _timed("fusion_check"):
-        _lib.call("mvsb200_fusion_check", d.data_ptr(), c.data_ptr(), cams.data_ptr(), src.data_ptr(), N, S, h, w, float(conf_min),
-                  float(reproj_px), float(rel_depth), int(min_views), mask.data_ptr(), count.data_ptr(), fused.data_ptr(),
-                  blocks.data_ptr(), _stream())
+        _lib.call("mvsb200_fusion_check", d.data_ptr(), c.data_ptr(), cams.data_ptr(), src.data_ptr(), N, src.shape[1], h, w,
+                  float(conf_min), float(reproj_px), float(rel_depth), int(min_views), mask.data_ptr(), count.data_ptr(),
+                  fused.data_ptr(), blocks.data_ptr(), _stream())
     return mask, count, fused, blocks, cams
+
+
+def _emit(mask, fused, blocks, cams, colours):
+    """The kept pixels of every view -> (xyz, rgb), view-major, row-major; the one device-to-host read is the point count."""
+    N, _, h, w = mask.shape
+    col = _maps(colours, N, 3, h, w, "colours")
+    offsets = torch.cumsum(blocks, 0) - blocks                    # exclusive scan, int64
+    M = int(offsets[-1] + blocks[-1]) if blocks.numel() else 0
+    xyz = torch.empty((M, 3), dtype=torch.float32, device=mask.device)
+    rgb = torch.empty((M, 3), dtype=torch.float32, device=mask.device)
+    if M:
+        with _timed("fusion_emit"):
+            _lib.call("mvsb200_fusion_emit", mask.data_ptr(), fused.data_ptr(), col.data_ptr(), cams.data_ptr(), offsets.data_ptr(),
+                      N, h, w, xyz.data_ptr(), rgb.data_ptr(), _stream())
+    return xyz, rgb
 
 
 def check_consistency(depth, conf, K, R, T, sources, *, normal="sweep", conf_min=CONF_MIN, reproj_px=REPROJ_PX,
@@ -125,16 +147,55 @@ def fuse_depth_maps(depth, conf, colours, K, R, T, sources, *, normal="sweep", c
     point is the fused depth unprojected at the reference pixel, its colour the colours of that pixel.  Points come view-major,
     row-major; two calls on the same inputs return the same bits."""
     mask, count, fused, blocks, cams = _check(depth, conf, K, R, T, sources, normal, conf_min, reproj_px, rel_depth, min_views)
-    N, _, h, w = depth.shape
-    col = _maps(colours, N, 3, h, w, "colours")
-    offsets = torch.cumsum(blocks, 0) - blocks                    # exclusive scan, int64
-    M = int(offsets[-1] + blocks[-1]) if blocks.numel() else 0
-    xyz = torch.empty((M, 3), dtype=torch.float32, device=depth.device)
-    rgb = torch.empty((M, 3), dtype=torch.float32, device=depth.device)
-    if M:
-        with _timed("fusion_emit"):
-            _lib.call("mvsb200_fusion_emit", mask.data_ptr(), fused.data_ptr(), col.data_ptr(), cams.data_ptr(), offsets.data_ptr(),
-                      N, h, w, xyz.data_ptr(), rgb.data_ptr(), _stream())
+    xyz, rgb = _emit(mask, fused, blocks, cams, colours)
+    return xyz, rgb, mask.bool()
+
+
+def _view_order(order, N):
+    if order is None:
+        return list(range(N))
+    if isinstance(order, torch.Tensor):
+        order = order.detach().cpu().numpy()
+    a = np.asarray(order)
+    if a.ndim != 1 or a.dtype.kind not in "iu" or not np.array_equal(np.sort(a), np.arange(N)):
+        _fail(f"visibility_fusion: order must be a permutation of range({N}), got {a.tolist()}")
+    return [int(i) for i in a]
+
+
+def visibility_fusion(depth, conf, colours, K, R, T, sources, *, order=None, normal="sweep", conf_min=CONF_MIN, reproj_px=REPROJ_PX,
+                      rel_depth=REL_DEPTH, min_views=MIN_VIEWS):
+    """fuse_depth_maps with visibility-based suppression: each surface point is emitted once, by the first view in `order` that
+    keeps it, instead of once per view that sees it -> (xyz fp32 [M, 3], rgb fp32 [M, 3], masks bool [N, 1, h, w]).
+
+    Inputs, thresholds and conventions are those of fuse_depth_maps; order is a permutation of range(N) (default: index order).
+    A state used [N, h, w] starts all false, and the views are checked one after another in `order`.  In reference view r a pixel
+    with used[r] set is not a reference (its mask is false: another view's point has absorbed it); every other pixel runs
+    fuse_depth_maps' test unchanged, and when it is kept, each consistent source j gets the pixel nearest the point's projection
+    there marked, used[j, floor(v + 1/2), floor(u + 1/2)] = true.  A marked pixel still serves as a source's depth sample for later
+    references; it only stops being a reference itself.  The points are fuse_depth_maps' points of the kept pixels, in its order
+    (view-major in index order, not in `order`; row-major).  So the masks are a subset of fuse_depth_maps' masks, where a pixel is
+    kept its fused depth is the same bits, and the first view in `order` keeps exactly what fuse_depth_maps keeps there.
+
+    This is fusibile-style (greedy suppression in view order), not fusibile: fusibile's disparity threshold and normal test are not
+    applied, and no number of fusibile's is claimed.  Refused with MvsB200Error: a view that lists itself among its sources, an
+    order that is not a permutation of range(N), and whatever fuse_depth_maps refuses.  One check launch per view in `order`, then
+    one compaction; the one device-to-host read is the point count.  Two calls on the same inputs return the same bits."""
+    if not isinstance(depth, torch.Tensor) or depth.dim() != 4:
+        _fail(f"depth maps [N, 1, h, w] expected, got {type(depth).__name__} {tuple(getattr(depth, 'shape', ()))}")
+    N = depth.shape[0]
+    own = np.nonzero((source_table(sources, N) == np.arange(N)[:, None]).any(1))[0]
+    if own.size:
+        _fail(f"visibility_fusion: view {int(own[0])} lists itself among its sources (it would mark the pixels it is reading)")
+    views = _view_order(order, N)
+    d, c, cams, src, mask, count, fused, blocks = _prepare(depth, conf, K, R, T, sources, normal)
+    _, _, h, w = depth.shape
+    used = torch.zeros((N, h, w), dtype=torch.uint8, device=depth.device)
+    for r in views:
+        with _timed("fusion_visibility"):
+            _lib.call("mvsb200_fusion_visibility", d.data_ptr(), c.data_ptr(), cams.data_ptr(), src.data_ptr(), N, src.shape[1], h, w,
+                      float(conf_min), float(reproj_px), float(rel_depth), int(min_views), r, used.data_ptr(), mask.data_ptr(),
+                      count.data_ptr(), fused.data_ptr(), blocks.data_ptr(), _stream())
+    xyz, rgb = _emit(mask, fused, blocks, cams, colours)
     return xyz, rgb, mask.bool()
 
 

@@ -455,6 +455,15 @@ int mvsb200_fusion_check(const float* depth, const float* conf, const float* cam
                          int h, int w, float conf_min, float reproj_px, float rel_depth, int min_views,
                          uint8_t* mask, int32_t* count, float* fused, int32_t* block_counts, void* stream);
 
+/* visibility fusion (fusibile-style greedy suppression): the check of reference view `ref` only, with a state used [N, h, w] uint8.
+ * A pixel with used[ref] set is no reference (mask 0, count 0, fused = d); every other pixel runs the test above, and a kept pixel
+ * sets used[j, floor(v + 1/2), floor(u + 1/2)] = 1 for every consistent source j, (u, v) its projection into j.  Writes the slices of
+ * view ref of mask, count, fused and block_counts (the arrays and layout of mvsb200_fusion_check).  Call once per view, in the
+ * chosen order, on one stream.  No view may list itself among its sources (the launch would write the marks it reads). */
+int mvsb200_fusion_visibility(const float* depth, const float* conf, const float* cams, const int32_t* sources, int N, int S,
+                              int h, int w, float conf_min, float reproj_px, float rel_depth, int min_views, int ref,
+                              uint8_t* used, uint8_t* mask, int32_t* count, float* fused, int32_t* block_counts, void* stream);
+
 /* compaction: offsets [N * blocks] int64, the exclusive scan of block_counts.  Writes xyz [M, 3] (the fused depth unprojected at the
  * reference pixel) and rgb [M, 3] (colours [N, 3, h, w] at that pixel) in view-major, row-major order; deterministic, no atomics. */
 int mvsb200_fusion_emit(const uint8_t* mask, const float* fused, const float* colours, const float* cams, const int64_t* offsets,
