@@ -259,9 +259,10 @@ __global__ void __launch_bounds__(256) conv_out_dgrad_march_kernel(const float* 
 // plane loop three times), the entering plane read through L1 (the 4 threads of a pixel and the 8 pixels of a warp share the
 // lines).  54 FMAs per 4 bytes of z instead of 8 per 16 bytes and tap (the previous form: a warp per line, lane = tap, 22
 // instructions per 216 MACs); no shared memory, no barrier in the loop (a first version staged g through a shared tile with
-// two CTA barriers per plane: 1.0 ms instead of 0.7 -- barrier bound).  CTAs are persistent (<= 592): accumulators run on
+// two CTA barriers per plane: 1.0 ms instead of 0.7 -- barrier bound).  CTAs are persistent (one wave): accumulators run on
 // across work items and are reduced once (shuffles in a fixed order, then the deterministic finalize).
 constexpr int kWTX = 16, kWTY = 4, kWDchunk = 48;    // pixel tile, planes per work item (a multiple of 3)
+constexpr int kWgMarchCtasPerSm = 2;                // persistent grid: CTAs per SM, the residency of __launch_bounds__(256, 2)
 __device__ float c_zero_row[4];                      // where the row pointer of a line outside the image points
 
 __global__ void __launch_bounds__(256, 2) conv_out_wgrad_march_kernel(const uint32_t* __restrict__ z, const float* __restrict__ g,
@@ -450,7 +451,17 @@ extern "C" int mvsb200_conv_out_wgrad(const void* z, const float* glogits, float
         const int tiles_x = (w + kWTX - 1) / kWTX, tiles_y = (h + kWTY - 1) / kWTY, nchunks = (D + kWDchunk - 1) / kWDchunk;
         const long items = (long)tiles_x * tiles_y * nchunks * B;
         MVS_REQUIRE(items < (1L << 31), "conv_out_wgrad: volume too large");
-        const int grid = (int)(items < kWgBlocks ? items : kWgBlocks);
+        // the persistent grid is one wave: as many CTAs as the device holds at once (2 per SM at 128 registers x 256 threads),
+        // taken from the device's SM count.  One CTA per SM would leave half of every SM to the streaming kernels the side
+        // stream's weight gradient runs beside (mvs_b200/ops.py, wgrad_fork), but measured slower in the cfg2 step: 15.97
+        // against 15.57 ms (profiles/r07_wgrad_overlap.md)
+        int sms = 148;
+        {
+            int dev = 0, n = 0;
+            if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
+        }
+        const long cap = (long)kWgMarchCtasPerSm * sms < kWgBlocks ? (long)kWgMarchCtasPerSm * sms : kWgBlocks;
+        const int grid = (int)(items < cap ? items : cap);
         conv_out_wgrad_march_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)z, glogits, workspace, B, D, h, w, tiles_x,
                                                                             tiles_y, nchunks, (int)items);
         MVS_CHECK_LAUNCH("conv_out_wgrad_march");

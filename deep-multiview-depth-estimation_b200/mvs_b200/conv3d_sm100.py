@@ -19,7 +19,7 @@ import torch
 import torch.nn.functional as F
 
 from . import _lib, conv3d as conv_backends
-from .ops import _stream, _timed
+from .ops import _stream, _timed, wgrad_fork
 
 _CIN_OK = (16, 32, 64)
 
@@ -137,7 +137,11 @@ class _Conv3dS1(torch.autograd.Function):
         x_cl, w = ctx.saved_tensors
         gy = gy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last_3d)
         gx = _s1_dgrad(gy, w, ctx.pad, x_cl.shape) if ctx.needs_input_grad[0] else None
-        gw = _s1_wgrad(x_cl, gy, w, ctx.pad) if ctx.needs_input_grad[1] else None
+        gw = None
+        if ctx.needs_input_grad[1]:
+            with wgrad_fork(w, (x_cl, gy)) as f:
+                f.result = _s1_wgrad(x_cl, gy, w, ctx.pad)
+            gw = f.grad()
         return gx, gw, None
 
 
@@ -363,8 +367,10 @@ class _ConvTranspose3dS2(torch.autograd.Function):
             mode = _s2_wgrad_mode(gy.shape, x_cl.shape)
             if mode != "cudnn":
                 # gW[ci][co][k] = sum_j x[j][ci] gy[2j - p + k][co]: the strided operand is the output gradient
-                g27 = s2_wgrad(gy, x_cl, pads, mode)                                     # [27, Cout, Cin]
-                gw = g27.reshape(3, 3, 3, cout_t, cin_t).permute(4, 3, 0, 1, 2).to(w.dtype)
+                with wgrad_fork(w, (gy, x_cl)) as f:
+                    g27 = s2_wgrad(gy, x_cl, pads, mode)                                 # [27, Cout, Cin]
+                    f.result = g27.reshape(3, 3, 3, cout_t, cin_t).permute(4, 3, 0, 1, 2).to(w.dtype)
+                gw = f.grad()
             else:
                 xs = torch.zeros((x_cl.shape[0], x_cl.shape[1]) + tuple(n_o), dtype=x_cl.dtype, device=x_cl.device,
                                  ).contiguous(memory_format=torch.channels_last_3d)
@@ -548,15 +554,17 @@ def _s2box_backward(x_cl, w, pads, out_dims, splits, holder, gys, need_x, need_w
     if own_dgrad or own_wgrad:
         if gy_box is None:
             gy_box = assemble((B, cout) + out_dims, tuple(slice(0, n) for n in out_dims))
-        if own_wgrad:
-            # gW[co][ci][k] = sum_o x[2o - pad + k][ci] gy[o][co]: the strided operand is the layer's input
-            g27 = s2_wgrad(x_cl, gy_box, pads, wg_mode)                            # [27, Cin, Cout]; gy_box may be a view
-            gw = g27.reshape(3, 3, 3, cin, cout).permute(4, 3, 0, 1, 2)
         if own_dgrad:
             # gx[2J + par] = sum_k W[k]^T gy[J + (par + pad - k)/2]: the forward weight [Cout, Cin, ...] IS the
             # ConvTranspose3d layout [in = Cout, out = Cin, ...] of that transposed convolution
             gx = conv_transpose3d_s2_kc(gy_box.contiguous(memory_format=torch.channels_last_3d), widths, w, pads,
                                         tuple(x_cl.shape[2:]), out=acc_into, accumulate=acc_into is not None)
+        if own_wgrad:                    # after the data gradient: a forked weight gradient overlaps what follows it
+            # gW[co][ci][k] = sum_o x[2o - pad + k][ci] gy[o][co]: the strided operand is the layer's input
+            with wgrad_fork(w, (x_cl, gy_box)) as f:
+                g27 = s2_wgrad(x_cl, gy_box, pads, wg_mode)                        # [27, Cin, Cout]; gy_box may be a view
+                f.result = g27.reshape(3, 3, 3, cin, cout).permute(4, 3, 0, 1, 2).to(w.dtype)
+            gw = f.grad()
     return gx, (gw.to(w.dtype) if gw is not None else None)
 
 
@@ -584,7 +592,10 @@ class _EntryConvs(torch.autograd.Function):
         if gy0 is not None:
             gy0 = gy0.to(torch.bfloat16).contiguous(memory_format=torch.channels_last_3d)
             gx = _s1_dgrad(gy0, w00, 1, x_cl.shape) if need_x else None
-            gw00 = _s1_wgrad(x_cl, gy0, w00, 1) if ctx.needs_input_grad[1] else None
+            if ctx.needs_input_grad[1]:
+                with wgrad_fork(w00, (x_cl, gy0)) as f:
+                    f.result = _s1_wgrad(x_cl, gy0, w00, 1)
+                gw00 = f.grad()
         acc = gx if gx is not None and gx.is_contiguous(memory_format=torch.channels_last_3d) and gx.dtype == torch.bfloat16 else None
         g2, gw_cat = _s2box_backward(x_cl, w_cat, ctx.pads, ctx.out_dims, ctx.splits, ctx.holder, gys, need_x,
                                      bool(ctx.needs_input_grad[2]), acc_into=acc)

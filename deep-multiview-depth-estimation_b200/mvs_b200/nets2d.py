@@ -89,6 +89,7 @@ class _Conv2dRows(torch.autograd.Function):
             raise _lib.MvsB200Error(f"2D convolution: {ci} -> {co} channels on rows of {cx} -> {cy}")
         y = _conv_rows(x, _pack2d(wf, "fwd", _n_rows(cy), max(cx, 16)), cy, 2.0 * 9 * ci * co * N * H * W)
         ctx.save_for_backward(x, wf)
+        ctx.w_arg = w                  # the weight as passed: a parameter, or k5s2_as_3x3 of one (ops.wgrad_fork follows it)
         return y
 
     @staticmethod
@@ -103,11 +104,13 @@ class _Conv2dRows(torch.autograd.Function):
         if ctx.needs_input_grad[0]:
             gx = _conv_rows(gy, _pack2d(w, "dgrad", _n_rows(cx), max(cy, 16)), cx, work)
         if ctx.needs_input_grad[1]:
-            gw27 = torch.empty((27, max(cx, 16), cy), dtype=torch.float32, device=gy.device)
-            with _timed("conv2d_wgrad_tc", work):
-                _lib.call("mvsb200_conv3d_s1_wgrad_ex", x.data_ptr(), gy.data_ptr(), gw27.data_ptr(), 1, N, H, W, cx, N, H, W, cy,
-                          -1, -1, -1, 2, _stream())
-            gw = gw27[9:18, :ci, :co].reshape(3, 3, ci, co).permute(3, 2, 0, 1)      # a view: the accumulation into .grad reads it strided
+            with ops.wgrad_fork(ctx.w_arg, (x, gy)) as f:
+                gw27 = torch.empty((27, max(cx, 16), cy), dtype=torch.float32, device=gy.device)
+                with _timed("conv2d_wgrad_tc", work):
+                    _lib.call("mvsb200_conv3d_s1_wgrad_ex", x.data_ptr(), gy.data_ptr(), gw27.data_ptr(), 1, N, H, W, cx, N, H, W, cy,
+                              -1, -1, -1, 2, _stream())
+                f.result = gw27[9:18, :ci, :co].reshape(3, 3, ci, co).permute(3, 2, 0, 1)   # a view: the accumulation into .grad reads it strided
+            gw = f.grad()
         return gx, gw, None
 
 
@@ -149,7 +152,10 @@ def k5s2_as_3x3(w5):
     space-to-depth form of its input (differentiable re-indexing; the 11 taps that fall outside the 5x5 support are zero)."""
     co, ci = w5.shape[:2]
     w6 = F.pad(w5.float(), (0, 1, 0, 1))
-    return w6.view(co, ci, 3, 2, 3, 2).permute(0, 3, 5, 1, 2, 4).reshape(co, 4 * ci, 3, 3)
+    w3 = w6.view(co, ci, 3, 2, 3, 2).permute(0, 3, 5, 1, 2, 4).reshape(co, 4 * ci, 3, 3)
+    # the same re-indexing backwards, for a gradient of w3 computed off the launching stream (ops.wgrad_fork)
+    w3._mvs_wgrad_to = [(w5, lambda g: g.reshape(co, 2, 2, ci, 3, 3).permute(0, 3, 4, 1, 5, 2).reshape(co, ci, 6, 6)[..., :5, :5])]
+    return w3
 
 
 def image_rows(images):

@@ -38,6 +38,100 @@ class _timed:
         return False
 
 
+# --------------------------------------------------------------------------------------------------
+# weight gradients off the critical path of the backward pass
+# --------------------------------------------------------------------------------------------------
+# A weight gradient reads the layer's saved input and its output gradient, and nothing later in the backward pass reads it.
+# Inside loss.backward() the convolution nodes therefore launch it on a side stream and return None for the weight; the
+# tensor-core weight-gradient kernels then run under the streaming BatchNorm / data-gradient kernels that follow on the
+# launching stream.  One end-of-backward callback joins the side stream and adds every such gradient into its parameter's
+# .grad, as AccumulateGrad would (allocated in the parameter's layout, or added in place -- a FlatGradAllReduce view stays one),
+# so .grad is complete on the current stream when backward() returns.  torch.autograd.grad, backward(inputs=...) without the
+# weight, and double backward keep the plain path: the node returns the gradient.
+WGRAD_FORK = True
+_SIDE = {}
+_PENDING = {}
+
+
+def _side_stream(device):
+    """One side stream per device.  0 is the lowest priority CUDA offers (the default and torch's streams sit there too)."""
+    st = _SIDE.get(device)
+    if st is None:
+        st = _SIDE[device] = torch.cuda.Stream(device, priority=0)
+    return st
+
+
+def _will_accumulate(p):
+    """p (a leaf) receives its gradient through AccumulateGrad in the running backward pass."""
+    try:
+        return p.is_leaf and p.requires_grad and torch._C._will_engine_execute_node(torch.autograd.graph.get_gradient_edge(p).node)
+    except RuntimeError:                     # torch.autograd.grad: the engine captures leaf gradients instead of accumulating them
+        return False
+
+
+def _wgrad_targets(w):
+    """[(leaf parameter, map from w's gradient to the parameter's)] when every parameter behind w accumulates in this pass."""
+    if not WGRAD_FORK or torch.is_grad_enabled() or not w.is_cuda:
+        return None
+    targets = [(w, None)] if w.is_leaf else getattr(w, "_mvs_wgrad_to", None)
+    if not targets or not all(_will_accumulate(p) for p, _ in targets):
+        return None
+    return targets
+
+
+class wgrad_fork:
+    """`with wgrad_fork(w, reads) as f: f.result = <weight gradient of w>` inside a backward node; then return f.grad() for w.
+    Forked, the body launches on the side stream, after all work the launching stream has issued so far; `reads` (the tensors
+    the body reads) stay allocated until the side stream is done with them."""
+
+    def __init__(self, w, reads):
+        self.targets, self.reads, self.result = _wgrad_targets(w), reads, None
+
+    def __enter__(self):
+        if self.targets is not None:
+            cur = torch.cuda.current_stream()
+            self.side = _side_stream(cur.device)
+            self.side.wait_stream(cur)
+            for t in self.reads:
+                t.record_stream(self.side)
+            self._guard = torch.cuda.stream(self.side)
+            self._guard.__enter__()
+        return self
+
+    def __exit__(self, *exc):
+        if self.targets is not None:
+            self._guard.__exit__(*exc)
+            if exc[0] is None:
+                task = torch._C._current_graph_task_id()
+                if task not in _PENDING:
+                    _PENDING[task] = []
+                    torch.autograd.Variable._execution_engine.queue_callback(lambda: _join(task))
+                _PENDING[task].append((self.side, self.result, self.targets))
+        return False
+
+    def grad(self):
+        return self.result if self.targets is None else None
+
+
+def _join(task):
+    """End of the backward pass: the current stream waits for the side stream(s), then every forked gradient goes into .grad."""
+    pending = _PENDING.pop(task)
+    cur = {}
+    with torch.no_grad():
+        for side, g, targets in pending:
+            st = cur.get(side)
+            if st is None:
+                st = cur[side] = torch.cuda.current_stream(side.device)
+                st.wait_stream(side)
+            g.record_stream(st)
+            for p, to_param in targets:
+                gp = g if to_param is None else to_param(g)
+                if p.grad is None:
+                    p.grad = torch.empty_like(p).copy_(gp)
+                else:
+                    p.grad.add_(gp)
+
+
 def _need_cuda(t: torch.Tensor, what: str):
     if not t.is_cuda:
         raise _lib.MvsB200Error(f"{what} must live on a CUDA device (got {t.device}); mvs_b200 has no CPU path")
@@ -534,7 +628,7 @@ class _ConvOut(torch.autograd.Function):
         with _timed("conv_out_fwd"):
             _lib.call("mvsb200_conv_out_fwd", zc.data_ptr(), w27.data_ptr(), out.data_ptr(), B, D, h, w, _stream())
         ctx.save_for_backward(zc, w27)
-        ctx.wdtype, ctx.zdtype = weight.dtype, z.dtype
+        ctx.wdtype, ctx.zdtype, ctx.w_arg = weight.dtype, z.dtype, weight
         return out
 
     @staticmethod
@@ -549,11 +643,13 @@ class _ConvOut(torch.autograd.Function):
                 _lib.call("mvsb200_conv_out_dgrad", g.data_ptr(), w27.data_ptr(), gz.data_ptr(), B, D, h, w, _stream())
             gz = gz.to(ctx.zdtype)
         if ctx.needs_input_grad[1]:
-            gw27 = torch.empty_like(w27)
-            with _timed("conv_out_wgrad"):
-                _lib.call("mvsb200_conv_out_wgrad", zc.data_ptr(), g.data_ptr(), _conv_out_workspace(zc.device).data_ptr(),
-                          gw27.data_ptr(), B, D, h, w, _stream())
-            gw = gw27.reshape(3, 3, 3, 8).permute(3, 0, 1, 2).unsqueeze(0).to(ctx.wdtype)
+            with wgrad_fork(ctx.w_arg, (zc, g)) as f:
+                gw27 = torch.empty_like(w27)
+                with _timed("conv_out_wgrad"):
+                    _lib.call("mvsb200_conv_out_wgrad", zc.data_ptr(), g.data_ptr(), _conv_out_workspace(zc.device).data_ptr(),
+                              gw27.data_ptr(), B, D, h, w, _stream())
+                f.result = gw27.reshape(3, 3, 3, 8).permute(3, 0, 1, 2).unsqueeze(0).to(ctx.wdtype)
+            gw = f.grad()
         return gz, gw
 
 

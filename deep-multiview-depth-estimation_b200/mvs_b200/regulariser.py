@@ -176,7 +176,13 @@ class CostVolumeReg(nn.Module):
         # the three stride-2 branches all read cv (model.py:104-110): ONE convolution with the weights stacked along
         # Cout (16+32+64 = 112) reads the cost volume once instead of three times; with conv_0_0 they form one autograd node
         # (the cost volume's gradient is accumulated inside the kernels, not by an elementwise pass of autograd)
-        w_cat = torch.cat([self._w(f"conv_{k}_0", wdt) for k in (1, 2, 3)], 0)
+        w_parts = [self._w(f"conv_{k}_0", wdt) for k in (1, 2, 3)]
+        w_cat = torch.cat(w_parts, 0)
+        # where a weight gradient of w_cat computed off the launching stream goes (ops.wgrad_fork): the rows of each branch
+        rows = [0]
+        for p in w_parts:
+            rows.append(rows[-1] + p.shape[0])
+        w_cat._mvs_wgrad_to = [(p, (lambda g, a=a, b=b: g[a:b])) for p, a, b in zip(w_parts, rows, rows[1:])]
         widths = [self.conv_1_0.out_channels, self.conv_2_0.out_channels, self.conv_3_0.out_channels]
         box_pads, box_dims = tuple(L for _, _, L in reg), tuple(hi - lo + 1 for lo, hi, _ in reg)
         S_parts = None
