@@ -13,6 +13,9 @@
 //   pc_thin_list_kernel      of lower-ranked points within dst (fp64, inclusive), then the list itself (CSR, scan order)
 //   pc_thin_round_kernel     one parallel greedy round: undecided -> kept when every lower-ranked neighbour is removed, removed
 //                            when one is kept; reads one state buffer and writes the other, counts the undecided points
+//   pc_transform_crop_kernel K9, Tanks and Temples: fp64 affine transform and polygon-volume crop, one thread per point
+//   pc_voxel_keys_kernel     K9: int64 voxel key of each fp64 point
+//   pc_voxel_mean_kernel     K9: one thread per occupied voxel, the sequential fp64 mean of its stably sorted points
 //
 // Nearest search.  Shells r = 0, 1, ... of fine cells around the query's (clamped) cell, up to kFineShells; then shells of coarse
 // blocks, skipping empty blocks, visiting an occupied block by its points (few) or by its fine cells (many).  A shell is entered
@@ -275,6 +278,92 @@ __global__ void __launch_bounds__(kThreads) pc_thin_round_kernel(const int64_t* 
     if (threadIdx.x == 0 && c) atomicAdd(undecided, c);         // an integer count: the same total in any order
 }
 
+// ---- Tanks and Temples pre-processing (DESIGN §4 "K9 Tanks and Temples evaluation") -------------------------------------------
+// fp64 with explicit round-to-nearest intrinsics, so that nvcc contracts nothing into an FMA: every bit equals a numpy restatement
+// written in the same operation order.
+
+constexpr int kMaxPolygon = 1024;
+
+struct Affine {
+    double a[12];                   // rows 0..2 of a 4 x 4 matrix whose last row is (0, 0, 0, 1), row-major
+};
+
+// one thread per point: p' = A [p; 1] (skipped when `transform` is 0), then Open3D's SelectionPolygonVolume::CropInPolygon with the
+// polygon's (u, v) columns in shared memory: outside when p_w is outside [axis_min, axis_max]; else inside iff an odd number of the
+// edge nodes crossing p_v lie below p_u
+__global__ void __launch_bounds__(kThreads) pc_transform_crop_kernel(const float* __restrict__ xyz, int n, Affine A, int transform,
+                                                                    const double* __restrict__ polygon, int k, int u, int v, int w,
+                                                                    double axis_min, double axis_max, double* __restrict__ out,
+                                                                    uint8_t* __restrict__ keep) {
+    __shared__ double bu[kMaxPolygon], bv[kMaxPolygon];
+    for (int t = threadIdx.x; t < k; t += kThreads) {
+        bu[t] = polygon[3 * t + u];
+        bv[t] = polygon[3 * t + v];
+    }
+    __syncthreads();
+    const int i = blockIdx.x * kThreads + threadIdx.x;
+    if (i >= n) return;
+    double p[3] = {xyz[3 * (size_t)i], xyz[3 * (size_t)i + 1], xyz[3 * (size_t)i + 2]};
+    if (transform) {
+        double q[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+            q[r] = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(A.a[4 * r], p[0]), __dmul_rn(A.a[4 * r + 1], p[1])),
+                                       __dmul_rn(A.a[4 * r + 2], p[2])), A.a[4 * r + 3]);
+        p[0] = q[0], p[1] = q[1], p[2] = q[2];
+    }
+    out[3 * (size_t)i] = p[0], out[3 * (size_t)i + 1] = p[1], out[3 * (size_t)i + 2] = p[2];
+    // selects, not p[u]: a run-time index would put p in a local-memory stack frame
+    const double pu = u == 0 ? p[0] : p[1], pv = v == 1 ? p[1] : p[2], pw = w == 0 ? p[0] : w == 1 ? p[1] : p[2];
+    bool in = false;
+    if (!(pw < axis_min || pw > axis_max)) {
+        for (int a = 0; a < k; ++a) {
+            const int b = a + 1 == k ? 0 : a + 1;
+            const double av = bv[a], bvv = bv[b];
+            if ((av < pv && bvv >= pv) || (bvv < pv && av >= pv)) {
+                const double node = __dadd_rn(bu[a], __dmul_rn(__ddiv_rn(__dsub_rn(pv, av), __dsub_rn(bvv, av)), __dsub_rn(bu[b], bu[a])));
+                in ^= node < pu;
+            }
+        }
+    }
+    keep[i] = in;
+}
+
+// one thread per point: the voxel index floor((p - vmin) / voxel) per axis (IEEE division) -> int64 key (iz ny + iy) nx + ix
+__global__ void __launch_bounds__(kThreads) pc_voxel_keys_kernel(const double* __restrict__ xyz, int n, double ox, double oy, double oz,
+                                                                double voxel, int64_t nx, int64_t ny, int64_t* __restrict__ keys) {
+    const int i = blockIdx.x * kThreads + threadIdx.x;
+    if (i >= n) return;
+    const int64_t ix = (int64_t)floor(__ddiv_rn(__dsub_rn(xyz[3 * (size_t)i], ox), voxel));
+    const int64_t iy = (int64_t)floor(__ddiv_rn(__dsub_rn(xyz[3 * (size_t)i + 1], oy), voxel));
+    const int64_t iz = (int64_t)floor(__ddiv_rn(__dsub_rn(xyz[3 * (size_t)i + 2], oz), voxel));
+    keys[i] = (iz * ny + iy) * nx + ix;
+}
+
+// one thread per occupied voxel: its points are perm[offsets[j] .. offsets[j + 1]) (a stable sort: ascending input order), summed
+// one after another from 0 in fp64, then divided by their count
+__global__ void __launch_bounds__(kThreads) pc_voxel_mean_kernel(const double* __restrict__ xyz, const int64_t* __restrict__ perm,
+                                                                const int64_t* __restrict__ offsets, int n_voxels,
+                                                                double* __restrict__ mean, float* __restrict__ mean_f32) {
+    const int j = blockIdx.x * kThreads + threadIdx.x;
+    if (j >= n_voxels) return;
+    const int64_t b = offsets[j], e = offsets[j + 1];
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    for (int64_t s = b; s < e; ++s) {
+        const int64_t i = __ldg(perm + s);
+        sx = __dadd_rn(sx, __ldg(xyz + 3 * i));
+        sy = __dadd_rn(sy, __ldg(xyz + 3 * i + 1));
+        sz = __dadd_rn(sz, __ldg(xyz + 3 * i + 2));
+    }
+    const double c = (double)(e - b);
+    const double m[3] = {__ddiv_rn(sx, c), __ddiv_rn(sy, c), __ddiv_rn(sz, c)};
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        mean[3 * (size_t)j + r] = m[r];
+        mean_f32[3 * (size_t)j + r] = (float)m[r];
+    }
+}
+
 int blocks_for(int n) { return (n + kThreads - 1) / kThreads; }
 
 bool grid_ok(float cell, int nbx, int nby, int nbz) {
@@ -350,5 +439,48 @@ extern "C" int mvsb200_pc_thin_round(const int64_t* offsets, const int32_t* list
     MVS_REQUIRE(n >= 1, "pc_thin_round: 1 <= n < 2^31 points");
     pc_thin_round_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(offsets, list, state_in, state_out, n, undecided);
     MVS_CHECK_LAUNCH("pc_thin_round");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_transform_crop(const float* xyz, int n, const double* affine12_host, const double* polygon, int k, int axis,
+                                         double axis_min, double axis_max, double* out, uint8_t* keep, void* stream) {
+    MVS_REQUIRE(xyz && polygon && out && keep, "pc_transform_crop: null pointer");
+    MVS_REQUIRE(n >= 1, "pc_transform_crop: 1 <= n < 2^31 points");
+    MVS_REQUIRE(k >= 3 && k <= kMaxPolygon, "pc_transform_crop: a polygon of 3 to %d vertices, got %d", kMaxPolygon, k);
+    MVS_REQUIRE(axis >= 0 && axis <= 2, "pc_transform_crop: orthogonal axis 0, 1 or 2, got %d", axis);
+    MVS_REQUIRE(isfinite(axis_min) && isfinite(axis_max), "pc_transform_crop: finite axis bounds");
+    Affine A{};
+    if (affine12_host) {
+        for (int t = 0; t < 12; ++t) {
+            MVS_REQUIRE(isfinite(affine12_host[t]), "pc_transform_crop: the transform must be finite");
+            A.a[t] = affine12_host[t];
+        }
+    }
+    // (u, v, w) of Open3D's CropInPolygon: x -> (1, 2, 0), y -> (0, 2, 1), z -> (0, 1, 2)
+    const int u = axis == 0 ? 1 : 0, v = axis == 2 ? 1 : 2;
+    pc_transform_crop_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(xyz, n, A, affine12_host != nullptr, polygon, k, u, v,
+                                                                                   axis, axis_min, axis_max, out, keep);
+    MVS_CHECK_LAUNCH("pc_transform_crop");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_voxel_keys(const double* xyz, int n, double ox, double oy, double oz, double voxel, int64_t nx, int64_t ny,
+                                     int64_t nz, int64_t* keys, void* stream) {
+    MVS_REQUIRE(xyz && keys, "pc_voxel_keys: null pointer");
+    MVS_REQUIRE(n >= 1, "pc_voxel_keys: 1 <= n < 2^31 points");
+    MVS_REQUIRE(voxel > 0.0 && isfinite(voxel) && isfinite(ox) && isfinite(oy) && isfinite(oz), "pc_voxel_keys: voxel > 0, finite origin");
+    MVS_REQUIRE(nx >= 1 && ny >= 1 && nz >= 1 && nx < (int64_t(1) << 62) / ny && nx * ny < (int64_t(1) << 62) / nz,
+                "pc_voxel_keys: 1 <= voxels per axis and nx ny nz < 2^62");
+    pc_voxel_keys_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(xyz, n, ox, oy, oz, voxel, nx, ny, keys);
+    MVS_CHECK_LAUNCH("pc_voxel_keys");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_voxel_mean(const double* xyz, const int64_t* perm, const int64_t* offsets, int n_voxels, double* mean,
+                                     float* mean_f32, void* stream) {
+    MVS_REQUIRE(xyz && perm && offsets && mean && mean_f32, "pc_voxel_mean: null pointer");
+    MVS_REQUIRE(n_voxels >= 1, "pc_voxel_mean: 1 <= n_voxels < 2^31");
+    pc_voxel_mean_kernel<<<blocks_for(n_voxels), kThreads, 0, (cudaStream_t)stream>>>(xyz, perm, offsets, n_voxels, mean, mean_f32);
+    MVS_CHECK_LAUNCH("pc_voxel_mean");
     return MVSB200_OK;
 }

@@ -98,6 +98,9 @@ _SIGNATURES = {
     "mvsb200_pc_nearest": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _P, _P]),
     "mvsb200_pc_thin_neighbours": (_I, [_P, _P, _P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_double, _P, _P, _P, _P]),
     "mvsb200_pc_thin_round": (_I, [_P, _P, _P, _P, _I, _P, _P]),
+    "mvsb200_pc_transform_crop": (_I, [_P, _I, _P, _P, _I, _I, _c.c_double, _c.c_double, _P, _P, _P]),
+    "mvsb200_pc_voxel_keys": (_I, [_P, _I] + [_c.c_double] * 4 + [_c.c_int64] * 3 + [_P, _P]),
+    "mvsb200_pc_voxel_mean": (_I, [_P, _P, _P, _I, _P, _P, _P]),
 }
 
 _lib = None

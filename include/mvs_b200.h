@@ -507,6 +507,25 @@ int mvsb200_pc_thin_neighbours(const float* pts, const int32_t* cells, const int
 int mvsb200_pc_thin_round(const int64_t* offsets, const int32_t* list, const uint8_t* state_in, uint8_t* state_out, int n,
                           int32_t* undecided, void* stream);
 
+/* ---- K9: Tanks and Temples pre-processing (the toolbox's transform, polygon-volume crop and voxel down-sampling) ----------------
+ * All fp64 with no FMA contraction (round-to-nearest multiply, add and IEEE division in the stated order).
+ * transform_crop: out [n, 3] fp64 = p' = A [p; 1] for the fp32 points xyz [n, 3], component i = ((A[i,0]x + A[i,1]y) + A[i,2]z) + A[i,3],
+ * with affine12_host the first three rows of A (HOST, row-major; NULL: no transform, p' = p).  keep [n] uint8 = p' lies in Open3D's
+ * SelectionPolygonVolume: axis = the orthogonal axis w (0, 1, 2 for x, y, z), (u, v) = (1, 2), (0, 2), (0, 1); outside when
+ * p'_w < axis_min or p'_w > axis_max; else inside iff an odd number of the edges (i, j = i + 1 mod k) of polygon [k, 3] fp64 (device)
+ * with b_i,v < p_v <= b_j,v or b_j,v < p_v <= b_i,v have b_i,u + (p_v - b_i,v) / (b_j,v - b_i,v) * (b_j,u - b_i,u) < p_u.
+ * 3 <= k <= 1024. */
+int mvsb200_pc_transform_crop(const float* xyz, int n, const double* affine12_host, const double* polygon, int k, int axis,
+                              double axis_min, double axis_max, double* out, uint8_t* keep, void* stream);
+/* voxel_keys: keys [n] int64 = (iz ny + iy) nx + ix with i_a = floor((p_a - o_a) / voxel) for the fp64 points xyz [n, 3]; the caller
+ * sizes the grid (nx ny nz < 2^62) so that every index lies in [0, n_a).
+ * voxel_mean: after a stable sort of the keys (perm [n] int64) with segment offsets [n_voxels + 1] int64, mean [n_voxels, 3] fp64 =
+ * (the sum of the segment's points, added in ascending sorted position from 0) / count, and mean_f32 its fp32 rounding. */
+int mvsb200_pc_voxel_keys(const double* xyz, int n, double ox, double oy, double oz, double voxel, int64_t nx, int64_t ny, int64_t nz,
+                          int64_t* keys, void* stream);
+int mvsb200_pc_voxel_mean(const double* xyz, const int64_t* perm, const int64_t* offsets, int n_voxels, double* mean,
+                          float* mean_f32, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

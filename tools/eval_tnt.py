@@ -1,0 +1,46 @@
+"""Tanks and Temples precision, recall and F-score of one reconstructed scene (mvs_b200.evaluate_tanks_and_temples on the GPU).
+
+    python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 [--out result.json]
+
+--tnt is the directory of T&T's evaluation data, one sub-directory per scene with {scene}.ply, {scene}.json and {scene}_trans.txt
+(INTEGRATION.md §2).  The reconstruction must be in the frame of T&T's COLMAP cameras: the toolbox's trajectory registration is not
+run.  --tau is the scene's threshold (the toolbox's table of per-scene values is not shipped).  Prints one JSON line: precision,
+recall, fscore, the counts, and the histogram edges and cumulative curves."""
+import argparse
+import json
+import os
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, os.path.join(ROOT, "deep-multiview-depth-estimation_b200"))
+
+import numpy as np  # noqa: E402
+import torch  # noqa: E402
+
+import mvs_b200  # noqa: E402
+from mvs_b200 import tanks  # noqa: E402
+
+
+def main(argv=None):
+    ap = argparse.ArgumentParser(description=__doc__.splitlines()[0])
+    ap.add_argument("--ply", required=True, help="the reconstruction (binary little-endian or ASCII PLY)")
+    ap.add_argument("--tnt", required=True, help="T&T's evaluation directory ({scene}/{scene}.ply, .json, _trans.txt)")
+    ap.add_argument("--scene", required=True)
+    ap.add_argument("--tau", type=float, required=True, help="the scene's distance threshold, in the ground truth's units")
+    ap.add_argument("--stretch", type=float, default=tanks.STRETCH, help="the histograms span [0, stretch * tau)")
+    ap.add_argument("--out", help="also write the result as JSON to this file")
+    ap.add_argument("--device", default="cuda:0")
+    a = ap.parse_args(argv)
+    xyz, _ = mvs_b200.read_ply(a.ply)
+    gt, crop, trans = mvs_b200.load_tnt_eval(a.tnt, a.scene)
+    dev = torch.device(a.device)
+    r = mvs_b200.evaluate_tanks_and_temples(xyz.to(dev), gt.to(dev), crop, trans, a.tau, stretch=a.stretch)
+    r = {"scene": a.scene, "ply": a.ply, **{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in r.items()}}
+    print(json.dumps(r))
+    if a.out:
+        with open(a.out, "w") as f:
+            json.dump(r, f, indent=1)
+
+
+if __name__ == "__main__":
+    main()
