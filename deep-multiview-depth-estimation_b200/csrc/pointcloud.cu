@@ -8,7 +8,7 @@
 //   pc_grid_cells_kernel     one thread per sorted position: the point as float4 (x, y, z, original index), and the first / last
 //                            point of its cell and of its block -> cells[key] = {begin, end}, blocks[block] = {begin, end}.
 //                            Each entry is written by exactly one thread; untouched entries stay {0, 0} (empty).
-//   pc_nearest_kernel        one thread per query: exact nearest distance, capped at max_dist (below)
+//   pc_nearest_kernel        one thread per query: exact nearest distance, capped at max_dist (below); <true>: and its index
 //   pc_thin_count_kernel     thinning (greedy minimum-distance, reducePts_haa) on a grid with cell >= dst: per point the number
 //   pc_thin_list_kernel      of lower-ranked points within dst (fp64, inclusive), then the list itself (CSR, scan order)
 //   pc_thin_round_kernel     one parallel greedy round: undecided -> kept when every lower-ranked neighbour is removed, removed
@@ -16,6 +16,8 @@
 //   pc_transform_crop_kernel K9, Tanks and Temples: fp64 affine transform and polygon-volume crop, one thread per point
 //   pc_voxel_keys_kernel     K9: int64 voxel key of each fp64 point
 //   pc_voxel_mean_kernel     K9: one thread per occupied voxel, the sequential fp64 mean of its stably sorted points
+//   pc_icp_sums_{a,b}_kernel K9 registration: the Umeyama sums of the correspondences in two passes, a deterministic fp64 reduction
+//   pc_transform64_kernel    K9 registration: an fp64 affine update of the source in place, and its fp32 rounding
 //
 // Nearest search.  Shells r = 0, 1, ... of fine cells around the query's (clamped) cell, up to kFineShells; then shells of coarse
 // blocks, skipping empty blocks, visiting an occupied block by its points (few) or by its fine cells (many).  A shell is entered
@@ -71,10 +73,19 @@ __device__ __forceinline__ float shell_bound(float qx, float qy, float qz, int c
 
 __device__ __forceinline__ float sq(float a) { return a * a; }
 
-__device__ __forceinline__ void scan_points(const float4* __restrict__ pts, int b, int e, float qx, float qy, float qz, float& best) {
+// IDX: also the original index of the best point (pts[].w), the smaller index on an exact tie of the squared fp32 distance
+template <bool IDX>
+__device__ __forceinline__ void scan_points(const float4* __restrict__ pts, int b, int e, float qx, float qy, float qz, float& best,
+                                            int& bi) {
     for (int p = b; p < e; ++p) {
         const float4 t = __ldg(pts + p);
-        best = fminf(best, sq(t.x - qx) + sq(t.y - qy) + sq(t.z - qz));
+        const float d = sq(t.x - qx) + sq(t.y - qy) + sq(t.z - qz);
+        if constexpr (IDX) {
+            const int j = __float_as_int(t.w);
+            if (d < best || (d == best && j < bi)) best = d, bi = j;
+        } else {
+            best = fminf(best, d);
+        }
     }
 }
 
@@ -102,9 +113,13 @@ __global__ void __launch_bounds__(kThreads) pc_grid_cells_kernel(const float* __
     if (kn < 0 || (k >> 9) != (kn >> 9)) blocks[k >> 9].y = s + 1;
 }
 
+// IDX: also index[i] = the original index of the nearest point (ties: the smaller index), -1 where dist[i] is +inf.  Pruning is the
+// same in both forms: a tied point is never pruned, because every lower bound is below the true gap by `slack`.
+template <bool IDX>
 __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __restrict__ query, int n, const float4* __restrict__ pts,
                                                              const int2* __restrict__ cells, const int2* __restrict__ blocks, Grid g,
-                                                             float slack, float max_dist, float* __restrict__ dist) {
+                                                             float slack, float max_dist, float* __restrict__ dist,
+                                                             int32_t* __restrict__ index) {
     const int i = blockIdx.x * kThreads + threadIdx.x;
     if (i >= n) return;
     const float qx = query[3 * (size_t)i], qy = query[3 * (size_t)i + 1], qz = query[3 * (size_t)i + 2];
@@ -117,6 +132,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
         const double ez = fmax(fmax((double)g.oz - qz, (double)qz - (g.oz + nz * c)), 0.0);
         if (ex * ex + ey * ey + ez * ez >= (double)max_dist * max_dist) {
             dist[i] = kInf;
+            if constexpr (IDX) index[i] = -1;
             return;
         }
     }
@@ -124,6 +140,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
     const float lim = max_dist * max_dist;
     const int cx = cell_of(qx, g.ox, g.inv, nx), cy = cell_of(qy, g.oy, g.inv, ny), cz = cell_of(qz, g.oz, g.inv, nz);
     float best = kInf;                                                  // squared
+    int bi = -1;
     int r = 0;
     for (; r <= kFineShells; ++r) {
         const float L = shell_bound(qx, qy, qz, cx, cy, cz, r, nx, ny, nz, g, g.cell, sl);
@@ -142,7 +159,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
                     if (ix < 0 || ix >= nx) continue;
                     if (gy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= fminf(best, lim)) continue;
                     const int2 c = __ldg(cells + key_of(ix, iy, iz, g));
-                    scan_points(pts, c.x, c.y, qx, qy, qz, best);
+                    scan_points<IDX>(pts, c.x, c.y, qx, qy, qz, best, bi);
                 }
             }
         }
@@ -172,7 +189,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
                         const int2 br = __ldg(blocks + blk);
                         if (br.y <= br.x) continue;                     // empty block
                         if (br.y - br.x <= kDirect) {
-                            scan_points(pts, br.x, br.y, qx, qy, qz, best);
+                            scan_points<IDX>(pts, br.x, br.y, qx, qy, qz, best, bi);
                             continue;
                         }
                         for (int lz = 0; lz < 8; ++lz) {
@@ -189,7 +206,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
                                     if (near_zy && abs(ix - cx) <= kFineShells) continue;      // visited in the fine shells
                                     if (fy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= fminf(best, lim)) continue;
                                     const int2 c = __ldg(cells + (blk << 9) + (lz << 6) + (ly << 3) + lx);
-                                    scan_points(pts, c.x, c.y, qx, qy, qz, best);
+                                    scan_points<IDX>(pts, c.x, c.y, qx, qy, qz, best, bi);
                                 }
                             }
                         }
@@ -208,6 +225,7 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
         d = fmaf(0.5f * y, fmaf(-d, d, best), d);
     }
     dist[i] = d < max_dist ? d : kInf;
+    if constexpr (IDX) index[i] = d < max_dist ? bi : -1;
 }
 
 // the lower-ranked points within dst of sorted point s (fp64 on the fp32 coordinates, inclusive), in scan order; list == NULL: count
@@ -364,6 +382,116 @@ __global__ void __launch_bounds__(kThreads) pc_voxel_mean_kernel(const double* _
     }
 }
 
+// ---- K9 registration: the ICP loop of the toolbox's three stages (DESIGN §4 "K9 registration") ------------------------------------
+// Per correspondence i -> index[i] (>= 0) of the source src [n, 3] fp64 and the target tgt [m, 3] fp64, two passes, each a fixed
+// grid-stride split over at most kSumBlocks blocks, a fixed shared-memory tree per block, per-block fp64 partials, and the last block
+// to finish (an integer ticket) adding the partials in block order with the same tree.  No float atomics: the bits depend on n only.
+//   pass A  sums[0..7]  = c, sum |s - t|^2, sum s (3), sum t (3)
+//   pass B  sums[8..17] = sum (t - mu_t)(s - mu_s)^T (row-major, t's axis first), sum |s - mu_s|^2, with mu = sum / c read from
+//           pass A's sums in device memory (zeros when c = 0)
+
+constexpr int kSumBlocks = MVSB200_PC_ICP_BLOCKS;
+constexpr int kSumsA = 8, kSumsB = 10;
+
+// the block's K values -> partial[blockIdx.x]; the last block adds the partials in block order -> out[0..K); its ticket is reset
+template <int K>
+__device__ __forceinline__ void reduce_sums(double (&v)[K], double* __restrict__ partial, double* __restrict__ out,
+                                            unsigned* __restrict__ ticket) {
+    __shared__ double sh[K][kThreads];
+    __shared__ bool last;
+    const int t = threadIdx.x;
+#pragma unroll
+    for (int k = 0; k < K; ++k) sh[k][t] = v[k];
+    __syncthreads();
+    for (int h = kThreads / 2; h > 0; h >>= 1) {
+        if (t < h) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) sh[k][t] = __dadd_rn(sh[k][t], sh[k][t + h]);
+        }
+        __syncthreads();
+    }
+    if (t < K) partial[(size_t)blockIdx.x * K + t] = sh[t][0];
+    __threadfence();
+    __syncthreads();
+    if (t == 0) last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        double a = 0.0;
+        for (int b = t; b < (int)gridDim.x; b += kThreads) a = __dadd_rn(a, __ldcg(partial + (size_t)b * K + k));
+        sh[k][t] = a;
+    }
+    __syncthreads();
+    for (int h = kThreads / 2; h > 0; h >>= 1) {
+        if (t < h) {
+#pragma unroll
+            for (int k = 0; k < K; ++k) sh[k][t] = __dadd_rn(sh[k][t], sh[k][t + h]);
+        }
+        __syncthreads();
+    }
+    if (t < K) out[t] = sh[t][0];
+    if (t == 0) *ticket = 0u;
+}
+
+__global__ void __launch_bounds__(kThreads) pc_icp_sums_a_kernel(const double* __restrict__ src, const int32_t* __restrict__ index, int n,
+                                                                const double* __restrict__ tgt, double* __restrict__ partial,
+                                                                double* __restrict__ sums, unsigned* __restrict__ ticket) {
+    double v[kSumsA] = {};
+    for (int i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {
+        const int j = __ldg(index + i);
+        if (j < 0) continue;
+        const double sx = __ldg(src + 3 * (size_t)i), sy = __ldg(src + 3 * (size_t)i + 1), sz = __ldg(src + 3 * (size_t)i + 2);
+        const double tx = __ldg(tgt + 3 * (size_t)j), ty = __ldg(tgt + 3 * (size_t)j + 1), tz = __ldg(tgt + 3 * (size_t)j + 2);
+        const double dx = sx - tx, dy = sy - ty, dz = sz - tz;
+        v[0] += 1.0;
+        v[1] += dx * dx + dy * dy + dz * dz;
+        v[2] += sx, v[3] += sy, v[4] += sz;
+        v[5] += tx, v[6] += ty, v[7] += tz;
+    }
+    reduce_sums<kSumsA>(v, partial, sums, ticket);
+}
+
+__global__ void __launch_bounds__(kThreads) pc_icp_sums_b_kernel(const double* __restrict__ src, const int32_t* __restrict__ index, int n,
+                                                                const double* __restrict__ tgt, double* __restrict__ partial,
+                                                                double* __restrict__ sums, unsigned* __restrict__ ticket) {
+    const double c = sums[0];
+    double ms[3] = {0.0, 0.0, 0.0}, mt[3] = {0.0, 0.0, 0.0};
+    if (c > 0.0) {
+#pragma unroll
+        for (int r = 0; r < 3; ++r) ms[r] = __ddiv_rn(sums[2 + r], c), mt[r] = __ddiv_rn(sums[5 + r], c);
+    }
+    double v[kSumsB] = {};
+    for (int i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {
+        const int j = __ldg(index + i);
+        if (j < 0) continue;
+        double a[3], b[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) a[r] = __ldg(src + 3 * (size_t)i + r) - ms[r], b[r] = __ldg(tgt + 3 * (size_t)j + r) - mt[r];
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+#pragma unroll
+            for (int q = 0; q < 3; ++q) v[3 * r + q] += b[r] * a[q];
+        v[9] += a[0] * a[0] + a[1] * a[1] + a[2] * a[2];
+    }
+    reduce_sums<kSumsB>(v, partial, sums + kSumsA, ticket);
+}
+
+// one thread per point, in place: p' = A [p; 1] in K9's operation order (no contraction), and its fp32 rounding
+__global__ void __launch_bounds__(kThreads) pc_transform64_kernel(double* __restrict__ xyz, int n, Affine A, float* __restrict__ xyz_f32) {
+    const int i = blockIdx.x * kThreads + threadIdx.x;
+    if (i >= n) return;
+    const double p[3] = {xyz[3 * (size_t)i], xyz[3 * (size_t)i + 1], xyz[3 * (size_t)i + 2]};
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const double q = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(A.a[4 * r], p[0]), __dmul_rn(A.a[4 * r + 1], p[1])),
+                                             __dmul_rn(A.a[4 * r + 2], p[2])), A.a[4 * r + 3]);
+        xyz[3 * (size_t)i + r] = q;
+        xyz_f32[3 * (size_t)i + r] = (float)q;
+    }
+}
+
 int blocks_for(int n) { return (n + kThreads - 1) / kThreads; }
 
 bool grid_ok(float cell, int nbx, int nby, int nbz) {
@@ -403,10 +531,26 @@ extern "C" int mvsb200_pc_nearest(const float* query, int n, const float* pts, c
     MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "pc_nearest: cell > 0 and at most %d cells", MVSB200_PC_MAX_CELLS);
     MVS_REQUIRE(max_dist > 0.f && isfinite(max_dist) && slack >= 0.f, "pc_nearest: max_dist > 0 (finite), slack >= 0");
     if (n == 0) return MVSB200_OK;
-    pc_nearest_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
-                                                                            (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
-                                                                            slack, max_dist, dist);
+    pc_nearest_kernel<false><<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
+                                                                                   (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
+                                                                                   slack, max_dist, dist, nullptr);
     MVS_CHECK_LAUNCH("pc_nearest");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_nearest_index(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks,
+                                        float ox, float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist,
+                                        float* dist, int32_t* index, void* stream) {
+    MVS_REQUIRE(query && pts && cells && blocks && dist && index, "pc_nearest_index: null pointer");
+    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "pc_nearest_index: misaligned buffer");
+    MVS_REQUIRE(n >= 0, "pc_nearest_index: 0 <= n < 2^31 queries");
+    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "pc_nearest_index: cell > 0 and at most %d cells", MVSB200_PC_MAX_CELLS);
+    MVS_REQUIRE(max_dist > 0.f && isfinite(max_dist) && slack >= 0.f, "pc_nearest_index: max_dist > 0 (finite), slack >= 0");
+    if (n == 0) return MVSB200_OK;
+    pc_nearest_kernel<true><<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
+                                                                                  (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
+                                                                                  slack, max_dist, dist, index);
+    MVS_CHECK_LAUNCH("pc_nearest_index");
     return MVSB200_OK;
 }
 
@@ -482,5 +626,30 @@ extern "C" int mvsb200_pc_voxel_mean(const double* xyz, const int64_t* perm, con
     MVS_REQUIRE(n_voxels >= 1, "pc_voxel_mean: 1 <= n_voxels < 2^31");
     pc_voxel_mean_kernel<<<blocks_for(n_voxels), kThreads, 0, (cudaStream_t)stream>>>(xyz, perm, offsets, n_voxels, mean, mean_f32);
     MVS_CHECK_LAUNCH("pc_voxel_mean");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_icp_sums(const double* src, const int32_t* index, int n, const double* tgt, double* partial, uint32_t* ticket,
+                                   double* sums, void* stream) {
+    MVS_REQUIRE(src && index && tgt && partial && ticket && sums, "pc_icp_sums: null pointer");
+    MVS_REQUIRE(n >= 1, "pc_icp_sums: 1 <= n < 2^31 source points");
+    const int nb = blocks_for(n) < kSumBlocks ? blocks_for(n) : kSumBlocks;
+    pc_icp_sums_a_kernel<<<nb, kThreads, 0, (cudaStream_t)stream>>>(src, index, n, tgt, partial, sums, ticket);
+    MVS_CHECK_LAUNCH("pc_icp_sums_a");
+    pc_icp_sums_b_kernel<<<nb, kThreads, 0, (cudaStream_t)stream>>>(src, index, n, tgt, partial, sums, ticket + 1);
+    MVS_CHECK_LAUNCH("pc_icp_sums_b");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_transform64(double* xyz, int n, const double* affine12_host, float* xyz_f32, void* stream) {
+    MVS_REQUIRE(xyz && affine12_host && xyz_f32, "pc_transform64: null pointer");
+    MVS_REQUIRE(n >= 1, "pc_transform64: 1 <= n < 2^31 points");
+    Affine A{};
+    for (int t = 0; t < 12; ++t) {
+        MVS_REQUIRE(isfinite(affine12_host[t]), "pc_transform64: the transform must be finite");
+        A.a[t] = affine12_host[t];
+    }
+    pc_transform64_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(xyz, n, A, xyz_f32);
+    MVS_CHECK_LAUNCH("pc_transform64");
     return MVSB200_OK;
 }

@@ -14,6 +14,7 @@ F32, BF16 = 0, 1
 VIEW_PARAM_FLOATS = 16
 FUSION_CAM_FLOATS, FUSION_BLOCK_PIXELS, FUSION_MAX_SOURCES = 32, 128, 16     # MVSB200_FUSION_* of include/mvs_b200.h
 PC_MAX_CELLS = 1 << 28                                                       # MVSB200_PC_MAX_CELLS
+PC_ICP_BLOCKS, PC_ICP_SUMS = 1024, 18                                        # MVSB200_PC_ICP_*
 
 _c = ctypes
 _P, _I = _c.c_void_p, _c.c_int
@@ -96,11 +97,14 @@ _SIGNATURES = {
     "mvsb200_pc_grid_keys": (_I, [_P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _P, _P]),
     "mvsb200_pc_grid_cells": (_I, [_P, _P, _P, _I, _P, _P, _P, _P]),
     "mvsb200_pc_nearest": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _P, _P]),
+    "mvsb200_pc_nearest_index": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _P, _P, _P]),
     "mvsb200_pc_thin_neighbours": (_I, [_P, _P, _P, _I] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_double, _P, _P, _P, _P]),
     "mvsb200_pc_thin_round": (_I, [_P, _P, _P, _P, _I, _P, _P]),
     "mvsb200_pc_transform_crop": (_I, [_P, _I, _P, _P, _I, _I, _c.c_double, _c.c_double, _P, _P, _P]),
     "mvsb200_pc_voxel_keys": (_I, [_P, _I] + [_c.c_double] * 4 + [_c.c_int64] * 3 + [_P, _P]),
     "mvsb200_pc_voxel_mean": (_I, [_P, _P, _P, _I, _P, _P, _P]),
+    "mvsb200_pc_icp_sums": (_I, [_P, _P, _I, _P, _P, _P, _P, _P]),
+    "mvsb200_pc_transform64": (_I, [_P, _I, _P, _P, _P]),
 }
 
 _lib = None

@@ -133,6 +133,27 @@ def nearest_distance(query, target, max_dist, *, grid=None):
     return out
 
 
+def nearest_index_into(q, g, max_dist, dist, index):
+    """The index-returning search of the fp32 CUDA points q [n, 3], n >= 1, on the grid g, into dist fp32 [n] and index int32 [n]."""
+    with _timed("pc_nearest_index"):
+        _lib.call("mvsb200_pc_nearest_index", q.data_ptr(), q.shape[0], g.pts.data_ptr(), g.cells.data_ptr(), g.blocks.data_ptr(),
+                  *g.args(), float(g.slack()), float(max_dist), dist.data_ptr(), index.data_ptr(), _stream())
+
+
+def nearest_neighbour(query, target, max_dist, *, grid=None):
+    """nearest_distance, and which target point it is -> (dist fp32 [n], index int64 [n]): index[i] is the row of `target` nearest to
+    query[i] (the smaller row on an exact tie of the fp32 distance), -1 where dist[i] is +inf.  Same search, same distances."""
+    q = _cloud(query, "query")
+    t = _cloud(target, "target")
+    max_dist = _positive(max_dist, "max_dist")
+    n, m = q.shape[0], t.shape[0]
+    dist = torch.full((n,), float("inf"), dtype=torch.float32, device=q.device)
+    index = torch.full((n,), -1, dtype=torch.int32, device=q.device)
+    if n and m:
+        nearest_index_into(q, grid if grid is not None else build_grid(t), max_dist, dist, index)
+    return dist, index.long()
+
+
 def _order(order, seed, n):
     if order is None:
         return torch.randperm(n, generator=torch.Generator().manual_seed(int(seed)))

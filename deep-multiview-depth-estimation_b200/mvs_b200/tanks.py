@@ -7,8 +7,14 @@ ComputePointCloudDistance); DESIGN §4 K9 states the contract and where it diffe
     gt, crop, trans = load_tnt_eval("/data/tnt", "Barn")
     out = evaluate_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, trans, tau=0.01)
 
-The toolbox's registration (RANSAC + ICP of the camera trajectory) is not part of it: the reconstruction must already be in the
-frame `transform` maps to the ground truth's, as one made with T&T's own COLMAP cameras and its `_trans.txt` is.
+`transform` is used as given.  The toolbox first refines `_trans.txt` with three ICP stages; that is
+mvs_b200.register_tanks_and_temples (mvs_b200/registration.py), whose `transformation` this takes unchanged:
+
+    reg = register_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, trans, tau=0.01)
+    out = evaluate_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, reg["transformation"], tau=0.01)
+
+The toolbox's RANSAC trajectory alignment is not provided: the reconstruction must start in a frame `transform` maps near the
+ground truth's, as one made with T&T's own COLMAP cameras and its `_trans.txt` is.
 
 The hot paths are kernels of this library: the fp64 transform and polygon crop, the voxel keys and sequential fp64 voxel means,
 and K8's grid and exact capped nearest search.  Torch does the plumbing only: compaction, the stable sort, segment bounds, the

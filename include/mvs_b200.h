@@ -494,6 +494,12 @@ int mvsb200_pc_nearest(const float* query, int n, const float* pts, const int32_
                        float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, float* dist,
                        void* stream);
 
+/* The same search, also writing index[n] int32: the original index (position in the grid's input cloud) of the nearest point, the
+ * smaller index on an exact tie of the squared fp32 distance, -1 where dist is +inf.  mvsb200_pc_nearest's kernel is unchanged. */
+int mvsb200_pc_nearest_index(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
+                             float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, float* dist,
+                             int32_t* index, void* stream);
+
 /* Greedy minimum-distance thinning (reducePts_haa for a given visiting order) as parallel rounds, on a grid with cell >= dst built
  * over the cloud itself.  rank_sorted [m] int32: the position in the visiting order of each sorted point.  offsets == NULL: counts
  * [m] = the number of points of lower rank within dst (|p - q| <= dst in fp64 on the fp32 coordinates); otherwise list[offsets[s]
@@ -525,6 +531,20 @@ int mvsb200_pc_voxel_keys(const double* xyz, int n, double ox, double oy, double
                           int64_t* keys, void* stream);
 int mvsb200_pc_voxel_mean(const double* xyz, const int64_t* perm, const int64_t* offsets, int n_voxels, double* mean,
                           float* mean_f32, void* stream);
+
+/* ---- K9 registration: the ICP of the toolbox's three registration stages ----------------------------------------------------
+ * icp_sums: the Umeyama sums of the correspondences i -> index[i] >= 0 (index[i] < 0: none) of src [n, 3] fp64 into tgt [m, 3]
+ * fp64, two launches, deterministic (fixed split over min(ceil(n / 256), MVSB200_PC_ICP_BLOCKS) blocks, fixed fp64 trees, no float
+ * atomics).  sums [MVSB200_PC_ICP_SUMS] fp64 (device): [0] c, [1] sum |s - t|^2, [2..4] sum s, [5..7] sum t, then, about the means
+ * mu = sum / c read back from [2..7] on the device, [8..16] sum (t - mu_t)(s - mu_s)^T row-major, [17] sum |s - mu_s|^2.
+ * partial: MVSB200_PC_ICP_BLOCKS * 10 fp64 of scratch; ticket: 2 uint32, ZEROED by the caller once (every call leaves them 0).
+ * transform64: in place, p = A [p; 1] for the fp64 points xyz [n, 3] in transform_crop's operation order, and xyz_f32 [n, 3] its fp32
+ * rounding; affine12_host as for transform_crop (HOST, not NULL). */
+#define MVSB200_PC_ICP_BLOCKS 1024
+#define MVSB200_PC_ICP_SUMS 18
+int mvsb200_pc_icp_sums(const double* src, const int32_t* index, int n, const double* tgt, double* partial, uint32_t* ticket,
+                        double* sums, void* stream);
+int mvsb200_pc_transform64(double* xyz, int n, const double* affine12_host, float* xyz_f32, void* stream);
 
 #ifdef __cplusplus
 }

@@ -3,9 +3,12 @@
     python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 [--out result.json]
 
 --tnt is the directory of T&T's evaluation data, one sub-directory per scene with {scene}.ply, {scene}.json and {scene}_trans.txt
-(INTEGRATION.md §2).  The reconstruction must be in the frame of T&T's COLMAP cameras: the toolbox's trajectory registration is not
-run.  --tau is the scene's threshold (the toolbox's table of per-scene values is not shipped).  Prints one JSON line: precision,
-recall, fscore, the counts, and the histogram edges and cumulative curves."""
+(INTEGRATION.md §2).  The reconstruction must be in the frame of T&T's COLMAP cameras, or --init must map it near the ground truth:
+the toolbox's RANSAC trajectory alignment is not run.  --register first refines that alignment with the toolbox's three ICP stages
+(mvs_b200.register_tanks_and_temples) and evaluates under the refined transform, as the toolbox does; without it {scene}_trans.txt
+(or --init) is used as given.  --tau is the scene's threshold (the toolbox's table of per-scene values is not shipped).  Prints one
+JSON line: precision, recall, fscore, the counts, and the histogram edges and cumulative curves; with --register also a
+`registration` record (the refined transform and, per stage, its sizes, iterations, fitness, rmse and transform)."""
 import argparse
 import json
 import os
@@ -30,12 +33,24 @@ def main(argv=None):
     ap.add_argument("--stretch", type=float, default=tanks.STRETCH, help="the histograms span [0, stretch * tau)")
     ap.add_argument("--out", help="also write the result as JSON to this file")
     ap.add_argument("--device", default="cuda:0")
+    ap.add_argument("--register", action="store_true", help="refine the alignment with the toolbox's three ICP stages first")
+    ap.add_argument("--init", help="a 4 x 4 text file to start from instead of {scene}_trans.txt")
     a = ap.parse_args(argv)
     xyz, _ = mvs_b200.read_ply(a.ply)
     gt, crop, trans = mvs_b200.load_tnt_eval(a.tnt, a.scene)
+    if a.init:
+        trans = np.loadtxt(a.init, dtype=np.float64)
     dev = torch.device(a.device)
-    r = mvs_b200.evaluate_tanks_and_temples(xyz.to(dev), gt.to(dev), crop, trans, a.tau, stretch=a.stretch)
+    xyz, gt = xyz.to(dev), gt.to(dev)
+    reg = None
+    if a.register:
+        reg = mvs_b200.register_tanks_and_temples(xyz, gt, crop, trans, a.tau)
+        trans = reg["transformation"]
+    r = mvs_b200.evaluate_tanks_and_temples(xyz, gt, crop, trans, a.tau, stretch=a.stretch)
     r = {"scene": a.scene, "ply": a.ply, **{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in r.items()}}
+    if reg is not None:
+        r["registration"] = {"transformation": reg["transformation"].tolist(), "init": reg["init"].tolist(),
+                             "stages": [{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in st.items()} for st in reg["stages"]]}
     print(json.dumps(r))
     if a.out:
         with open(a.out, "w") as f:
