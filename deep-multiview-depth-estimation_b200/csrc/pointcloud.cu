@@ -492,6 +492,208 @@ __global__ void __launch_bounds__(kThreads) pc_transform64_kernel(double* __rest
     }
 }
 
+// ---- K9 trajectory alignment: the toolbox's RANSAC over camera centres (DESIGN §4 "K9 trajectory alignment") --------------------
+// Correspondences i <-> i of src [n, 3] (the camera centres to register) and tgt [n, 3] (the reference centres), fp64.
+//   pc_ransac_hyp_kernel     one thread per hypothesis h: its ransac_n counter-based draws, Eigen's Umeyama on them with a
+//                            one-sided Jacobi SVD, then good / error2 over every correspondence, staged through shared memory in
+//                            tiles that every thread of the block reads at the same address
+//   pc_ransac_select_kernel  one block: the lexicographic best (max good, min rmse, min h) in a fixed strided scan and a fixed tree;
+//                            the comparison is a total order, so the winner does not depend on the split
+
+constexpr int kHypThreads = 128;
+constexpr int kAlignTile = 256;
+constexpr int kSelectThreads = 256;
+constexpr int kJacobiSweeps = 16;
+constexpr int kMaxSample = MVSB200_PC_RANSAC_MAX_SAMPLE;
+
+// draw j of hypothesis h: a SplitMix64 step from seed at counter h * ransac_n + j + 1, reduced mod n
+__device__ __forceinline__ int ransac_draw(uint64_t seed, int h, int ransac_n, int j, int n) {
+    uint64_t z = seed + ((uint64_t)h * (uint64_t)ransac_n + (uint64_t)j + 1ull) * 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return (int)((z ^ (z >> 31)) % (uint64_t)n);
+}
+
+// one Jacobi rotation of columns P, Q of B = Sigma V (b[column][row]) that makes them orthogonal; V accumulates it
+template <int P, int Q>
+__device__ __forceinline__ bool jacobi_pair(double (&b)[3][3], double (&v)[3][3]) {
+    const double alpha = b[P][0] * b[P][0] + b[P][1] * b[P][1] + b[P][2] * b[P][2];
+    const double beta = b[Q][0] * b[Q][0] + b[Q][1] * b[Q][1] + b[Q][2] * b[Q][2];
+    const double gamma = b[P][0] * b[Q][0] + b[P][1] * b[Q][1] + b[P][2] * b[Q][2];
+    if (!(fabs(gamma) > 1e-15 * sqrt(alpha * beta))) return false;
+    const double zeta = (beta - alpha) / (2.0 * gamma);
+    const double t = copysign(1.0, zeta) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+    const double c = 1.0 / sqrt(1.0 + t * t), s = c * t;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        const double bp = b[P][r], bq = b[Q][r], vp = v[P][r], vq = v[Q][r];
+        b[P][r] = c * bp - s * bq, b[Q][r] = s * bp + c * bq;
+        v[P][r] = c * vp - s * vq, v[Q][r] = s * vp + c * vq;
+    }
+    return true;
+}
+
+// Eigen's umeyama(src^T, dst^T, with_scaling) on the pairs drawn for hypothesis h -> T, rows 0..2 of [cR | t].  False (T
+// untouched) when the draws hold fewer than 3 distinct indices.  Sigma = (1/k) sum (t - mu_t)(s - mu_s)^T = B V^T after the
+// sweeps, with V a product of rotations (det V = +1); for the column k of smallest norm and (i, j, k) a cyclic order,
+// u_i = b_i / |b_i|, u_j = b_j / |b_j| and w = u_i x u_j give R = U S V^T = u_i v_i^T + u_j v_j^T + w v_k^T and
+// tr(D S) = |b_i| + |b_j| + b_k . w, whichever sign the third left singular vector takes.
+__device__ __forceinline__ bool ransac_umeyama(const double* __restrict__ src, const double* __restrict__ tgt, int n, uint64_t seed,
+                                               int h, int rn, int with_scaling, double (&T)[12]) {
+    const int a = ransac_draw(seed, h, rn, 0, n);
+    int b2 = -1;
+    bool three = false;
+    for (int j = 1; j < rn; ++j) {
+        const int i = ransac_draw(seed, h, rn, j, n);
+        if (i != a) {
+            if (b2 < 0) b2 = i;
+            else three |= i != b2;
+        }
+    }
+    if (!three) return false;
+    const double inv = 1.0 / (double)rn;
+    double ms[3] = {0.0, 0.0, 0.0}, mt[3] = {0.0, 0.0, 0.0};
+    for (int j = 0; j < rn; ++j) {
+        const size_t i = (size_t)ransac_draw(seed, h, rn, j, n);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) ms[r] += __ldg(src + 3 * i + r), mt[r] += __ldg(tgt + 3 * i + r);
+    }
+#pragma unroll
+    for (int r = 0; r < 3; ++r) ms[r] *= inv, mt[r] *= inv;
+    double b[3][3] = {}, var = 0.0;                 // b[q][r] = Sigma[r][q]: column q
+    for (int j = 0; j < rn; ++j) {
+        const size_t i = (size_t)ransac_draw(seed, h, rn, j, n);
+        double ds[3], dt[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) ds[r] = __ldg(src + 3 * i + r) - ms[r], dt[r] = __ldg(tgt + 3 * i + r) - mt[r];
+#pragma unroll
+        for (int q = 0; q < 3; ++q)
+#pragma unroll
+            for (int r = 0; r < 3; ++r) b[q][r] += dt[r] * ds[q];
+        var += ds[0] * ds[0] + ds[1] * ds[1] + ds[2] * ds[2];
+    }
+#pragma unroll
+    for (int q = 0; q < 3; ++q)
+#pragma unroll
+        for (int r = 0; r < 3; ++r) b[q][r] *= inv;
+    var *= inv;
+    double v[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+        bool rotated = jacobi_pair<0, 1>(b, v);
+        rotated |= jacobi_pair<0, 2>(b, v);
+        rotated |= jacobi_pair<1, 2>(b, v);
+        if (!rotated) break;
+    }
+    double sig[3];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) sig[q] = sqrt(b[q][0] * b[q][0] + b[q][1] * b[q][1] + b[q][2] * b[q][2]);
+    const int k = sig[2] <= sig[0] && sig[2] <= sig[1] ? 2 : sig[1] <= sig[0] ? 1 : 0;
+    // selects, not b[(k + 1) % 3]: a run-time index would put the matrices in a local-memory stack frame
+    double ui[3], uj[3], vi[3], vj[3], vk[3], bk[3];
+    const double si = k == 0 ? sig[1] : k == 1 ? sig[2] : sig[0], sj = k == 0 ? sig[2] : k == 1 ? sig[0] : sig[1];
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        ui[r] = (k == 0 ? b[1][r] : k == 1 ? b[2][r] : b[0][r]) / si;
+        uj[r] = (k == 0 ? b[2][r] : k == 1 ? b[0][r] : b[1][r]) / sj;
+        bk[r] = k == 0 ? b[0][r] : k == 1 ? b[1][r] : b[2][r];
+        vi[r] = k == 0 ? v[1][r] : k == 1 ? v[2][r] : v[0][r];
+        vj[r] = k == 0 ? v[2][r] : k == 1 ? v[0][r] : v[1][r];
+        vk[r] = k == 0 ? v[0][r] : k == 1 ? v[1][r] : v[2][r];
+    }
+    const double w[3] = {ui[1] * uj[2] - ui[2] * uj[1], ui[2] * uj[0] - ui[0] * uj[2], ui[0] * uj[1] - ui[1] * uj[0]};
+    const double c = with_scaling ? (si + sj + (bk[0] * w[0] + bk[1] * w[1] + bk[2] * w[2])) / var : 1.0;
+#pragma unroll
+    for (int r = 0; r < 3; ++r) {
+        double R[3];
+#pragma unroll
+        for (int q = 0; q < 3; ++q) R[q] = ui[r] * vi[q] + uj[r] * vj[q] + w[r] * vk[q];
+        T[4 * r] = c * R[0], T[4 * r + 1] = c * R[1], T[4 * r + 2] = c * R[2];
+        T[4 * r + 3] = mt[r] - c * (R[0] * ms[0] + R[1] * ms[1] + R[2] * ms[2]);
+    }
+    return true;
+}
+
+__global__ void __launch_bounds__(kHypThreads) pc_ransac_hyp_kernel(const double* __restrict__ src, const double* __restrict__ tgt, int n,
+                                                                   int n_hyp, int rn, double max_dist2, int with_scaling, uint64_t seed,
+                                                                   int32_t* __restrict__ good_out, double* __restrict__ error2_out,
+                                                                   double* __restrict__ trans_out, int32_t* __restrict__ samples) {
+    __shared__ double ss[3][kAlignTile], st[3][kAlignTile];
+    const int h = blockIdx.x * kHypThreads + threadIdx.x;
+    double T[12];
+    bool active = false;
+    if (h < n_hyp) {
+        active = ransac_umeyama(src, tgt, n, seed, h, rn, with_scaling, T);
+        if (samples)
+            for (int j = 0; j < rn; ++j) samples[(size_t)h * rn + j] = ransac_draw(seed, h, rn, j, n);
+#pragma unroll
+        for (int e = 0; e < 12; ++e) trans_out[(size_t)h * 12 + e] = active ? T[e] : __longlong_as_double(0x7ff8000000000000ll);
+    }
+    int good = 0;
+    double error2 = 0.0;
+    for (long long base = 0; base < n; base += kAlignTile) {
+        const int cnt = n - base < kAlignTile ? (int)(n - base) : kAlignTile;
+        __syncthreads();
+        for (int t = threadIdx.x; t < 3 * cnt; t += kHypThreads) {
+            const int p = t / 3, r = t - 3 * p;
+            ss[r][p] = __ldg(src + 3 * base + t);
+            st[r][p] = __ldg(tgt + 3 * base + t);
+        }
+        __syncthreads();
+        if (!active) continue;
+        for (int p = 0; p < cnt; ++p) {
+            const double x = ss[0][p], y = ss[1][p], z = ss[2][p];
+            double d[3];
+#pragma unroll
+            for (int r = 0; r < 3; ++r)
+                d[r] = __dsub_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(T[4 * r], x), __dmul_rn(T[4 * r + 1], y)), __dmul_rn(T[4 * r + 2], z)),
+                                           T[4 * r + 3]), st[r][p]);
+            const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(d[0], d[0]), __dmul_rn(d[1], d[1])), __dmul_rn(d[2], d[2]));
+            if (d2 < max_dist2) ++good, error2 = __dadd_rn(error2, d2);
+        }
+    }
+    if (h < n_hyp) good_out[h] = good, error2_out[h] = error2;
+}
+
+struct Candidate {
+    int good, h;
+    double rmse;
+};
+
+// a beats b: more inliers, or as many with a smaller rmse, or both equal and an earlier hypothesis
+__device__ __forceinline__ bool beats(const Candidate& a, const Candidate& b) {
+    return a.good > b.good || (a.good == b.good && (a.rmse < b.rmse || (a.rmse == b.rmse && a.h < b.h)));
+}
+
+// record: [0] h (-1: no hypothesis has an inlier), [1] good, [2] error2, [3] rmse, [4..15] T (rows 0..2; the identity for h = -1),
+// [16..16 + rn) the winner's draws
+__global__ void __launch_bounds__(kSelectThreads) pc_ransac_select_kernel(const int32_t* __restrict__ good, const double* __restrict__ error2,
+                                                                         const double* __restrict__ trans, int n_hyp, int n, int rn,
+                                                                         uint64_t seed, double* __restrict__ record) {
+    __shared__ int sg[kSelectThreads], sh[kSelectThreads];
+    __shared__ double sr[kSelectThreads];
+    const int t = threadIdx.x;
+    Candidate best{0, -1, 0.0};
+    for (int h = t; h < n_hyp; h += kSelectThreads) {
+        const int g = good[h];
+        if (g == 0) continue;
+        const Candidate c{g, h, __dsqrt_rn(__ddiv_rn(error2[h], (double)g))};
+        if (beats(c, best)) best = c;
+    }
+    sg[t] = best.good, sh[t] = best.h, sr[t] = best.rmse;
+    __syncthreads();
+    for (int w = kSelectThreads / 2; w > 0; w >>= 1) {
+        if (t < w) {
+            const Candidate o{sg[t + w], sh[t + w], sr[t + w]};
+            if (beats(o, Candidate{sg[t], sh[t], sr[t]})) sg[t] = o.good, sh[t] = o.h, sr[t] = o.rmse;
+        }
+        __syncthreads();
+    }
+    const int h = sh[0];
+    if (t == 0) record[0] = (double)h, record[1] = (double)sg[0], record[2] = h < 0 ? 0.0 : error2[h], record[3] = sr[0];
+    if (t < 12) record[4 + t] = h < 0 ? (t % 5 == 0 ? 1.0 : 0.0) : trans[(size_t)h * 12 + t];
+    if (t < rn) record[16 + t] = h < 0 ? -1.0 : (double)ransac_draw(seed, h, rn, t, n);
+}
+
 int blocks_for(int n) { return (n + kThreads - 1) / kThreads; }
 
 bool grid_ok(float cell, int nbx, int nby, int nbz) {
@@ -651,5 +853,21 @@ extern "C" int mvsb200_pc_transform64(double* xyz, int n, const double* affine12
     }
     pc_transform64_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(xyz, n, A, xyz_f32);
     MVS_CHECK_LAUNCH("pc_transform64");
+    return MVSB200_OK;
+}
+
+extern "C" int mvsb200_pc_ransac_align(const double* src, const double* tgt, int n, int n_hyp, int ransac_n, double max_dist2,
+                                       int with_scaling, uint64_t seed, int32_t* good, double* error2, double* trans, int32_t* samples,
+                                       double* record, void* stream) {
+    MVS_REQUIRE(src && tgt && good && error2 && trans && record, "pc_ransac_align: null pointer");
+    MVS_REQUIRE(n >= 1, "pc_ransac_align: 1 <= n < 2^31 correspondences");
+    MVS_REQUIRE(n_hyp >= 1, "pc_ransac_align: 1 <= n_hyp < 2^31 hypotheses");
+    MVS_REQUIRE(ransac_n >= 3 && ransac_n <= kMaxSample, "pc_ransac_align: 3 <= ransac_n <= %d, got %d", kMaxSample, ransac_n);
+    MVS_REQUIRE(max_dist2 > 0.0 && isfinite(max_dist2), "pc_ransac_align: max_dist2 > 0 (finite)");
+    pc_ransac_hyp_kernel<<<(n_hyp + kHypThreads - 1) / kHypThreads, kHypThreads, 0, (cudaStream_t)stream>>>(
+        src, tgt, n, n_hyp, ransac_n, max_dist2, with_scaling != 0, seed, good, error2, trans, samples);
+    MVS_CHECK_LAUNCH("pc_ransac_hyp");
+    pc_ransac_select_kernel<<<1, kSelectThreads, 0, (cudaStream_t)stream>>>(good, error2, trans, n_hyp, n, ransac_n, seed, record);
+    MVS_CHECK_LAUNCH("pc_ransac_select");
     return MVSB200_OK;
 }

@@ -18,8 +18,9 @@ from .ops import depth_confidence  # noqa: F401
 from .fusion import fuse_depth_maps, visibility_fusion, infer_scene, write_ply, read_ply  # noqa: F401
 from .evaluation import thin_points, nearest_distance, nearest_neighbour, evaluate_point_cloud, load_dtu_eval  # noqa: F401
 from .tanks import (CropVolume, read_crop_volume, crop_points, voxel_down_sample, evaluate_tanks_and_temples,  # noqa: F401
-                    load_tnt_eval)
-from .registration import uniform_down_sample, icp_point_to_point, register_tanks_and_temples  # noqa: F401
+                    load_tnt_eval, Mapping, read_trajectory, write_trajectory, read_mapping, load_tnt_trajectory, camera_poses)
+from .registration import (uniform_down_sample, icp_point_to_point, register_tanks_and_temples,  # noqa: F401
+                           trajectory_points, align_trajectory)
 
 __all__ = ["homography_warping", "assemble_cost_volume", "extract_depth_map", "CostVolumeReg",
            "WarpedFeatureVolumes", "PlaneSweep", "warp_variance", "warp_materialize", "softmax_depth",
@@ -28,4 +29,6 @@ __all__ = ["homography_warping", "assemble_cost_volume", "extract_depth_map", "C
            "nearest_neighbour", "evaluate_point_cloud", "load_dtu_eval", "CropVolume", "read_crop_volume", "crop_points",
            "voxel_down_sample",
            "evaluate_tanks_and_temples", "load_tnt_eval", "uniform_down_sample", "icp_point_to_point", "register_tanks_and_temples",
+           "Mapping", "read_trajectory", "write_trajectory", "read_mapping", "load_tnt_trajectory", "camera_poses",
+           "trajectory_points", "align_trajectory",
            "MvsB200Error", "launch_count", "load_library"]

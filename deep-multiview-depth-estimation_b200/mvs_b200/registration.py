@@ -1,16 +1,21 @@
-"""Registration of a reconstruction to the Tanks and Temples ground truth: the three ICP stages the official toolbox runs before it
-scores a cloud (python_toolbox/evaluation: run.py, registration.py::registration_vol_ds / registration_unif), with Open3D 0.10's
-point-to-point ICP with scaling (RegistrationICP, TransformationEstimationPointToPoint).  DESIGN §4 "K9 registration" states the
-contract and where it differs.
+"""Registration of a reconstruction to the Tanks and Temples ground truth: the official toolbox's (python_toolbox/evaluation: run.py,
+registration.py) RANSAC trajectory alignment over camera centres (trajectory_alignment, with Open3D 0.10's
+RegistrationRANSACBasedOnCorrespondence) and the three ICP stages it runs before it scores a cloud (registration_vol_ds /
+registration_unif, with Open3D 0.10's point-to-point ICP with scaling, RegistrationICP, TransformationEstimationPointToPoint).
+DESIGN §4 "K9 trajectory alignment" and "K9 registration" state the contracts and where they differ.
 
     gt, crop, trans = load_tnt_eval("/data/tnt", "Barn")
-    reg = register_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, trans, tau=0.01)
+    ref, mapping = load_tnt_trajectory("/data/tnt", "Barn")
+    _, poses = read_trajectory("Barn.log")                      # the cameras of the reconstruction, in its own frame
+    init = align_trajectory(poses, ref, trans, mapping=mapping)["transformation"]
+    reg = register_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, init, tau=0.01)
     out = evaluate_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, reg["transformation"], tau=0.01)
 
-The hot path is kernels of this library: per ICP iteration the capped nearest search with indices, the Umeyama sums in two
-deterministic fp64 passes and the fp64 update of the source; K9's transform, crop and voxel down-sampling per stage.  The host
-solves the 3 x 3 SVD and composes the 4 x 4 matrices in fp64 numpy from one read-back of 18 sums per iteration.  There is no CPU
-path."""
+For a reconstruction already in T&T's COLMAP frame, `trans` itself is the init.  The hot path is kernels of this library: for the
+alignment, one thread per RANSAC hypothesis (draws, Umeyama with an fp64 Jacobi SVD, scoring) and a deterministic selection; per ICP
+iteration the capped nearest search with indices, the Umeyama sums in two deterministic fp64 passes and the fp64 update of the
+source; K9's transform, crop and voxel down-sampling per stage.  The host reads camera centres, solves ICP's 3 x 3 SVD and composes
+the 4 x 4 matrices in fp64 numpy.  There is no CPU path."""
 from __future__ import annotations
 
 import math
@@ -24,6 +29,7 @@ from .ops import _stream, _timed
 from .tanks import CropVolume, _crop_volume, crop_points, voxel_down_sample
 
 MAX_POINT_NUMBER = 4_000_000                     # the toolbox's MAX_POINT_NUMBER: stage 3's uniform down-sampling target
+MAX_DENSE_POSES = 1600                           # a trajectory with more poses is every video frame: it is sampled by the mapping
 RELATIVE_FITNESS, RELATIVE_RMSE, MAX_ITERATION = 1e-6, 20.0, 30     # ICPConvergenceCriteria(1e-6, 20) as the toolbox writes it
 
 
@@ -220,3 +226,94 @@ def register_tanks_and_temples(xyz, gt, crop, init, tau, *, max_points=MAX_POINT
                    fitness=r["fitness"], inlier_rmse=r["inlier_rmse"], correspondences=r["correspondences"], transformation=T)
         stages.append(rec)
     return {"transformation": T, "init": T0, "tau": tau, "stages": stages}
+
+
+def _poses(p, what):
+    a = p.detach().cpu().numpy() if isinstance(p, torch.Tensor) else p
+    try:
+        a = np.asarray(a, dtype=np.float64)
+    except (TypeError, ValueError):
+        _fail(f"{what} must be numeric")
+    if a.ndim != 3 or a.shape[1:] != (4, 4):
+        _fail(f"{what}: poses [n, 4, 4] expected, got shape {a.shape}")
+    if not np.isfinite(a).all():
+        _fail(f"{what} must be finite")
+    return a
+
+
+def trajectory_points(poses, reference_poses, gt_trans, mapping=None):
+    """The point sets of the toolbox's trajectory_alignment -> (source fp64 [k, 3], reference fp64 [k, 3]), paired row by row:
+    reference = the centres pose[:3, 3] of reference_poses mapped by gt_trans in K9 step 1's operation order; source = the centres
+    of `poses`, or, when there are more than MAX_DENSE_POSES of them, of poses[m[1] - 1] for each row m of the mapping (a
+    tanks.Mapping or rows [k, 2]), cut to the reference's length.  Refused: a trajectory over MAX_DENSE_POSES poses without a
+    mapping, a mapping row outside 1..len(poses), and fewer source points than reference points."""
+    P = _poses(poses, "poses")
+    ref = _poses(reference_poses, "reference_poses")
+    A = _matrix(gt_trans, "gt_trans")
+    if len(P) > MAX_DENSE_POSES:
+        if mapping is None:
+            _fail(f"a trajectory of {len(P)} > {MAX_DENSE_POSES} poses is every video frame: the scene's mapping is needed")
+        rows = np.asarray(getattr(mapping, "rows", mapping))
+        if rows.ndim != 2 or rows.shape[1] != 2 or not np.array_equal(rows, rows.astype(np.int64)):
+            _fail(f"mapping: integer rows [k, 2] expected, got shape {rows.shape}")
+        frames = rows[:, 1].astype(np.int64)
+        if len(frames) and (frames.min() < 1 or frames.max() > len(P)):
+            _fail(f"mapping: frame numbers must lie in 1..{len(P)} (1-based), got {frames.min()}..{frames.max()}")
+        P = P[frames - 1]
+    c = ref[:, :3, 3]
+    target = np.stack([((A[r, 0] * c[:, 0] + A[r, 1] * c[:, 1]) + A[r, 2] * c[:, 2]) + A[r, 3] for r in range(3)], 1)
+    if len(P) < len(target):
+        _fail(f"{len(P)} camera centres to register but {len(target)} reference centres: every reference centre needs its pair")
+    return np.ascontiguousarray(P[:len(target), :3, 3]), target
+
+
+def align_trajectory(poses, reference_poses, gt_trans, *, mapping=None, max_correspondence_distance=0.2, ransac_n=6,
+                     max_iteration=100000, with_scaling=True, seed=0, return_details=False):
+    """The toolbox's trajectory_alignment: RANSAC (Open3D 0.10's RegistrationRANSACBasedOnCorrespondence) over the camera centres
+    of trajectory_points, pair i <-> i.  Hypothesis h < max_iteration draws ransac_n pairs with replacement (counter-based
+    SplitMix64 from `seed`, DESIGN §4), solves Eigen's Umeyama on them and counts the pairs with |T s_i - r_i|^2 <
+    max_correspondence_distance^2: good, and error2 their sum; fitness = good / n, inlier_rmse = sqrt(error2 / good).  Fewer than 3
+    distinct indices in a draw: good = 0.  The result is the hypothesis with the most inliers, then the smallest rmse, then the
+    smallest h; the identity when none has an inlier.  Its ransac_n-point transform is returned as solved, without a refit.
+
+    -> dict with transformation (fp64 4 x 4, maps the reconstruction's frame into the ground truth's: the init of
+    register_tanks_and_temples), fitness, inlier_rmse, inliers, hypothesis (-1: none), sample (its draws), n_correspondences; with
+    return_details also, as CUDA tensors, good int32 [max_iteration], error2 fp64 [max_iteration], transforms fp64
+    [max_iteration, 3, 4] (NaN where no transform was solved) and samples int32 [max_iteration, ransac_n]."""
+    src, tgt = trajectory_points(poses, reference_poses, gt_trans, mapping)
+    d_max = _positive(max_correspondence_distance, "max_correspondence_distance")
+    if isinstance(ransac_n, bool) or int(ransac_n) != ransac_n or not 3 <= int(ransac_n) <= _lib.PC_RANSAC_MAX_SAMPLE:
+        _fail(f"ransac_n must be an integer in 3..{_lib.PC_RANSAC_MAX_SAMPLE}, got {ransac_n!r}")
+    if isinstance(max_iteration, bool) or int(max_iteration) != max_iteration or not 0 <= int(max_iteration) < 2 ** 31:
+        _fail(f"max_iteration must be an integer in 0..2^31 - 1, got {max_iteration!r}")
+    if isinstance(seed, bool) or int(seed) != seed or not 0 <= int(seed) < 2 ** 64:
+        _fail(f"seed must be an integer in 0..2^64 - 1, got {seed!r}")
+    rn, n_hyp, n = int(ransac_n), int(max_iteration), len(src)
+    out = {"transformation": np.eye(4), "fitness": 0.0, "inlier_rmse": 0.0, "inliers": 0, "hypothesis": -1, "sample": [],
+           "n_correspondences": n}
+    dev = torch.device("cuda", torch.cuda.current_device())
+    good = torch.empty(n_hyp, dtype=torch.int32, device=dev)
+    error2 = torch.empty(n_hyp, dtype=torch.float64, device=dev)
+    trans = torch.empty((n_hyp, 3, 4), dtype=torch.float64, device=dev)
+    samples = torch.empty((n_hyp, rn), dtype=torch.int32, device=dev) if return_details else None
+    if n == 0:                                                                # no pair: no hypothesis can be drawn
+        good.zero_(), error2.zero_(), trans.fill_(float("nan"))
+        if samples is not None:
+            samples.fill_(-1)
+    elif n_hyp:
+        s, t = torch.from_numpy(src).to(dev), torch.from_numpy(tgt).to(dev)
+        record = torch.empty(_lib.PC_RANSAC_RECORD, dtype=torch.float64, device=dev)
+        with _timed("pc_ransac_align"):
+            _lib.call("mvsb200_pc_ransac_align", s.data_ptr(), t.data_ptr(), n, n_hyp, rn, d_max * d_max, int(bool(with_scaling)),
+                      int(seed), good.data_ptr(), error2.data_ptr(), trans.data_ptr(), samples.data_ptr() if return_details else None,
+                      record.data_ptr(), _stream())
+        r = record.cpu().numpy()                                              # the one read-back
+        h = int(r[0])
+        if h >= 0:
+            T = np.eye(4)
+            T[:3] = r[4:16].reshape(3, 4)
+            out.update(transformation=T, fitness=float(r[1]) / n, inlier_rmse=float(r[3]), inliers=int(r[1]), hypothesis=h,
+                       sample=[int(v) for v in r[16:16 + rn]])
+    if return_details:
+        out.update(good=good, error2=error2, transforms=trans, samples=samples)
+    return out

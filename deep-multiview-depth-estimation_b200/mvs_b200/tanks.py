@@ -13,8 +13,13 @@ mvs_b200.register_tanks_and_temples (mvs_b200/registration.py), whose `transform
     reg = register_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, trans, tau=0.01)
     out = evaluate_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, reg["transformation"], tau=0.01)
 
-The toolbox's RANSAC trajectory alignment is not provided: the reconstruction must start in a frame `transform` maps near the
-ground truth's, as one made with T&T's own COLMAP cameras and its `_trans.txt` is.
+A reconstruction made with the user's own cameras is first brought near the ground truth by the toolbox's RANSAC over camera
+centres, mvs_b200.align_trajectory, from the user's `.log` trajectory and T&T's COLMAP one (read_trajectory, load_tnt_trajectory):
+
+    poses = camera_poses(R, T)                       # the cameras the reconstruction was made with; write_trajectory(path, poses)
+    ref, mapping = load_tnt_trajectory("/data/tnt", "Barn")
+    init = align_trajectory(poses, ref, trans, mapping=mapping)["transformation"]
+    reg = register_tanks_and_temples(xyz.cuda(), gt.cuda(), crop, init, tau=0.01)
 
 The hot paths are kernels of this library: the fp64 transform and polygon crop, the voxel keys and sequential fp64 voxel means,
 and K8's grid and exact capped nearest search.  Torch does the plumbing only: compaction, the stable sort, segment bounds, the
@@ -288,3 +293,113 @@ def load_tnt_eval(root, scene):
     if trans.shape != (4, 4):
         _fail(f"load_tnt_eval: {paths[2]}: a 4 x 4 matrix expected, got shape {trans.shape}")
     return gt, crop, trans
+
+
+# ---- trajectories (the toolbox's trajectory_io.py and registration.py::read_mapping; DESIGN §4 "K9 trajectory alignment") ----------
+
+class Mapping(NamedTuple):
+    """T&T's {scene}_mapping_reference.txt: rows [n_sampled, 2] int64, where the sparse trajectory takes traj[rows[k, 1] - 1] (the
+    second column is 1-based), and n_total, the frame count the file states (not used by the alignment)."""
+    n_total: int
+    rows: np.ndarray
+
+
+def _lines(path):
+    """The non-blank lines of a text file, each split into its fields, with their 1-based line numbers."""
+    with open(path) as f:
+        return [(k + 1, ln.split()) for k, ln in enumerate(f) if ln.strip()]
+
+
+def _ints(fields, path, line, count):
+    try:
+        v = [int(x) for x in fields]
+    except ValueError:
+        _fail(f"{path}:{line}: integers expected, got {' '.join(fields)!r}")
+    if len(v) != count:
+        _fail(f"{path}:{line}: {count} integers expected, got {len(v)}")
+    return v
+
+
+def read_trajectory(path):
+    """A trajectory file (.log): per camera one line of three integers (metadata, not interpreted) and four lines of its 4 x 4
+    camera-to-world pose -> (metadata int64 [n, 3], poses fp64 [n, 4, 4]).  Blank lines are skipped.  Refused with MvsB200Error: a
+    short block, a line with the wrong number of values, a non-numeric or non-finite value, a pose whose last row is not exactly
+    0 0 0 1."""
+    lines = _lines(path)
+    if len(lines) % 5:
+        _fail(f"{path}: {len(lines)} lines do not make blocks of 5 (metadata and a 4 x 4 pose): the last block is short")
+    meta = np.zeros((len(lines) // 5, 3), np.int64)
+    poses = np.zeros((len(lines) // 5, 4, 4))
+    for b in range(len(meta)):
+        line, fields = lines[5 * b]
+        meta[b] = _ints(fields, path, line, 3)
+        for r in range(4):
+            line, fields = lines[5 * b + 1 + r]
+            try:
+                row = [float(x) for x in fields]
+            except ValueError:
+                _fail(f"{path}:{line}: numbers expected, got {' '.join(fields)!r}")
+            if len(row) != 4 or not np.isfinite(row).all():
+                _fail(f"{path}:{line}: a pose row of 4 finite numbers expected, got {' '.join(fields)!r}")
+            poses[b, r] = row
+        if not np.array_equal(poses[b, 3], [0.0, 0.0, 0.0, 1.0]):
+            _fail(f"{path}: pose {b}: last row exactly 0 0 0 1 expected, got {poses[b, 3].tolist()}")
+    return meta, poses
+
+
+def write_trajectory(path, poses, metadata=None):
+    """Write poses [n, 4, 4] (camera-to-world) as a trajectory file.  metadata [n, 3] integers; default i, i, i + 1 per camera i, as
+    Open3D's LOG writer writes it (the toolbox's reader ignores it).  Values are written with 17 significant digits, so
+    read_trajectory gives back the same fp64 poses."""
+    p = np.asarray(poses, np.float64)
+    if p.ndim != 3 or p.shape[1:] != (4, 4):
+        _fail(f"write_trajectory: poses [n, 4, 4] expected, got shape {p.shape}")
+    m = np.stack([np.arange(len(p))] * 2 + [np.arange(1, len(p) + 1)], 1) if metadata is None else np.asarray(metadata)
+    if m.shape != (len(p), 3) or not np.array_equal(m, np.asarray(m, np.int64)):
+        _fail(f"write_trajectory: metadata [{len(p)}, 3] integers expected, got shape {m.shape}")
+    with open(path, "w") as f:
+        for k in range(len(p)):
+            f.write(" ".join(str(int(v)) for v in m[k]) + "\n")
+            for r in range(4):
+                f.write(" ".join(f"{v:.17g}" for v in p[k, r]) + "\n")
+
+
+def read_mapping(path):
+    """T&T's {scene}_mapping_reference.txt: n_sampled, n_total, then n_sampled lines of two integers -> Mapping.  Refused with
+    MvsB200Error: non-integer values, a row that is not two integers, or a row count other than n_sampled."""
+    lines = _lines(path)
+    if len(lines) < 2:
+        _fail(f"{path}: n_sampled and n_total expected on the first two lines")
+    n_sampled = _ints(lines[0][1], path, lines[0][0], 1)[0]
+    n_total = _ints(lines[1][1], path, lines[1][0], 1)[0]
+    rows = np.array([_ints(f, path, line, 2) for line, f in lines[2:]], np.int64).reshape(-1, 2)
+    if len(rows) != n_sampled:
+        _fail(f"{path}: n_sampled is {n_sampled} but {len(rows)} mapping rows follow")
+    return Mapping(n_total, rows)
+
+
+def load_tnt_trajectory(root, scene):
+    """T&T's reference trajectory of one scene -> (COLMAP poses fp64 [n, 4, 4], Mapping or None), read from
+        {root}/{scene}/{scene}_COLMAP_SfM.log            the camera poses of T&T's COLMAP reconstruction
+        {root}/{scene}/{scene}_mapping_reference.txt     which video frames those cameras are (None when the file is absent)"""
+    d = os.path.join(root, scene)
+    log = os.path.join(d, f"{scene}_COLMAP_SfM.log")
+    if not os.path.exists(log):
+        _fail(f"load_tnt_trajectory: {log} not found")
+    mp = os.path.join(d, f"{scene}_mapping_reference.txt")
+    return read_trajectory(log)[1], (read_mapping(mp) if os.path.exists(mp) else None)
+
+
+def camera_poses(R, T):
+    """MVSNet's world-to-camera extrinsics R [n, 3, 3], T [n, 3] (or [n, 3, 1]) -> camera-to-world poses [R^T | -R^T T; 0 0 0 1]
+    fp64 [n, 4, 4], the poses a trajectory file holds."""
+    R = _finite(R.detach().cpu() if isinstance(R, torch.Tensor) else R, "R")
+    T = _finite(T.detach().cpu() if isinstance(T, torch.Tensor) else T, "T")
+    if R.ndim != 3 or R.shape[1:] != (3, 3) or T.shape not in ((len(R), 3), (len(R), 3, 1)):
+        _fail(f"camera_poses: R [n, 3, 3] and T [n, 3] expected, got {R.shape} and {T.shape}")
+    Rt = R.transpose(0, 2, 1)
+    out = np.zeros((len(R), 4, 4))
+    out[:, :3, :3] = Rt
+    out[:, :3, 3] = -(Rt @ T.reshape(-1, 3, 1))[..., 0]
+    out[:, 3, 3] = 1.0
+    return out

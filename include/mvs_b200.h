@@ -546,6 +546,22 @@ int mvsb200_pc_icp_sums(const double* src, const int32_t* index, int n, const do
                         double* sums, void* stream);
 int mvsb200_pc_transform64(double* xyz, int n, const double* affine12_host, float* xyz_f32, void* stream);
 
+/* ---- K9 trajectory alignment: the toolbox's RANSAC over camera-centre correspondences i <-> i ------------------------------------
+ * ransac_align: n_hyp hypotheses over src [n, 3] (the centres to register) and tgt [n, 3] (the reference centres), fp64 (device).
+ * Hypothesis h draws index j < ransac_n as SplitMix64(seed + (h ransac_n + j + 1) 0x9E3779B97F4A7C15 mod 2^64) mod n, solves
+ * Eigen's Umeyama (with_scaling: the scale, else 1) on those pairs, and scores every pair i: d2 = |T s_i - t_i|^2 (transform_crop's
+ * operation order), good = #(d2 < max_dist2), error2 = the sum of those d2 in pair order.  Fewer than 3 distinct indices: good 0.
+ * Writes good [n_hyp] int32, error2 [n_hyp] fp64, trans [n_hyp, 12] fp64 (rows 0..2 of T; NaN where no transform was solved),
+ * samples [n_hyp, ransac_n] int32 the draws (NULL: not written), and record [MVSB200_PC_RANSAC_RECORD] fp64: [0] the winner h (-1
+ * when no hypothesis has good > 0), [1] its good, [2] error2, [3] rmse = sqrt(error2 / good), [4..15] its trans (the identity for
+ * -1), [16 ..) its ransac_n draws.  The winner has the most inliers, then the smallest rmse, then the smallest h.  Deterministic:
+ * no float atomics.  3 <= ransac_n <= MVSB200_PC_RANSAC_MAX_SAMPLE; two launches. */
+#define MVSB200_PC_RANSAC_MAX_SAMPLE 64
+#define MVSB200_PC_RANSAC_RECORD (16 + MVSB200_PC_RANSAC_MAX_SAMPLE)
+int mvsb200_pc_ransac_align(const double* src, const double* tgt, int n, int n_hyp, int ransac_n, double max_dist2,
+                            int with_scaling, uint64_t seed, int32_t* good, double* error2, double* trans, int32_t* samples,
+                            double* record, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

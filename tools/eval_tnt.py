@@ -2,13 +2,20 @@
 
     python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 [--out result.json]
 
---tnt is the directory of T&T's evaluation data, one sub-directory per scene with {scene}.ply, {scene}.json and {scene}_trans.txt
-(INTEGRATION.md §2).  The reconstruction must be in the frame of T&T's COLMAP cameras, or --init must map it near the ground truth:
-the toolbox's RANSAC trajectory alignment is not run.  --register first refines that alignment with the toolbox's three ICP stages
-(mvs_b200.register_tanks_and_temples) and evaluates under the refined transform, as the toolbox does; without it {scene}_trans.txt
-(or --init) is used as given.  --tau is the scene's threshold (the toolbox's table of per-scene values is not shipped).  Prints one
-JSON line: precision, recall, fscore, the counts, and the histogram edges and cumulative curves; with --register also a
-`registration` record (the refined transform and, per stage, its sizes, iterations, fitness, rmse and transform)."""
+    python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 --traj Barn.log [--seed 0]
+
+--tnt is the directory of T&T's evaluation data, one sub-directory per scene with {scene}.ply, {scene}.json and {scene}_trans.txt,
+and for --traj also {scene}_COLMAP_SfM.log and, for a trajectory of every video frame, {scene}_mapping_reference.txt
+(INTEGRATION.md §2).  --traj runs the toolbox's whole chain: the RANSAC alignment of the reconstruction's camera trajectory (a .log
+file in the reconstruction's frame) to T&T's COLMAP one mapped by {scene}_trans.txt (mvs_b200.align_trajectory, draws seeded by
+--seed), then the three ICP stages from that alignment, then the evaluation; it implies --register and excludes --init.  Without
+--traj the reconstruction must be in the frame of T&T's COLMAP cameras, or --init must map it near the ground truth.  --register
+refines that alignment with the toolbox's three ICP stages (mvs_b200.register_tanks_and_temples) and evaluates under the refined
+transform, as the toolbox does; without it {scene}_trans.txt (or --init) is used as given.  --tau is the scene's threshold (the
+toolbox's table of per-scene values is not shipped).  Prints one JSON line: precision, recall, fscore, the counts, and the
+histogram edges and cumulative curves; with --register also a `registration` record (the refined transform and, per stage, its
+sizes, iterations, fitness, rmse and transform); with --traj also an `alignment` record (the RANSAC transform, fitness, rmse,
+inliers, the winning hypothesis and its sample, the correspondence count and the seed)."""
 import argparse
 import json
 import os
@@ -35,19 +42,33 @@ def main(argv=None):
     ap.add_argument("--device", default="cuda:0")
     ap.add_argument("--register", action="store_true", help="refine the alignment with the toolbox's three ICP stages first")
     ap.add_argument("--init", help="a 4 x 4 text file to start from instead of {scene}_trans.txt")
+    ap.add_argument("--traj", help="the reconstruction's camera trajectory (.log): align it to T&T's first (implies --register)")
+    ap.add_argument("--seed", type=int, help="the seed of the alignment's RANSAC draws (with --traj; default 0)")
     a = ap.parse_args(argv)
+    if a.traj and a.init:
+        ap.error("--traj and --init exclude each other: --traj computes the initial alignment")
+    if a.seed is not None and not a.traj:
+        ap.error("--seed applies to --traj only")
     xyz, _ = mvs_b200.read_ply(a.ply)
     gt, crop, trans = mvs_b200.load_tnt_eval(a.tnt, a.scene)
     if a.init:
         trans = np.loadtxt(a.init, dtype=np.float64)
     dev = torch.device(a.device)
     xyz, gt = xyz.to(dev), gt.to(dev)
-    reg = None
-    if a.register:
+    reg = align = None
+    if a.traj:
+        _, poses = mvs_b200.read_trajectory(a.traj)
+        ref, mapping = mvs_b200.load_tnt_trajectory(a.tnt, a.scene)
+        with torch.cuda.device(dev):
+            align = mvs_b200.align_trajectory(poses, ref, trans, mapping=mapping, seed=a.seed or 0)
+        trans = align["transformation"]
+    if a.register or a.traj:
         reg = mvs_b200.register_tanks_and_temples(xyz, gt, crop, trans, a.tau)
         trans = reg["transformation"]
     r = mvs_b200.evaluate_tanks_and_temples(xyz, gt, crop, trans, a.tau, stretch=a.stretch)
     r = {"scene": a.scene, "ply": a.ply, **{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in r.items()}}
+    if align is not None:
+        r["alignment"] = {**{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in align.items()}, "seed": a.seed or 0}
     if reg is not None:
         r["registration"] = {"transformation": reg["transformation"].tolist(), "init": reg["init"].tolist(),
                              "stages": [{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in st.items()} for st in reg["stages"]]}
