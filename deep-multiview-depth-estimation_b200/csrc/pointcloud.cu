@@ -18,6 +18,8 @@
 //   pc_voxel_mean_kernel     K9: one thread per occupied voxel, the sequential fp64 mean of its stably sorted points
 //   pc_icp_sums_{a,b}_kernel K9 registration: the Umeyama sums of the correspondences in two passes, a deterministic fp64 reduction
 //   pc_transform64_kernel    K9 registration: an fp64 affine update of the source in place, and its fp32 rounding
+//   pc_knn_kernel            K10: one thread per query, the exact k nearest points in the order (d^2, index), capped at max_dist;
+//                            <true>: on the cloud itself, the normal of each point's neighbourhood (fp64 covariance, Jacobi)
 //
 // Nearest search.  Shells r = 0, 1, ... of fine cells around the query's (clamped) cell, up to kFineShells; then shells of coarse
 // blocks, skipping empty blocks, visiting an occupied block by its points (few) or by its fine cells (many).  A shell is entered
@@ -694,6 +696,218 @@ __global__ void __launch_bounds__(kSelectThreads) pc_ransac_select_kernel(const 
     if (t < rn) record[16 + t] = h < 0 ? -1.0 : (double)ransac_draw(seed, h, rn, t, n);
 }
 
+// ---- K10 normals: exact k-nearest neighbours on K8's grid and per-point normals (DESIGN §4 "K10 normals") --------------------------
+// Each thread keeps its list ascending in (d^2, index) in dynamic shared memory laid out [slot][thread] (consecutive threads hit
+// consecutive banks), k * kThreads floats of d^2 then as many ints of index.  kd, kj: the k-th entry once the list is full, and
+// (lim, -1) before, so that "before (kd, kj)" is both the cap d^2 < max_dist^2 and the order test, and kd is the pruning bound.
+
+constexpr int kKnnMax = MVSB200_PC_KNN_MAX;
+
+// pc_nearest_kernel's square root of s, +inf for s >= lim
+__device__ __forceinline__ float root_below(float s, float lim) {
+    float d = kInf;
+    if (s == 0.f) {
+        d = 0.f;
+    } else if (s < lim) {
+        const float y = rsqrtf(s);
+        d = s * y;
+        d = fmaf(0.5f * y, fmaf(-d, d, s), d);
+    }
+    return d;
+}
+
+// a candidate the order test admitted: insertion into the sorted list sd / si (this thread's slot 0) of cnt <= k entries
+__device__ __forceinline__ void knn_insert(float d, int j, float* sd, int* si, int k, int& cnt, float& kd, int& kj) {
+    int p = cnt < k ? cnt : k - 1;
+    for (; p > 0; --p) {
+        const float pd = sd[(p - 1) * kThreads];
+        const int pj = si[(p - 1) * kThreads];
+        if (pd < d || (pd == d && pj < j)) break;
+        sd[p * kThreads] = pd, si[p * kThreads] = pj;
+    }
+    sd[p * kThreads] = d, si[p * kThreads] = j;
+    if (cnt < k) ++cnt;
+    if (cnt == k) kd = sd[(k - 1) * kThreads], kj = si[(k - 1) * kThreads];
+}
+
+// scan_points for the list: the candidates the order test admits are inserted
+__device__ __forceinline__ void knn_scan(const float4* __restrict__ pts, int b, int e, float qx, float qy, float qz, float* sd, int* si,
+                                         int k, int& cnt, float& kd, int& kj) {
+    for (int p = b; p < e; ++p) {
+        const float4 t = __ldg(pts + p);
+        const float d = sq(t.x - qx) + sq(t.y - qy) + sq(t.z - qz);
+        const int j = __float_as_int(t.w);
+        if (d < kd || (d == kd && j < kj)) knn_insert(d, j, sd, si, k, cnt, kd, kj);
+    }
+}
+
+// NORMALS = false: dist / index [n, k].  NORMALS = true: query is also the grid's cloud (index j -> query[3 j ..]); normals [n, 3]
+// from the list, which is never written out.  view_mode 0: none, 1: view[0..2], 2: view[3 i ..].
+template <bool NORMALS>
+__global__ void __launch_bounds__(kThreads, 2) pc_knn_kernel(const float* __restrict__ query, int n, const float4* __restrict__ pts,
+                                                          const int2* __restrict__ cells, const int2* __restrict__ blocks, Grid g,
+                                                          float slack, float max_dist, int k, float* __restrict__ dist,
+                                                          int32_t* __restrict__ index, const double* __restrict__ view, int view_mode,
+                                                          float* __restrict__ normals) {
+    extern __shared__ float knn_smem[];
+    float* sd = knn_smem + threadIdx.x;
+    int* si = reinterpret_cast<int*>(knn_smem + k * kThreads) + threadIdx.x;
+    const int i = blockIdx.x * kThreads + threadIdx.x;
+    if (i >= n) return;
+    const float qx = query[3 * (size_t)i], qy = query[3 * (size_t)i + 1], qz = query[3 * (size_t)i + 2];
+    const int nx = 8 * g.nbx, ny = 8 * g.nby, nz = 8 * g.nbz;
+    const float lim = max_dist * max_dist;
+    int cnt = 0;
+    float kd = lim;
+    int kj = -1;
+    bool reach = true;
+    {
+        const double c = g.cell;
+        const double ex = fmax(fmax((double)g.ox - qx, (double)qx - (g.ox + nx * c)), 0.0);
+        const double ey = fmax(fmax((double)g.oy - qy, (double)qy - (g.oy + ny * c)), 0.0);
+        const double ez = fmax(fmax((double)g.oz - qz, (double)qz - (g.oz + nz * c)), 0.0);
+        reach = ex * ex + ey * ey + ez * ez < (double)max_dist * max_dist;
+    }
+    if (reach) {
+        const float sl = slack + 2.4e-7f * (fabsf(qx) + fabsf(qy) + fabsf(qz));
+        const int cx = cell_of(qx, g.ox, g.inv, nx), cy = cell_of(qy, g.oy, g.inv, ny), cz = cell_of(qz, g.oz, g.inv, nz);
+        int r = 0;
+        for (; r <= kFineShells; ++r) {
+            const float L = shell_bound(qx, qy, qz, cx, cy, cz, r, nx, ny, nz, g, g.cell, sl);
+            if (L * L >= kd) break;
+            for (int dz = -r; dz <= r; ++dz) {
+                const int iz = cz + dz;
+                if (iz < 0 || iz >= nz) continue;
+                const float gz = sq(fmaxf(gap(qz, g.oz, g.cell, iz) - sl, 0.f));
+                for (int dy = -r; dy <= r; ++dy) {
+                    const int iy = cy + dy;
+                    if (iy < 0 || iy >= ny) continue;
+                    const float gy = gz + sq(fmaxf(gap(qy, g.oy, g.cell, iy) - sl, 0.f));
+                    const int step = (dz == -r || dz == r || dy == -r || dy == r) ? 1 : max(2 * r, 1);
+                    for (int dx = -r; dx <= r; dx += step) {
+                        const int ix = cx + dx;
+                        if (ix < 0 || ix >= nx) continue;
+                        if (gy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= kd) continue;
+                        const int2 c = __ldg(cells + key_of(ix, iy, iz, g));
+                        knn_scan(pts, c.x, c.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
+                    }
+                }
+            }
+        }
+        if (r > kFineShells && sq(shell_bound(qx, qy, qz, cx, cy, cz, kFineShells + 1, nx, ny, nz, g, g.cell, sl)) < kd) {
+            const float bc = 8.f * g.cell;
+            const int bx = cx >> 3, by = cy >> 3, bz = cz >> 3;
+            for (int R = 0;; ++R) {
+                const float L = shell_bound(qx, qy, qz, bx, by, bz, R, g.nbx, g.nby, g.nbz, g, bc, sl);
+                if (L * L >= kd) break;
+                for (int dz = -R; dz <= R; ++dz) {
+                    const int jz = bz + dz;
+                    if (jz < 0 || jz >= g.nbz) continue;
+                    const float gz = sq(fmaxf(gap(qz, g.oz, bc, jz) - sl, 0.f));
+                    for (int dy = -R; dy <= R; ++dy) {
+                        const int jy = by + dy;
+                        if (jy < 0 || jy >= g.nby) continue;
+                        const float gy = gz + sq(fmaxf(gap(qy, g.oy, bc, jy) - sl, 0.f));
+                        const int step = (dz == -R || dz == R || dy == -R || dy == R) ? 1 : max(2 * R, 1);
+                        for (int dx = -R; dx <= R; dx += step) {
+                            const int jx = bx + dx;
+                            if (jx < 0 || jx >= g.nbx) continue;
+                            if (gy + sq(fmaxf(gap(qx, g.ox, bc, jx) - sl, 0.f)) >= kd) continue;
+                            const int blk = (jz * g.nby + jy) * g.nbx + jx;
+                            const int2 br = __ldg(blocks + blk);
+                            if (br.y <= br.x) continue;
+                            // a block within one of the query's may hold fine cells the shells visited: always by its cells, so
+                            // that no point is listed twice
+                            if (br.y - br.x <= kDirect && R > 1) {
+                                knn_scan(pts, br.x, br.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
+                                continue;
+                            }
+                            for (int lz = 0; lz < 8; ++lz) {
+                                const int iz = 8 * jz + lz;
+                                const float fz = sq(fmaxf(gap(qz, g.oz, g.cell, iz) - sl, 0.f));
+                                if (fz >= kd) continue;
+                                for (int ly = 0; ly < 8; ++ly) {
+                                    const int iy = 8 * jy + ly;
+                                    const float fy = fz + sq(fmaxf(gap(qy, g.oy, g.cell, iy) - sl, 0.f));
+                                    if (fy >= kd) continue;
+                                    const bool near_zy = abs(iz - cz) <= kFineShells && abs(iy - cy) <= kFineShells;
+                                    for (int lx = 0; lx < 8; ++lx) {
+                                        const int ix = 8 * jx + lx;
+                                        if (near_zy && abs(ix - cx) <= kFineShells) continue;
+                                        if (fy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= kd) continue;
+                                        const int2 c = __ldg(cells + (blk << 9) + (lz << 6) + (ly << 3) + lx);
+                                        knn_scan(pts, c.x, c.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
+                                    }
+                                }
+                            }
+                        }
+                    }
+                }
+            }
+        }
+    }
+    // the cap on the distance itself: the list is cut at the first entry whose root is not below max_dist
+    int c = 0;
+    for (; c < cnt; ++c)
+        if (!(root_below(sd[c * kThreads], lim) < max_dist)) break;
+    if constexpr (!NORMALS) {
+        for (int s = 0; s < k; ++s) {
+            dist[(size_t)i * k + s] = s < c ? root_below(sd[s * kThreads], lim) : kInf;
+            index[(size_t)i * k + s] = s < c ? si[s * kThreads] : -1;
+        }
+    } else {
+        double nrm[3] = {0.0, 0.0, 0.0};
+        if (c >= 3) {
+            double mx = 0.0, my = 0.0, mz = 0.0;
+            for (int s = 0; s < c; ++s) {
+                const size_t j = (size_t)si[s * kThreads];
+                mx += __ldg(query + 3 * j), my += __ldg(query + 3 * j + 1), mz += __ldg(query + 3 * j + 2);
+            }
+            mx /= c, my /= c, mz /= c;
+            double b[3][3] = {};                        // b[q][r] = C[r][q]: column q (C is symmetric)
+            for (int s = 0; s < c; ++s) {
+                const size_t j = (size_t)si[s * kThreads];
+                const double dx = __ldg(query + 3 * j) - mx, dy = __ldg(query + 3 * j + 1) - my, dz = __ldg(query + 3 * j + 2) - mz;
+                b[0][0] += dx * dx, b[0][1] += dx * dy, b[0][2] += dx * dz;
+                b[1][1] += dy * dy, b[1][2] += dy * dz, b[2][2] += dz * dz;
+            }
+            b[0][0] /= c, b[0][1] /= c, b[0][2] /= c, b[1][1] /= c, b[1][2] /= c, b[2][2] /= c;
+            b[1][0] = b[0][1], b[2][0] = b[0][2], b[2][1] = b[1][2];
+            if (b[0][0] + b[1][1] + b[2][2] > 0.0) {
+                // one-sided Jacobi on C's columns: B = C V with orthogonal columns b_q = lambda_q v_q, so for C positive semi-definite
+                // the column of V under the smallest |b_q| is the eigenvector of the smallest eigenvalue
+                double v[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+                for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+                    bool rotated = jacobi_pair<0, 1>(b, v);
+                    rotated |= jacobi_pair<0, 2>(b, v);
+                    rotated |= jacobi_pair<1, 2>(b, v);
+                    if (!rotated) break;
+                }
+                double s2[3];
+#pragma unroll
+                for (int q = 0; q < 3; ++q) s2[q] = b[q][0] * b[q][0] + b[q][1] * b[q][1] + b[q][2] * b[q][2];
+                const int q = s2[2] <= s2[0] && s2[2] <= s2[1] ? 2 : s2[1] <= s2[0] ? 1 : 0;
+                // selects, not v[q]: a run-time index would put v in a local-memory stack frame
+#pragma unroll
+                for (int r = 0; r < 3; ++r) nrm[r] = q == 0 ? v[0][r] : q == 1 ? v[1][r] : v[2][r];
+                const double ax = fabs(nrm[0]), ay = fabs(nrm[1]), az = fabs(nrm[2]);
+                const double big = ax >= ay && ax >= az ? nrm[0] : ay >= az ? nrm[1] : nrm[2];
+                double sgn = big < 0.0 ? -1.0 : 1.0;
+                if (view_mode) {
+                    const size_t o = view_mode == 2 ? 3 * (size_t)i : 0;
+                    const double dot = sgn * (nrm[0] * (__ldg(view + o) - qx) + nrm[1] * (__ldg(view + o + 1) - qy) +
+                                              nrm[2] * (__ldg(view + o + 2) - qz));
+                    if (dot < 0.0) sgn = -sgn;
+                }
+#pragma unroll
+                for (int r = 0; r < 3; ++r) nrm[r] *= sgn;
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 3; ++r) normals[3 * (size_t)i + r] = (float)nrm[r];
+    }
+}
+
 int blocks_for(int n) { return (n + kThreads - 1) / kThreads; }
 
 bool grid_ok(float cell, int nbx, int nby, int nbz) {
@@ -870,4 +1084,45 @@ extern "C" int mvsb200_pc_ransac_align(const double* src, const double* tgt, int
     pc_ransac_select_kernel<<<1, kSelectThreads, 0, (cudaStream_t)stream>>>(good, error2, trans, n_hyp, n, ransac_n, seed, record);
     MVS_CHECK_LAUNCH("pc_ransac_select");
     return MVSB200_OK;
+}
+
+namespace {
+
+template <bool NORMALS>
+int knn_launch(const char* what, const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
+               float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k, float* dist,
+               int32_t* index, const double* view, int view_mode, float* normals, void* stream) {
+    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "%s: misaligned buffer", what);
+    MVS_REQUIRE(n >= 0, "%s: 0 <= n < 2^31 queries", what);
+    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "%s: cell > 0 and at most %d cells", what, MVSB200_PC_MAX_CELLS);
+    MVS_REQUIRE(max_dist > 0.f && slack >= 0.f, "%s: max_dist > 0 (+inf allowed), slack >= 0", what);
+    MVS_REQUIRE(k >= 1 && k <= kKnnMax, "%s: 1 <= k <= %d, got %d", what, kKnnMax, k);
+    if (n == 0) return MVSB200_OK;
+    const int smem = k * kThreads * (int)(sizeof(float) + sizeof(int));
+    MVS_CUDA(cudaFuncSetAttribute(pc_knn_kernel<NORMALS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    pc_knn_kernel<NORMALS><<<blocks_for(n), kThreads, smem, (cudaStream_t)stream>>>(
+        query, n, (const float4*)pts, (const int2*)cells, (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
+        slack, max_dist, k, dist, index, view, view_mode, normals);
+    MVS_CHECK_LAUNCH(what);
+    return MVSB200_OK;
+}
+
+}  // namespace
+
+extern "C" int mvsb200_pc_knn(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox, float oy,
+                              float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k, float* dist,
+                              int32_t* index, void* stream) {
+    MVS_REQUIRE(query && pts && cells && blocks && dist && index, "pc_knn: null pointer");
+    return knn_launch<false>("pc_knn", query, n, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, slack, max_dist, k, dist, index,
+                             nullptr, 0, nullptr, stream);
+}
+
+extern "C" int mvsb200_pc_normals(const float* xyz, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
+                                  float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k,
+                                  const double* viewpoints, int view_mode, float* normals, void* stream) {
+    MVS_REQUIRE(xyz && pts && cells && blocks && normals, "pc_normals: null pointer");
+    MVS_REQUIRE(view_mode >= 0 && view_mode <= 2, "pc_normals: view_mode 0, 1 or 2, got %d", view_mode);
+    MVS_REQUIRE(view_mode == 0 || viewpoints, "pc_normals: view_mode %d needs viewpoints", view_mode);
+    return knn_launch<true>("pc_normals", xyz, n, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, slack, max_dist, k, nullptr,
+                            nullptr, viewpoints, view_mode, normals, stream);
 }

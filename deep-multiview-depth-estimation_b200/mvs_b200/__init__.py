@@ -15,10 +15,12 @@ from .refine import refine_depth  # noqa: F401
 from .nets2d import encode_features  # noqa: F401
 from .frozen import FrozenMVSNet  # noqa: F401
 from .ops import depth_confidence  # noqa: F401
-from .fusion import fuse_depth_maps, visibility_fusion, infer_scene, write_ply, read_ply  # noqa: F401
-from .evaluation import thin_points, nearest_distance, nearest_neighbour, evaluate_point_cloud, load_dtu_eval  # noqa: F401
+from .fusion import fuse_depth_maps, visibility_fusion, infer_scene, write_ply, read_ply, point_viewpoints  # noqa: F401
+from .evaluation import thin_points, nearest_distance, nearest_neighbour, k_nearest, evaluate_point_cloud, load_dtu_eval  # noqa: F401
+from .normals import estimate_normals  # noqa: F401
 from .tanks import (CropVolume, read_crop_volume, crop_points, voxel_down_sample, evaluate_tanks_and_temples,  # noqa: F401
-                    load_tnt_eval, Mapping, read_trajectory, write_trajectory, read_mapping, load_tnt_trajectory, camera_poses)
+                    load_tnt_eval, Mapping, read_trajectory, write_trajectory, read_mapping, load_tnt_trajectory, camera_poses,
+                    write_evaluation_files)
 from .registration import (uniform_down_sample, icp_point_to_point, register_tanks_and_temples,  # noqa: F401
                            trajectory_points, align_trajectory)
 
@@ -30,5 +32,5 @@ __all__ = ["homography_warping", "assemble_cost_volume", "extract_depth_map", "C
            "voxel_down_sample",
            "evaluate_tanks_and_temples", "load_tnt_eval", "uniform_down_sample", "icp_point_to_point", "register_tanks_and_temples",
            "Mapping", "read_trajectory", "write_trajectory", "read_mapping", "load_tnt_trajectory", "camera_poses",
-           "trajectory_points", "align_trajectory",
+           "trajectory_points", "align_trajectory", "k_nearest", "estimate_normals", "point_viewpoints", "write_evaluation_files",
            "MvsB200Error", "launch_count", "load_library"]

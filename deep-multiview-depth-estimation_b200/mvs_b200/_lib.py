@@ -16,6 +16,7 @@ FUSION_CAM_FLOATS, FUSION_BLOCK_PIXELS, FUSION_MAX_SOURCES = 32, 128, 16     # M
 PC_MAX_CELLS = 1 << 28                                                       # MVSB200_PC_MAX_CELLS
 PC_ICP_BLOCKS, PC_ICP_SUMS = 1024, 18                                        # MVSB200_PC_ICP_*
 PC_RANSAC_MAX_SAMPLE, PC_RANSAC_RECORD = 64, 80                             # MVSB200_PC_RANSAC_*
+PC_KNN_MAX = 32                                                              # MVSB200_PC_KNN_MAX
 
 _c = ctypes
 _P, _I = _c.c_void_p, _c.c_int
@@ -107,6 +108,8 @@ _SIGNATURES = {
     "mvsb200_pc_icp_sums": (_I, [_P, _P, _I, _P, _P, _P, _P, _P]),
     "mvsb200_pc_transform64": (_I, [_P, _I, _P, _P, _P]),
     "mvsb200_pc_ransac_align": (_I, [_P, _P, _I, _I, _I, _c.c_double, _I, _c.c_uint64, _P, _P, _P, _P, _P, _P]),
+    "mvsb200_pc_knn": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _I, _P, _P, _P]),
+    "mvsb200_pc_normals": (_I, [_P, _I, _P, _P, _P] + [_c.c_float] * 4 + [_I, _I, _I, _c.c_float, _c.c_float, _I, _P, _I, _P, _P]),
 }
 
 _lib = None

@@ -22,6 +22,7 @@ from .ops import _stream, _timed
 
 DST, MAX_DIST, BLOCK = 0.2, 20.0, 60.0          # DTU's values (BaseEvalMain_web.m)
 CELLS_PER_POINT = 0.25                           # search grid: one cell per 4 target points (measured, DESIGN §4 K8) ...
+KNN_CELLS_PER_POINT = 2.0                        # ... and for k-nearest searches: two cells per point (measured, DESIGN §4 K10)
 THIN_CELLS_PER_POINT = 16                        # thinning grid: finer, fewer candidates in the 27 cells around a point ...
 CELL_BUDGET = 1 << 26                            # ... and at most 2^26 cells (512 MB of {begin, end} pairs)
 _MAX_POINTS = (1 << 31) - 1
@@ -151,6 +152,44 @@ def nearest_neighbour(query, target, max_dist, *, grid=None):
     index = torch.full((n,), -1, dtype=torch.int32, device=q.device)
     if n and m:
         nearest_index_into(q, grid if grid is not None else build_grid(t), max_dist, dist, index)
+    return dist, index.long()
+
+
+def knn_k(k):
+    """k as an int in [1, PC_KNN_MAX], refused otherwise."""
+    if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= _lib.PC_KNN_MAX:
+        _fail(f"k must be an integer in [1, {_lib.PC_KNN_MAX}], got {k!r}")
+    return int(k)
+
+
+def knn_cap(max_dist):
+    """max_dist of a k-nearest search: > 0, +inf meaning no cap."""
+    v = float(max_dist)
+    if not v > 0:
+        _fail(f"max_dist must be > 0 (+inf: no cap), got {v}")
+    return v
+
+
+def k_nearest(query, target, k, max_dist=math.inf, *, grid=None):
+    """The k nearest target points [m, 3] of every query point [n, 3] (CUDA tensors) -> (dist fp32 [n, k], index int64 [n, k]).
+
+    Row i lists the target points that come first in the total order (d^2, row) among those with d < max_dist, ascending: d^2 is
+    the fp32 (dx^2 + dy^2) + dz^2 of nearest_distance and d its square root, so ties are exact and go to the smaller row, and
+    k = 1 is nearest_neighbour bit for bit.  A row holds fewer than k points only when the cap or the cloud leaves fewer; it is
+    padded with +inf / -1.  1 <= k <= 32; max_dist > 0 (+inf: no cap).  grid: a build_grid(target, cells_per_point=
+    KNN_CELLS_PER_POINT) to reuse.  Two calls return the same bits."""
+    q = _cloud(query, "query")
+    t = _cloud(target, "target")
+    k = knn_k(k)
+    max_dist = knn_cap(max_dist)
+    n, m = q.shape[0], t.shape[0]
+    dist = torch.full((n, k), float("inf"), dtype=torch.float32, device=q.device)
+    index = torch.full((n, k), -1, dtype=torch.int32, device=q.device)
+    if n and m:
+        g = grid if grid is not None else build_grid(t, cells_per_point=KNN_CELLS_PER_POINT)
+        with _timed("pc_knn"):
+            _lib.call("mvsb200_pc_knn", q.data_ptr(), n, g.pts.data_ptr(), g.cells.data_ptr(), g.blocks.data_ptr(), *g.args(),
+                      float(g.slack()), max_dist, k, dist.data_ptr(), index.data_ptr(), _stream())
     return dist, index.long()
 
 

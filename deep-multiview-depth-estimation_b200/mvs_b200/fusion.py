@@ -260,11 +260,29 @@ def infer_scene(frozen, images, K, R, T, d_min, d_int, pairs, n_views=3, batch_s
     return out_d, out_c, resize_colours(imgs, out_d.shape[2], out_d.shape[3])
 
 
-def write_ply(path, xyz, rgb=None):
-    """Binary little-endian PLY of the points xyz [M, 3] (float x, y, z) and, when given, their colours rgb [M, 3] in [0, 1]
-    (uchar red, green, blue: x 255, rounded, clamped)."""
+def point_viewpoints(masks, R, T):
+    """The centre C = -R^T T of the view that emitted each point of a fuse_depth_maps / visibility_fusion cloud -> fp64 [M, 3] on
+    the device of masks.  Both emit view-major in index order, so view i's centre repeats once per kept pixel of masks[i]; these
+    are the viewpoints estimate_normals takes to make each normal face the camera that saw its point.  masks [N, 1, h, w] (as returned), R [N, 3, 3], T [N, 3, 1]."""
+    if not isinstance(masks, torch.Tensor) or masks.dim() != 4 or masks.shape[1] != 1:
+        _fail(f"point_viewpoints: masks [N, 1, h, w] expected, got {tuple(getattr(masks, 'shape', ()))}")
+    N = masks.shape[0]
+    R, T = _f64(R, (N, 3, 3), "R"), _f64(T, (N, 3, 1), "T")
+    C = torch.from_numpy((-np.transpose(R, (0, 2, 1)) @ T).reshape(N, 3)).to(masks.device)
+    counts = masks.reshape(N, -1).bool().sum(1)
+    return torch.repeat_interleave(C, counts, dim=0)
+
+
+def write_ply(path, xyz, rgb=None, normals=None):
+    """Binary little-endian PLY of the points xyz [M, 3] (float x, y, z), when given their normals [M, 3] (float nx, ny, nz, after z
+    as Open3D writes them) and their colours rgb [M, 3] in [0, 1] (uchar red, green, blue: x 255, rounded, clamped)."""
     pts = (xyz.detach().cpu().numpy() if isinstance(xyz, torch.Tensor) else np.asarray(xyz)).astype("<f4").reshape(-1, 3)
     fields = [("x", "<f4"), ("y", "<f4"), ("z", "<f4")]
+    if normals is not None:
+        nrm = (normals.detach().cpu().numpy() if isinstance(normals, torch.Tensor) else np.asarray(normals)).astype("<f4").reshape(-1, 3)
+        if nrm.shape[0] != pts.shape[0]:
+            _fail(f"write_ply: {pts.shape[0]} points but {nrm.shape[0]} normals")
+        fields += [("nx", "<f4"), ("ny", "<f4"), ("nz", "<f4")]
     if rgb is not None:
         col = (rgb.detach().cpu().numpy() if isinstance(rgb, torch.Tensor) else np.asarray(rgb)).astype(np.float64).reshape(-1, 3)
         if col.shape[0] != pts.shape[0]:
@@ -272,10 +290,14 @@ def write_ply(path, xyz, rgb=None):
         fields += [("red", "u1"), ("green", "u1"), ("blue", "u1")]
     rec = np.empty(pts.shape[0], dtype=fields)
     rec["x"], rec["y"], rec["z"] = pts[:, 0], pts[:, 1], pts[:, 2]
+    if normals is not None:
+        rec["nx"], rec["ny"], rec["nz"] = nrm[:, 0], nrm[:, 1], nrm[:, 2]
     if rgb is not None:
         c8 = np.clip(np.rint(col * 255.0), 0, 255).astype(np.uint8)
         rec["red"], rec["green"], rec["blue"] = c8[:, 0], c8[:, 1], c8[:, 2]
     props = "".join(f"property float {n}\n" for n in "xyz")
+    if normals is not None:
+        props += "".join(f"property float {n}\n" for n in ("nx", "ny", "nz"))
     if rgb is not None:
         props += "".join(f"property uchar {n}\n" for n in ("red", "green", "blue"))
     header = f"ply\nformat binary_little_endian 1.0\nelement vertex {pts.shape[0]}\n{props}end_header\n"

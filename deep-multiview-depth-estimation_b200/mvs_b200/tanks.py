@@ -273,6 +273,73 @@ def evaluate_tanks_and_temples(xyz, gt, crop, transform, tau, *, stretch=STRETCH
     return out
 
 
+# matplotlib's "hot" segment data (x, value) per channel, as read from matplotlib's _cm.py, not diffed (matplotlib is not a
+# dependency); LinearSegmentedColormap interpolates them at N = 256 evenly spaced points, and "hot_r" is that table reversed
+_HOT = {"red": ((0.0, 0.0416), (0.365079, 1.0), (1.0, 1.0)),
+        "green": ((0.0, 0.0), (0.365079, 0.0), (0.746032, 1.0), (1.0, 1.0)),
+        "blue": ((0.0, 0.0), (0.746032, 0.0), (1.0, 1.0))}
+COLOUR_CLIP = 3                                  # the toolbox colours distances up to 3 tau (as read here, not diffed)
+NORMALS_KNN = 20                                 # the toolbox's KDTreeSearchParamKNN(knn=20) (as read here, not diffed)
+
+
+def hot_r_table(N=256):
+    """matplotlib's hot_r lookup table -> fp64 [N, 3] (RGB): row 0 is (1, 1, 1), row N - 1 is (0.0416, 0, 0)."""
+    idx = np.arange(N, dtype=np.float64)
+    lut = np.stack([np.interp(idx, [x * (N - 1) for x, _ in _HOT[c]], [v for _, v in _HOT[c]]) for c in ("red", "green", "blue")], 1)
+    return np.clip(lut, 0.0, 1.0)[::-1].copy()
+
+
+def hot_r(x, N=256):
+    """A matplotlib colormap call on values x in [0, 1]: row int(x N) of hot_r_table, with x = 1 mapped to the last row -> fp64 [.., 3]."""
+    i = np.floor(np.asarray(x, dtype=np.float64) * N)
+    i = np.clip(np.where(i == N, N - 1, i), 0, N - 1).astype(np.int64)
+    return hot_r_table(N)[i]
+
+
+def distance_colours(d, tau, clip=COLOUR_CLIP):
+    """The toolbox's colours of distances d (any shape, +inf allowed): hot_r(min(d, clip tau) / (clip tau)), fp64 [.., 3]."""
+    top = clip * tau
+    return hot_r(np.minimum(np.asarray(d, dtype=np.float64), top) / top)
+
+
+def write_evaluation_files(directory, scene, result, *, knn=NORMALS_KNN, stretch=STRETCH):
+    """The per-scene files of the toolbox's EvaluateHisto from evaluate_tanks_and_temples(..., return_details=True) -> their paths:
+        {scene}.precision.ply        xyz_down (rounded to fp32), estimate_normals(k=knn) with the canonical sign, distance_colours(d_s)
+        {scene}.recall.ply           the same for gt_down and d_t
+        {scene}.precision.txt        np.savetxt of cum_precision
+        {scene}.recall.txt           np.savetxt of cum_recall
+        {scene}.prf_tau_plotstr.txt  np.savetxt of [precision, recall, fscore, tau, stretch]
+    The names, contents and PLY property order are the toolbox's and Open3D's as read here, not diffed.  Refused with MvsB200Error:
+    a result without the details."""
+    from .fusion import write_ply
+    from .normals import estimate_normals
+    missing = [k for k in ("xyz_down", "gt_down", "d_s", "d_t") if k not in result]
+    if missing:
+        _fail(f"write_evaluation_files: the result has no {', '.join(missing)}: evaluate with return_details=True")
+    os.makedirs(directory, exist_ok=True)
+    base = os.path.join(directory, scene)
+    tau = float(result["tau"])
+    paths = []
+    for name, pts, d in (("precision", result["xyz_down"], result["d_s"]), ("recall", result["gt_down"], result["d_t"])):
+        p32 = pts.float().contiguous()
+        path = f"{base}.{name}.ply"
+        write_ply(path, p32, distance_colours(d.double().cpu().numpy(), tau), normals=estimate_normals(p32, knn))
+        paths.append(path)
+    return paths + write_curves(directory, scene, result, stretch=stretch)
+
+
+def write_curves(directory, scene, result, *, stretch=STRETCH):
+    """The three text files of write_evaluation_files ({scene}.precision.txt, .recall.txt, .prf_tau_plotstr.txt) -> their paths."""
+    base = os.path.join(directory, scene)
+    paths = []
+    for name, key in (("precision", "cum_precision"), ("recall", "cum_recall")):
+        paths.append(f"{base}.{name}.txt")
+        np.savetxt(paths[-1], np.asarray(result[key], dtype=np.float64))
+    paths.append(f"{base}.prf_tau_plotstr.txt")
+    np.savetxt(paths[-1], np.array([result["precision"], result["recall"], result["fscore"], float(result["tau"]), float(stretch)]))
+    return paths
+
+
 def load_tnt_eval(root, scene):
     """Tanks and Temples' evaluation files of one scene -> (gt fp32 [m, 3] CPU tensor, CropVolume, transform fp64 [4, 4]), read from
         {root}/{scene}/{scene}.ply          the ground-truth points

@@ -562,6 +562,24 @@ int mvsb200_pc_ransac_align(const double* src, const double* tgt, int n, int n_h
                             int with_scaling, uint64_t seed, int32_t* good, double* error2, double* trans, int32_t* samples,
                             double* record, void* stream);
 
+/* ---- K10 normals: exact k-nearest neighbours and oriented normals on K8's grid ---------------------------------------------------
+ * knn: for n queries [n, 3] against a grid built as above, the k points that come first in the total order (d^2, original index)
+ * among those with d < max_dist, where d^2 = (dx^2 + dy^2) + dz^2 in fp32 and d its square root (K8's; k = 1 is pc_nearest_index bit
+ * for bit).  dist [n, k] fp32 ascending (+inf padded) and index [n, k] int32 (-1 padded).  max_dist > 0, +inf allowed.
+ * normals: the same search with the cloud xyz [n, 3] as the queries AND the grid's cloud (the query point is its own neighbour at
+ * distance 0), then per point the fp64 covariance of its c neighbours centred in two passes (sums in list order), the unit
+ * eigenvector of its smallest eigenvalue (one-sided Jacobi), the largest-magnitude component made positive (the first such axis on
+ * a tie) and, with viewpoints, flipped iff n . (v - p) < 0 in fp64 -> normals [n, 3] fp32, zero where c < 3 or the trace is 0.
+ * view_mode 0: no viewpoints (viewpoints may be NULL); 1: one viewpoint [3] fp64; 2: one per point [n, 3] fp64 (device).
+ * 1 <= k <= MVSB200_PC_KNN_MAX.  One launch each; deterministic. */
+#define MVSB200_PC_KNN_MAX 32
+int mvsb200_pc_knn(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox, float oy,
+                   float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k, float* dist, int32_t* index,
+                   void* stream);
+int mvsb200_pc_normals(const float* xyz, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox, float oy,
+                       float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k, const double* viewpoints,
+                       int view_mode, float* normals, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

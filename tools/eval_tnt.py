@@ -4,6 +4,8 @@
 
     python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 --traj Barn.log [--seed 0]
 
+    python tools/eval_tnt.py --ply Barn.ply --tnt /data/tnt --scene Barn --tau 0.01 [--register | --traj Barn.log] --write out/
+
 --tnt is the directory of T&T's evaluation data, one sub-directory per scene with {scene}.ply, {scene}.json and {scene}_trans.txt,
 and for --traj also {scene}_COLMAP_SfM.log and, for a trajectory of every video frame, {scene}_mapping_reference.txt
 (INTEGRATION.md §2).  --traj runs the toolbox's whole chain: the RANSAC alignment of the reconstruction's camera trajectory (a .log
@@ -15,7 +17,9 @@ transform, as the toolbox does; without it {scene}_trans.txt (or --init) is used
 toolbox's table of per-scene values is not shipped).  Prints one JSON line: precision, recall, fscore, the counts, and the
 histogram edges and cumulative curves; with --register also a `registration` record (the refined transform and, per stage, its
 sizes, iterations, fitness, rmse and transform); with --traj also an `alignment` record (the RANSAC transform, fitness, rmse,
-inliers, the winning hypothesis and its sample, the correspondence count and the seed)."""
+inliers, the winning hypothesis and its sample, the correspondence count and the seed).  --write DIR also writes the toolbox's
+per-scene files into DIR (mvs_b200.write_evaluation_files): {scene}.precision.ply and {scene}.recall.ply, the down-sampled clouds
+with normals and coloured by distance, and {scene}.precision.txt, {scene}.recall.txt and {scene}.prf_tau_plotstr.txt."""
 import argparse
 import json
 import os
@@ -44,11 +48,14 @@ def main(argv=None):
     ap.add_argument("--init", help="a 4 x 4 text file to start from instead of {scene}_trans.txt")
     ap.add_argument("--traj", help="the reconstruction's camera trajectory (.log): align it to T&T's first (implies --register)")
     ap.add_argument("--seed", type=int, help="the seed of the alignment's RANSAC draws (with --traj; default 0)")
+    ap.add_argument("--write", metavar="DIR", help="also write the toolbox's coloured precision / recall clouds and curves to DIR")
     a = ap.parse_args(argv)
     if a.traj and a.init:
         ap.error("--traj and --init exclude each other: --traj computes the initial alignment")
     if a.seed is not None and not a.traj:
         ap.error("--seed applies to --traj only")
+    if a.write is not None and (not a.write or (os.path.exists(a.write) and not os.path.isdir(a.write))):
+        ap.error(f"--write needs a directory, got {a.write!r}")
     xyz, _ = mvs_b200.read_ply(a.ply)
     gt, crop, trans = mvs_b200.load_tnt_eval(a.tnt, a.scene)
     if a.init:
@@ -65,7 +72,12 @@ def main(argv=None):
     if a.register or a.traj:
         reg = mvs_b200.register_tanks_and_temples(xyz, gt, crop, trans, a.tau)
         trans = reg["transformation"]
-    r = mvs_b200.evaluate_tanks_and_temples(xyz, gt, crop, trans, a.tau, stretch=a.stretch)
+    r = mvs_b200.evaluate_tanks_and_temples(xyz, gt, crop, trans, a.tau, stretch=a.stretch, return_details=a.write is not None)
+    if a.write is not None:
+        with torch.cuda.device(dev):
+            mvs_b200.write_evaluation_files(a.write, a.scene, r, stretch=a.stretch)
+        for k in ("xyz_down", "gt_down", "d_s", "d_t"):
+            del r[k]
     r = {"scene": a.scene, "ply": a.ply, **{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in r.items()}}
     if align is not None:
         r["alignment"] = {**{k: v.tolist() if isinstance(v, np.ndarray) else v for k, v in align.items()}, "seed": a.seed or 0}
