@@ -21,11 +21,15 @@
 //   pc_knn_kernel            K10: one thread per query, the exact k nearest points in the order (d^2, index), capped at max_dist;
 //                            <true>: on the cloud itself, the normal of each point's neighbourhood (fp64 covariance, Jacobi)
 //
-// Nearest search.  Shells r = 0, 1, ... of fine cells around the query's (clamped) cell, up to kFineShells; then shells of coarse
-// blocks, skipping empty blocks, visiting an occupied block by its points (few) or by its fine cells (many).  A shell is entered
-// only while a lower bound on the distance to every cell of it and beyond is below min(best, max_dist), so the result is exact:
-// a minimum does not depend on the visiting order.  Lower bounds subtract `slack` (set by the host above the fp32 rounding of
-// the box coordinates), so a point whose cell was decided in fp64 is never pruned by a rounding of its cell's faces.
+// Grid search (grid_search, the one traversal of pc_nearest_kernel and pc_knn_kernel).  Shells r = 0, 1, ... of fine cells around
+// the query's (clamped) cell, up to kFineShells; then shells of coarse blocks, skipping empty blocks, visiting an occupied block by
+// its points (few) or by its fine cells (many).  A shell is entered, and a cell or block visited, only while a lower bound on its
+// distance is below the caller's squared bound: min(best, max_dist^2) for the nearest point, the k-th entry of the list for the k
+// nearest.  So every point below the bound is visited and the result is exact: neither a minimum nor a list in a total order
+// depends on the visiting order.  Lower bounds subtract `slack` (set by the host above the fp32 rounding of the box coordinates),
+// so a point whose cell was decided in fp64 is never pruned by a rounding of its cell's faces, and a point that ties the bound is
+// never pruned.  The one variation: the k-nearest list must not hold a point twice, so there a sparse block within one block of
+// the query's (it may hold fine cells the shells visited) is visited by its fine cells rather than point by point.
 #include "common.cuh"
 
 using namespace mvsb200;
@@ -115,38 +119,42 @@ __global__ void __launch_bounds__(kThreads) pc_grid_cells_kernel(const float* __
     if (kn < 0 || (k >> 9) != (kn >> 9)) blocks[k >> 9].y = s + 1;
 }
 
-// IDX: also index[i] = the original index of the nearest point (ties: the smaller index), -1 where dist[i] is +inf.  Pruning is the
-// same in both forms: a tied point is never pruned, because every lower bound is below the true gap by `slack`.
-template <bool IDX>
-__global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __restrict__ query, int n, const float4* __restrict__ pts,
-                                                             const int2* __restrict__ cells, const int2* __restrict__ blocks, Grid g,
-                                                             float slack, float max_dist, float* __restrict__ dist,
-                                                             int32_t* __restrict__ index) {
-    const int i = blockIdx.x * kThreads + threadIdx.x;
-    if (i >= n) return;
-    const float qx = query[3 * (size_t)i], qy = query[3 * (size_t)i + 1], qz = query[3 * (size_t)i + 2];
-    const int nx = 8 * g.nbx, ny = 8 * g.nby, nz = 8 * g.nbz;
-    // the grid's box is farther than max_dist: nothing to find (fp64, once per query)
-    {
-        const double c = g.cell;
-        const double ex = fmax(fmax((double)g.ox - qx, (double)qx - (g.ox + nx * c)), 0.0);
-        const double ey = fmax(fmax((double)g.oy - qy, (double)qy - (g.oy + ny * c)), 0.0);
-        const double ez = fmax(fmax((double)g.oz - qz, (double)qz - (g.oz + nz * c)), 0.0);
-        if (ex * ex + ey * ey + ez * ez >= (double)max_dist * max_dist) {
-            dist[i] = kInf;
-            if constexpr (IDX) index[i] = -1;
-            return;
-        }
+// the squared distance from q to the grid's box of nx x ny x nz fine cells (fp64, once per query)
+__device__ __forceinline__ double box_gap2(float qx, float qy, float qz, const Grid& g, int nx, int ny, int nz) {
+    const double c = g.cell;
+    const double ex = fmax(fmax((double)g.ox - qx, (double)qx - (g.ox + nx * c)), 0.0);
+    const double ey = fmax(fmax((double)g.oy - qy, (double)qy - (g.oy + ny * c)), 0.0);
+    const double ez = fmax(fmax((double)g.oz - qz, (double)qz - (g.oz + nz * c)), 0.0);
+    return ex * ex + ey * ey + ez * ez;
+}
+
+// the square root of s by one Newton step on the approximate reciprocal root (within an ulp; no IEEE slow-path call frame),
+// +inf for s >= lim
+__device__ __forceinline__ float root_below(float s, float lim) {
+    float d = kInf;
+    if (s == 0.f) {
+        d = 0.f;
+    } else if (s < lim) {
+        const float y = rsqrtf(s);
+        d = s * y;
+        d = fmaf(0.5f * y, fmaf(-d, d, s), d);
     }
-    const float sl = slack + 2.4e-7f * (fabsf(qx) + fabsf(qy) + fabsf(qz));
-    const float lim = max_dist * max_dist;
-    const int cx = cell_of(qx, g.ox, g.inv, nx), cy = cell_of(qy, g.oy, g.inv, ny), cz = cell_of(qz, g.oz, g.inv, nz);
-    float best = kInf;                                                  // squared
-    int bi = -1;
+    return d;
+}
+
+// The search of the header comment around query q in its cell (cx, cy, cz), with `sl` the query's slack.  bound(): the current
+// squared pruning bound, compared with every lower bound (a point at the bound is not pruned: the bounds lie sl below the true
+// gaps); scan(b, e): visit the sorted points [b, e).  ONCE: every point is visited at most once, so a sparse block within one block
+// of the query's is visited by its fine cells; without it such a block is scanned point by point, and a point of the fine shells
+// may be visited again, which a minimum does not notice.
+template <bool ONCE, class Bound, class Scan>
+__device__ __forceinline__ void grid_search(float qx, float qy, float qz, int cx, int cy, int cz, const Grid& g, float sl,
+                                            const int2* __restrict__ cells, const int2* __restrict__ blocks, Bound bound, Scan scan) {
+    const int nx = 8 * g.nbx, ny = 8 * g.nby, nz = 8 * g.nbz;
     int r = 0;
     for (; r <= kFineShells; ++r) {
         const float L = shell_bound(qx, qy, qz, cx, cy, cz, r, nx, ny, nz, g, g.cell, sl);
-        if (L * L >= fminf(best, lim)) break;
+        if (L * L >= bound()) break;
         for (int dz = -r; dz <= r; ++dz) {
             const int iz = cz + dz;
             if (iz < 0 || iz >= nz) continue;
@@ -159,21 +167,20 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
                 for (int dx = -r; dx <= r; dx += step) {
                     const int ix = cx + dx;
                     if (ix < 0 || ix >= nx) continue;
-                    if (gy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= fminf(best, lim)) continue;
+                    if (gy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= bound()) continue;
                     const int2 c = __ldg(cells + key_of(ix, iy, iz, g));
-                    scan_points<IDX>(pts, c.x, c.y, qx, qy, qz, best, bi);
+                    scan(c.x, c.y);
                 }
             }
         }
     }
-    if (r > kFineShells &&
-        sq(shell_bound(qx, qy, qz, cx, cy, cz, kFineShells + 1, nx, ny, nz, g, g.cell, sl)) < fminf(best, lim)) {
+    if (r > kFineShells && sq(shell_bound(qx, qy, qz, cx, cy, cz, kFineShells + 1, nx, ny, nz, g, g.cell, sl)) < bound()) {
         // coarse level: blocks of 8 fine cells per axis; the fine cells within kFineShells of (cx, cy, cz) are done
         const float bc = 8.f * g.cell;
         const int bx = cx >> 3, by = cy >> 3, bz = cz >> 3;
         for (int R = 0;; ++R) {
             const float L = shell_bound(qx, qy, qz, bx, by, bz, R, g.nbx, g.nby, g.nbz, g, bc, sl);
-            if (L * L >= fminf(best, lim)) break;
+            if (L * L >= bound()) break;
             for (int dz = -R; dz <= R; ++dz) {
                 const int jz = bz + dz;
                 if (jz < 0 || jz >= g.nbz) continue;
@@ -186,29 +193,29 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
                     for (int dx = -R; dx <= R; dx += step) {
                         const int jx = bx + dx;
                         if (jx < 0 || jx >= g.nbx) continue;
-                        if (gy + sq(fmaxf(gap(qx, g.ox, bc, jx) - sl, 0.f)) >= fminf(best, lim)) continue;
+                        if (gy + sq(fmaxf(gap(qx, g.ox, bc, jx) - sl, 0.f)) >= bound()) continue;
                         const int blk = (jz * g.nby + jy) * g.nbx + jx;
                         const int2 br = __ldg(blocks + blk);
                         if (br.y <= br.x) continue;                     // empty block
-                        if (br.y - br.x <= kDirect) {
-                            scan_points<IDX>(pts, br.x, br.y, qx, qy, qz, best, bi);
+                        if (br.y - br.x <= kDirect && (!ONCE || R > 1)) {
+                            scan(br.x, br.y);
                             continue;
                         }
                         for (int lz = 0; lz < 8; ++lz) {
                             const int iz = 8 * jz + lz;
                             const float fz = sq(fmaxf(gap(qz, g.oz, g.cell, iz) - sl, 0.f));
-                            if (fz >= fminf(best, lim)) continue;
+                            if (fz >= bound()) continue;
                             for (int ly = 0; ly < 8; ++ly) {
                                 const int iy = 8 * jy + ly;
                                 const float fy = fz + sq(fmaxf(gap(qy, g.oy, g.cell, iy) - sl, 0.f));
-                                if (fy >= fminf(best, lim)) continue;
+                                if (fy >= bound()) continue;
                                 const bool near_zy = abs(iz - cz) <= kFineShells && abs(iy - cy) <= kFineShells;
                                 for (int lx = 0; lx < 8; ++lx) {
                                     const int ix = 8 * jx + lx;
                                     if (near_zy && abs(ix - cx) <= kFineShells) continue;      // visited in the fine shells
-                                    if (fy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= fminf(best, lim)) continue;
+                                    if (fy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= bound()) continue;
                                     const int2 c = __ldg(cells + (blk << 9) + (lz << 6) + (ly << 3) + lx);
-                                    scan_points<IDX>(pts, c.x, c.y, qx, qy, qz, best, bi);
+                                    scan(c.x, c.y);
                                 }
                             }
                         }
@@ -217,15 +224,31 @@ __global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __
             }
         }
     }
-    // sqrt by one Newton step on the approximate reciprocal root (within an ulp; no IEEE slow-path call frame)
-    float d = kInf;
-    if (best == 0.f) {
-        d = 0.f;
-    } else if (best < lim) {
-        const float y = rsqrtf(best);
-        d = best * y;
-        d = fmaf(0.5f * y, fmaf(-d, d, best), d);
+}
+
+// IDX: also index[i] = the original index of the nearest point (ties: the smaller index), -1 where dist[i] is +inf
+template <bool IDX>
+__global__ void __launch_bounds__(kThreads, 2) pc_nearest_kernel(const float* __restrict__ query, int n, const float4* __restrict__ pts,
+                                                             const int2* __restrict__ cells, const int2* __restrict__ blocks, Grid g,
+                                                             float slack, float max_dist, float* __restrict__ dist,
+                                                             int32_t* __restrict__ index) {
+    const int i = blockIdx.x * kThreads + threadIdx.x;
+    if (i >= n) return;
+    const float qx = query[3 * (size_t)i], qy = query[3 * (size_t)i + 1], qz = query[3 * (size_t)i + 2];
+    const int nx = 8 * g.nbx, ny = 8 * g.nby, nz = 8 * g.nbz;
+    if (box_gap2(qx, qy, qz, g, nx, ny, nz) >= (double)max_dist * max_dist) {          // nothing within max_dist
+        dist[i] = kInf;
+        if constexpr (IDX) index[i] = -1;
+        return;
     }
+    const float sl = slack + 2.4e-7f * (fabsf(qx) + fabsf(qy) + fabsf(qz));
+    const float lim = max_dist * max_dist;
+    const int cx = cell_of(qx, g.ox, g.inv, nx), cy = cell_of(qy, g.oy, g.inv, ny), cz = cell_of(qz, g.oz, g.inv, nz);
+    float best = kInf;                                                  // squared
+    int bi = -1;
+    grid_search<false>(qx, qy, qz, cx, cy, cz, g, sl, cells, blocks, [&] { return fminf(best, lim); },
+                       [&](int b, int e) { scan_points<IDX>(pts, b, e, qx, qy, qz, best, bi); });
+    const float d = root_below(best, lim);
     dist[i] = d < max_dist ? d : kInf;
     if constexpr (IDX) index[i] = d < max_dist ? bi : -1;
 }
@@ -703,19 +726,6 @@ __global__ void __launch_bounds__(kSelectThreads) pc_ransac_select_kernel(const 
 
 constexpr int kKnnMax = MVSB200_PC_KNN_MAX;
 
-// pc_nearest_kernel's square root of s, +inf for s >= lim
-__device__ __forceinline__ float root_below(float s, float lim) {
-    float d = kInf;
-    if (s == 0.f) {
-        d = 0.f;
-    } else if (s < lim) {
-        const float y = rsqrtf(s);
-        d = s * y;
-        d = fmaf(0.5f * y, fmaf(-d, d, s), d);
-    }
-    return d;
-}
-
 // a candidate the order test admitted: insertion into the sorted list sd / si (this thread's slot 0) of cnt <= k entries
 __device__ __forceinline__ void knn_insert(float d, int j, float* sd, int* si, int k, int& cnt, float& kd, int& kj) {
     int p = cnt < k ? cnt : k - 1;
@@ -757,98 +767,17 @@ __global__ void __launch_bounds__(kThreads, 2) pc_knn_kernel(const float* __rest
     const float qx = query[3 * (size_t)i], qy = query[3 * (size_t)i + 1], qz = query[3 * (size_t)i + 2];
     const int nx = 8 * g.nbx, ny = 8 * g.nby, nz = 8 * g.nbz;
     const float lim = max_dist * max_dist;
-    int cnt = 0;
-    float kd = lim;
-    int kj = -1;
-    bool reach = true;
-    {
-        const double c = g.cell;
-        const double ex = fmax(fmax((double)g.ox - qx, (double)qx - (g.ox + nx * c)), 0.0);
-        const double ey = fmax(fmax((double)g.oy - qy, (double)qy - (g.oy + ny * c)), 0.0);
-        const double ez = fmax(fmax((double)g.oz - qz, (double)qz - (g.oz + nz * c)), 0.0);
-        reach = ex * ex + ey * ey + ez * ez < (double)max_dist * max_dist;
-    }
-    if (reach) {
+    // the list's count and k-th entry: as one object the kernel takes 61 registers, as three locals 62
+    struct { int cnt; float kd; int kj; } top{0, lim, -1};
+    if (box_gap2(qx, qy, qz, g, nx, ny, nz) < (double)max_dist * max_dist) {
         const float sl = slack + 2.4e-7f * (fabsf(qx) + fabsf(qy) + fabsf(qz));
         const int cx = cell_of(qx, g.ox, g.inv, nx), cy = cell_of(qy, g.oy, g.inv, ny), cz = cell_of(qz, g.oz, g.inv, nz);
-        int r = 0;
-        for (; r <= kFineShells; ++r) {
-            const float L = shell_bound(qx, qy, qz, cx, cy, cz, r, nx, ny, nz, g, g.cell, sl);
-            if (L * L >= kd) break;
-            for (int dz = -r; dz <= r; ++dz) {
-                const int iz = cz + dz;
-                if (iz < 0 || iz >= nz) continue;
-                const float gz = sq(fmaxf(gap(qz, g.oz, g.cell, iz) - sl, 0.f));
-                for (int dy = -r; dy <= r; ++dy) {
-                    const int iy = cy + dy;
-                    if (iy < 0 || iy >= ny) continue;
-                    const float gy = gz + sq(fmaxf(gap(qy, g.oy, g.cell, iy) - sl, 0.f));
-                    const int step = (dz == -r || dz == r || dy == -r || dy == r) ? 1 : max(2 * r, 1);
-                    for (int dx = -r; dx <= r; dx += step) {
-                        const int ix = cx + dx;
-                        if (ix < 0 || ix >= nx) continue;
-                        if (gy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= kd) continue;
-                        const int2 c = __ldg(cells + key_of(ix, iy, iz, g));
-                        knn_scan(pts, c.x, c.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
-                    }
-                }
-            }
-        }
-        if (r > kFineShells && sq(shell_bound(qx, qy, qz, cx, cy, cz, kFineShells + 1, nx, ny, nz, g, g.cell, sl)) < kd) {
-            const float bc = 8.f * g.cell;
-            const int bx = cx >> 3, by = cy >> 3, bz = cz >> 3;
-            for (int R = 0;; ++R) {
-                const float L = shell_bound(qx, qy, qz, bx, by, bz, R, g.nbx, g.nby, g.nbz, g, bc, sl);
-                if (L * L >= kd) break;
-                for (int dz = -R; dz <= R; ++dz) {
-                    const int jz = bz + dz;
-                    if (jz < 0 || jz >= g.nbz) continue;
-                    const float gz = sq(fmaxf(gap(qz, g.oz, bc, jz) - sl, 0.f));
-                    for (int dy = -R; dy <= R; ++dy) {
-                        const int jy = by + dy;
-                        if (jy < 0 || jy >= g.nby) continue;
-                        const float gy = gz + sq(fmaxf(gap(qy, g.oy, bc, jy) - sl, 0.f));
-                        const int step = (dz == -R || dz == R || dy == -R || dy == R) ? 1 : max(2 * R, 1);
-                        for (int dx = -R; dx <= R; dx += step) {
-                            const int jx = bx + dx;
-                            if (jx < 0 || jx >= g.nbx) continue;
-                            if (gy + sq(fmaxf(gap(qx, g.ox, bc, jx) - sl, 0.f)) >= kd) continue;
-                            const int blk = (jz * g.nby + jy) * g.nbx + jx;
-                            const int2 br = __ldg(blocks + blk);
-                            if (br.y <= br.x) continue;
-                            // a block within one of the query's may hold fine cells the shells visited: always by its cells, so
-                            // that no point is listed twice
-                            if (br.y - br.x <= kDirect && R > 1) {
-                                knn_scan(pts, br.x, br.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
-                                continue;
-                            }
-                            for (int lz = 0; lz < 8; ++lz) {
-                                const int iz = 8 * jz + lz;
-                                const float fz = sq(fmaxf(gap(qz, g.oz, g.cell, iz) - sl, 0.f));
-                                if (fz >= kd) continue;
-                                for (int ly = 0; ly < 8; ++ly) {
-                                    const int iy = 8 * jy + ly;
-                                    const float fy = fz + sq(fmaxf(gap(qy, g.oy, g.cell, iy) - sl, 0.f));
-                                    if (fy >= kd) continue;
-                                    const bool near_zy = abs(iz - cz) <= kFineShells && abs(iy - cy) <= kFineShells;
-                                    for (int lx = 0; lx < 8; ++lx) {
-                                        const int ix = 8 * jx + lx;
-                                        if (near_zy && abs(ix - cx) <= kFineShells) continue;
-                                        if (fy + sq(fmaxf(gap(qx, g.ox, g.cell, ix) - sl, 0.f)) >= kd) continue;
-                                        const int2 c = __ldg(cells + (blk << 9) + (lz << 6) + (ly << 3) + lx);
-                                        knn_scan(pts, c.x, c.y, qx, qy, qz, sd, si, k, cnt, kd, kj);
-                                    }
-                                }
-                            }
-                        }
-                    }
-                }
-            }
-        }
+        grid_search<true>(qx, qy, qz, cx, cy, cz, g, sl, cells, blocks, [&] { return top.kd; },
+                          [&](int b, int e) { knn_scan(pts, b, e, qx, qy, qz, sd, si, k, top.cnt, top.kd, top.kj); });
     }
     // the cap on the distance itself: the list is cut at the first entry whose root is not below max_dist
     int c = 0;
-    for (; c < cnt; ++c)
+    for (; c < top.cnt; ++c)
         if (!(root_below(sd[c * kThreads], lim) < max_dist)) break;
     if constexpr (!NORMALS) {
         for (int s = 0; s < k; ++s) {
@@ -915,6 +844,31 @@ bool grid_ok(float cell, int nbx, int nby, int nbz) {
            (long long)nbx * nby * nbz * 512 <= (long long)MVSB200_PC_MAX_CELLS;
 }
 
+// the checks of a search on a built grid (float4 points, int2 cells and blocks; blocks may be null) -> g
+int search_grid(const char* what, const float* pts, const int32_t* cells, const int32_t* blocks, float ox, float oy, float oz,
+                float cell, int nbx, int nby, int nbz, Grid& g) {
+    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "%s: misaligned buffer", what);
+    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "%s: cell > 0 and at most %d cells", what, MVSB200_PC_MAX_CELLS);
+    g = Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell};
+    return MVSB200_OK;
+}
+
+template <bool IDX>
+int nearest_launch(const char* what, const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
+                   float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, float* dist, int32_t* index,
+                   void* stream) {
+    MVS_REQUIRE(n >= 0, "%s: 0 <= n < 2^31 queries", what);
+    Grid g;
+    const int rc = search_grid(what, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, g);
+    if (rc != MVSB200_OK) return rc;
+    MVS_REQUIRE(max_dist > 0.f && isfinite(max_dist) && slack >= 0.f, "%s: max_dist > 0 (finite), slack >= 0", what);
+    if (n == 0) return MVSB200_OK;
+    pc_nearest_kernel<IDX><<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
+                                                                                 (const int2*)blocks, g, slack, max_dist, dist, index);
+    MVS_CHECK_LAUNCH(what);
+    return MVSB200_OK;
+}
+
 }  // namespace
 
 extern "C" int mvsb200_pc_grid_keys(const float* xyz, int n, float ox, float oy, float oz, float cell, int nbx, int nby, int nbz,
@@ -942,32 +896,16 @@ extern "C" int mvsb200_pc_nearest(const float* query, int n, const float* pts, c
                                   float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, float* dist,
                                   void* stream) {
     MVS_REQUIRE(query && pts && cells && blocks && dist, "pc_nearest: null pointer");
-    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "pc_nearest: misaligned buffer");
-    MVS_REQUIRE(n >= 0, "pc_nearest: 0 <= n < 2^31 queries");
-    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "pc_nearest: cell > 0 and at most %d cells", MVSB200_PC_MAX_CELLS);
-    MVS_REQUIRE(max_dist > 0.f && isfinite(max_dist) && slack >= 0.f, "pc_nearest: max_dist > 0 (finite), slack >= 0");
-    if (n == 0) return MVSB200_OK;
-    pc_nearest_kernel<false><<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
-                                                                                   (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
-                                                                                   slack, max_dist, dist, nullptr);
-    MVS_CHECK_LAUNCH("pc_nearest");
-    return MVSB200_OK;
+    return nearest_launch<false>("pc_nearest", query, n, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, slack, max_dist, dist,
+                                 nullptr, stream);
 }
 
 extern "C" int mvsb200_pc_nearest_index(const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks,
                                         float ox, float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist,
                                         float* dist, int32_t* index, void* stream) {
     MVS_REQUIRE(query && pts && cells && blocks && dist && index, "pc_nearest_index: null pointer");
-    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "pc_nearest_index: misaligned buffer");
-    MVS_REQUIRE(n >= 0, "pc_nearest_index: 0 <= n < 2^31 queries");
-    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "pc_nearest_index: cell > 0 and at most %d cells", MVSB200_PC_MAX_CELLS);
-    MVS_REQUIRE(max_dist > 0.f && isfinite(max_dist) && slack >= 0.f, "pc_nearest_index: max_dist > 0 (finite), slack >= 0");
-    if (n == 0) return MVSB200_OK;
-    pc_nearest_kernel<true><<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>(query, n, (const float4*)pts, (const int2*)cells,
-                                                                                  (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
-                                                                                  slack, max_dist, dist, index);
-    MVS_CHECK_LAUNCH("pc_nearest_index");
-    return MVSB200_OK;
+    return nearest_launch<true>("pc_nearest_index", query, n, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, slack, max_dist, dist,
+                                index, stream);
 }
 
 extern "C" int mvsb200_pc_thin_neighbours(const float* pts, const int32_t* cells, const int32_t* rank_sorted, int n, float ox, float oy,
@@ -975,11 +913,11 @@ extern "C" int mvsb200_pc_thin_neighbours(const float* pts, const int32_t* cells
                                           int32_t* counts, int32_t* list, void* stream) {
     MVS_REQUIRE(pts && cells && rank_sorted, "pc_thin_neighbours: null pointer");
     MVS_REQUIRE(offsets ? list != nullptr : counts != nullptr, "pc_thin_neighbours: counts, or offsets and list");
-    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0, "pc_thin_neighbours: misaligned buffer");
     MVS_REQUIRE(n >= 1, "pc_thin_neighbours: 1 <= n < 2^31 points");
-    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "pc_thin_neighbours: cell > 0 and at most %d cells", MVSB200_PC_MAX_CELLS);
+    Grid g;
+    const int rc = search_grid("pc_thin_neighbours", pts, cells, nullptr, ox, oy, oz, cell, nbx, nby, nbz, g);
+    if (rc != MVSB200_OK) return rc;
     MVS_REQUIRE(dst > 0.0 && (double)cell >= dst, "pc_thin_neighbours: 0 < dst <= cell");
-    const Grid g{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell};
     if (offsets) {
         pc_thin_list_kernel<<<blocks_for(n), kThreads, 0, (cudaStream_t)stream>>>((const float4*)pts, (const int2*)cells, rank_sorted, n, g,
                                                                                   dst * dst, offsets, list);
@@ -1092,17 +1030,17 @@ template <bool NORMALS>
 int knn_launch(const char* what, const float* query, int n, const float* pts, const int32_t* cells, const int32_t* blocks, float ox,
                float oy, float oz, float cell, int nbx, int nby, int nbz, float slack, float max_dist, int k, float* dist,
                int32_t* index, const double* view, int view_mode, float* normals, void* stream) {
-    MVS_REQUIRE(aligned16(pts) && ((uintptr_t)cells & 7) == 0 && ((uintptr_t)blocks & 7) == 0, "%s: misaligned buffer", what);
     MVS_REQUIRE(n >= 0, "%s: 0 <= n < 2^31 queries", what);
-    MVS_REQUIRE(grid_ok(cell, nbx, nby, nbz), "%s: cell > 0 and at most %d cells", what, MVSB200_PC_MAX_CELLS);
+    Grid g;
+    const int rc = search_grid(what, pts, cells, blocks, ox, oy, oz, cell, nbx, nby, nbz, g);
+    if (rc != MVSB200_OK) return rc;
     MVS_REQUIRE(max_dist > 0.f && slack >= 0.f, "%s: max_dist > 0 (+inf allowed), slack >= 0", what);
     MVS_REQUIRE(k >= 1 && k <= kKnnMax, "%s: 1 <= k <= %d, got %d", what, kKnnMax, k);
     if (n == 0) return MVSB200_OK;
     const int smem = k * kThreads * (int)(sizeof(float) + sizeof(int));
     MVS_CUDA(cudaFuncSetAttribute(pc_knn_kernel<NORMALS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     pc_knn_kernel<NORMALS><<<blocks_for(n), kThreads, smem, (cudaStream_t)stream>>>(
-        query, n, (const float4*)pts, (const int2*)cells, (const int2*)blocks, Grid{ox, oy, oz, cell, nbx, nby, nbz, 1.0 / (double)cell},
-        slack, max_dist, k, dist, index, view, view_mode, normals);
+        query, n, (const float4*)pts, (const int2*)cells, (const int2*)blocks, g, slack, max_dist, k, dist, index, view, view_mode, normals);
     MVS_CHECK_LAUNCH(what);
     return MVSB200_OK;
 }
