@@ -39,7 +39,21 @@ extern std::atomic<uint64_t> g_launches;
             MVS_FAIL(MVSB200_E_LAUNCH, "%s: %s", #call, cudaGetErrorString(e_)); \
     } while (0)
 
+// return the error of a call that reports one (MVSB200_OK = 0 otherwise)
+#define MVS_TRY(call)                                               \
+    do {                                                            \
+        const int rc_ = (call);                                     \
+        if (rc_ != MVSB200_OK) return rc_;                          \
+    } while (0)
+
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// SM count of the current device; 148 (a B200) if the query fails
+inline int sm_count() {
+    int dev = 0, n = 0;
+    if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) return n;
+    return 148;
+}
 
 // Unsigned 32-bit division by a run-time constant without a divide instruction (multiply-high + shift; the branch-free
 // scheme of Granlund & Montgomery as used by libdivide; exact for every 32-bit numerator, checked by brute force on the host).

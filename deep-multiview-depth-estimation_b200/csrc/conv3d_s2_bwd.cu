@@ -264,8 +264,6 @@ int launch_s2_wgrad_lines(const void* big, const void* small, float* gw, int B, 
                           int Cs, int pad_d, int pad_h, int pad_w, const long long* ss, cudaStream_t st) {
     constexpr int ROWA = 4 * CB;
     constexpr int ATOMS = 128 / (2 * CB);
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "conv3d_s2_wgrad_lines: cuTensorMapEncodeTiled is not available from the driver");
     S2WgLineParams p;
     p.B = B; p.Ds = Ds; p.Hs = Hs; p.Ws = Ws; p.Db = Db; p.Hb = Hb;
     p.pad_d = pad_d; p.pad_h = pad_h; p.pad_w = pad_w;
@@ -289,16 +287,8 @@ int launch_s2_wgrad_lines(const void* big, const void* small, float* gw, int B, 
     MVS_REQUIRE(p.n_stages >= 2, "conv3d_s2_wgrad_lines: lines of %d voxels do not fit shared memory (Cb=%d, Cs=%d)", Ws, CB, Cs);
 
     CUtensorMap tm_big, tm_small;
-    {
-        const cuuint64_t rowb = (cuuint64_t)2 * CB;          // bytes of one voxel of big
-        const cuuint64_t dims[5] = {(cuuint64_t)2 * CB, (cuuint64_t)Wb / 2, (cuuint64_t)Hb, (cuuint64_t)Db, (cuuint64_t)B};
-        const cuuint64_t strides[4] = {2 * rowb, rowb * Wb, rowb * Wb * Hb, rowb * Wb * Hb * Db};
-        const cuuint32_t box[5] = {(cuuint32_t)2 * CB, (cuuint32_t)(Ws + 1), 1, 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_big, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(big), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWA), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s2_wgrad_lines: cuTensorMapEncodeTiled(big) failed (%d)", (int)r);
-    }
+    // big as rows of voxel pairs (Wb is even): 2 * CB channels, Wb / 2 rows per line
+    MVS_TRY(encode_volume(&tm_big, big, 2 * CB, 2 * CB, Wb / 2, Hb, Db, B, Ws + 1, 1, "conv3d_s2_wgrad_lines", "big"));
     {
         // voxel-row strides of small in bytes: dense channel-last, or those of the allocation the box lives in (ss: elements)
         const cuuint64_t rowb = (cuuint64_t)2 * Cs;
@@ -307,30 +297,15 @@ int launch_s2_wgrad_lines(const void* big, const void* small, float* gw, int B, 
         const cuuint64_t strides[4] = {ss ? (cuuint64_t)ss[3] * 2 : dense[0], ss ? (cuuint64_t)ss[2] * 2 : dense[1],
                                        ss ? (cuuint64_t)ss[1] * 2 : dense[2], ss ? (cuuint64_t)ss[0] * 2 : dense[3]};
         const cuuint32_t box[5] = {(cuuint32_t)p.chunk_ch, (cuuint32_t)Ws, 1, 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_small, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(small), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWG), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s2_wgrad_lines: cuTensorMapEncodeTiled(small) failed (%d)", (int)r);
+        MVS_TRY(encode_tiled(&tm_small, small, 5, dims, strides, box, swizzle_for(ROWG), "conv3d_s2_wgrad_lines", "small"));
     }
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
+    int sms = sm_count();
     if (sms < 3) sms = 3;
     // lines of small per item: balance (items per CTA of a depth tap) x (lines + the extra big lines at an item's start)
     const long nrank = p.nkd == 1 ? sms / 3 : sms;
-    long best_cost = -1;
-    int best_nyc = 1;
-    for (int nyc = 1; nyc <= Hs; ++nyc) {
-        const int yc = (Hs + nyc - 1) / nyc;
-        if ((long)(nyc - 1) * yc >= Hs) continue;
-        const long items = (long)B * Ds * nyc;
-        const long cost = ((items + nrank - 1) / nrank) * (yc + 2);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_nyc = nyc; }
-    }
-    p.nychunks = best_nyc;
-    p.ychunk = (Hs + best_nyc - 1) / best_nyc;
+    const Runs runs = choose_runs(Ds, B, Hs, nrank, 2);
+    p.nychunks = runs.nchunks;
+    p.ychunk = runs.chunk;
     p.gw = gw;
     p.dbg = 0;
     if (const char* e = getenv("MVSB200_S2WG_DBG")) p.dbg = atoi(e);
@@ -641,8 +616,6 @@ template <int NOUT>
 int launch_deconv_kc(const void* x, int x_cs, const void* w, const int* kc_off, const int* kc_n, int n_kc, void* y, int B, int Di,
                      int Hi, int Wi, int Do, int Ho, int Wo, int cout, int n_rows, int pad_d, int pad_h, int pad_w,
                      const long long* ys, int accumulate, cudaStream_t st) {
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "deconv3d_s2_kc: cuTensorMapEncodeTiled is not available from the driver");
     DeconvKcParams p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo;
     p.Jd = (Do + 1) / 2; p.Jh = (Ho + 1) / 2; p.Jw = (Wo + 1) / 2;
@@ -650,7 +623,7 @@ int launch_deconv_kc(const void* x, int x_cs, const void* w, const int* kc_off, 
     p.n_split = (cout + NOUT - 1) / NOUT;
     p.dbg = 0;
     if (const char* e = getenv("MVSB200_KC_DBG")) p.dbg = atoi(e);
-    { const int rc = build_deconv_wide(pad_d, pad_h, pad_w, NOUT, p.g); if (rc != MVSB200_OK) return rc; }
+    MVS_TRY(build_deconv_wide(pad_d, pad_h, pad_w, NOUT, p.g));
     {
         int ksteps = 0;
         for (int c = 0; c < n_kc; ++c) ksteps += kc_n[c] / 16;
@@ -691,51 +664,21 @@ int launch_deconv_kc(const void* x, int x_cs, const void* w, const int* kc_off, 
     CUtensorMap tm_x[kKcMax], tm_w[kKcMax];
     const char* wp = reinterpret_cast<const char*>(w);
     for (int c = 0; c < n_kc; ++c) {
-        const int rowb = 2 * kc_n[c];
-        {
-            const cuuint64_t vox = (cuuint64_t)x_cs * 2;
-            const cuuint64_t dims[5] = {(cuuint64_t)x_cs, (cuuint64_t)Wi, (cuuint64_t)Hi, (cuuint64_t)Di, (cuuint64_t)B};
-            const cuuint64_t strides[4] = {vox, vox * Wi, vox * Wi * Hi, vox * Wi * Hi * Di};
-            const cuuint32_t box[5] = {(cuuint32_t)kc_n[c], (cuuint32_t)p.BW, (cuuint32_t)(p.L + 1), 1, 1};
-            const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-            CUresult r = enc(&tm_x[c], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), dims, strides, box, es,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(rowb), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            MVS_REQUIRE(r == CUDA_SUCCESS, "deconv3d_s2_kc: cuTensorMapEncodeTiled(x, chunk %d) failed (%d)", c, (int)r);
-        }
-        {
-            // packed filter of the chunk: [28 * n_rows][kc_n] bf16 (tap 27 = zeros), chunks one after the other
-            const cuuint64_t dims[2] = {(cuuint64_t)kc_n[c], (cuuint64_t)28 * n_rows};
-            const cuuint64_t strides[1] = {(cuuint64_t)rowb};
-            const cuuint32_t box[2] = {(cuuint32_t)kc_n[c], (cuuint32_t)NOUT};
-            const cuuint32_t es[2] = {1, 1};
-            CUresult r = enc(&tm_w[c], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<char*>(wp), dims, strides, box, es,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(rowb), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            MVS_REQUIRE(r == CUDA_SUCCESS, "deconv3d_s2_kc: cuTensorMapEncodeTiled(w, chunk %d) failed (%d)", c, (int)r);
-            wp += (size_t)28 * n_rows * rowb;
-        }
+        MVS_TRY(encode_volume(&tm_x[c], x, x_cs, kc_n[c], Wi, Hi, Di, B, p.BW, p.L + 1, "deconv3d_s2_kc", "x, chunk", c));
+        // packed filter of the chunk: [28 * n_rows][kc_n] bf16 (tap 27 = zeros), chunks one after the other
+        MVS_TRY(encode_filter(&tm_w[c], wp, kc_n[c], 28 * n_rows, NOUT, "deconv3d_s2_kc", "w, chunk", c));
+        wp += (size_t)28 * n_rows * 2 * kc_n[c];
     }
     for (int c = n_kc; c < kKcMax; ++c) { tm_x[c] = tm_x[0]; tm_w[c] = tm_w[0]; }
     p.y_sb = ys[0]; p.y_sd = ys[1]; p.y_sh = ys[2]; p.y_sw = ys[3];
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
     p.wide_io = (cout % 16 == 0 && ys[0] % 16 == 0 && ys[1] % 16 == 0 && ys[2] % 16 == 0 && ys[3] % 16 == 0 && ((uintptr_t)y & 31u) == 0) ? 1 : 0;
     const long tiles = (long)p.tiles_x * p.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, nsm = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && nsm > 0) sms = nsm;
-    }
+    const int sms = sm_count();
     const long walkers_max = sms / p.n_split > 0 ? sms / p.n_split : 1;
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= p.Jd; ++nc) {
-        const int dc = (p.Jd + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= p.Jd) continue;
-        const long items = tiles * nc * B;
-        const long cost = ((items + walkers_max - 1) / walkers_max) * (dc + 3);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (p.Jd + best_chunks - 1) / best_chunks;
+    const Runs runs = choose_runs(tiles, B, p.Jd, walkers_max, 3);
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     p.n_items = (int)(tiles * p.nchunks * B);
     const long walkers = p.n_items < walkers_max ? p.n_items : walkers_max;
     if (p.dbg & 4) fprintf(stderr, "kc: NOUT=%d split=%d BW=%d L=%d tiles=%dx%d dchunk=%d nchunks=%d items=%d groups=%d slots=%d slab=%d w=%d\n", NOUT, p.n_split, p.BW, p.L, p.tiles_x, p.tiles_y, p.dchunk, p.nchunks, p.n_items, p.g.n_groups, p.g.n_slots, p.slab_bytes, p.w_bytes);
@@ -755,15 +698,14 @@ extern "C" int mvsb200_conv3d_s2_wgrad_lines(const void* big, const void* small,
                                              int Ds, int Hs, int Ws, int Cs, int pad_d, int pad_h, int pad_w,
                                              const int64_t* small_strides4, void* stream) {
     const char* name = "conv3d_s2_wgrad_lines";
-    MVS_REQUIRE(big && small && gw, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(big) && aligned16(small) && aligned16(gw), "%s: pointers must be 16-byte aligned", name);
+    MVS_TRY(check_pointers(name, {big, small, gw}));
     MVS_REQUIRE(B >= 1 && B <= 65535 && Db >= 1 && Hb >= 1 && Wb >= 2 && Ds >= 1 && Hs >= 1 && Ws >= 1, "%s: bad shape", name);
     MVS_REQUIRE(Wb % 2 == 0, "%s: the strided operand needs an even number of voxels per line (got %d)", name, Wb);
     MVS_REQUIRE(Ws + 1 <= 256, "%s: lines of the dense operand are limited to 255 voxels (got %d)", name, Ws);
     MVS_REQUIRE(Cb == 8 || Cb == 16 || Cb == 32, "%s: the strided operand must have 8, 16 or 32 channels (got %d)", name, Cb);
     MVS_REQUIRE(Cs == 16 || Cs == 32 || Cs == 64 || (Cs > 64 && Cs <= 128 && Cs % 16 == 0),
                 "%s: the dense operand needs 16, 32, 64 or 80..128 (multiple of 16) channels (got %d)", name, Cs);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
+    MVS_TRY(check_pads(name, pad_d, pad_h, pad_w));
     long long ssv[4];
     const long long* ss = nullptr;
     if (small_strides4) {
@@ -786,8 +728,7 @@ extern "C" int mvsb200_deconv3d_s2_kc_fwd(const void* x, int x_cs, const void* w
                                           void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout, int n_rows,
                                           int pad_d, int pad_h, int pad_w, const int64_t* y_strides4, int accumulate, void* stream) {
     const char* name = "deconv3d_s2_kc_fwd";
-    MVS_REQUIRE(x && w_packed && y && y_strides4 && kc_off && kc_n, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "%s: pointers must be 16-byte aligned", name);
+    MVS_TRY(check_pointers(name, {x, w_packed, y}, {y_strides4, kc_off, kc_n}));
     MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
     MVS_REQUIRE(n_kc >= 1 && n_kc <= 3 && x_cs % 8 == 0, "%s: 1..3 K chunks, channel stride a multiple of 8 (got %d, %d)", name, n_kc, x_cs);
     int ktot = 0;
@@ -798,9 +739,9 @@ extern "C" int mvsb200_deconv3d_s2_kc_fwd(const void* x, int x_cs, const void* w
     }
     MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 64,
                 "%s: cout must be a multiple of 8 and n_rows a multiple of 16 <= 64 (cout=%d n_rows=%d)", name, cout, n_rows);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
-    const long long ys[4] = {(long long)y_strides4[0], (long long)y_strides4[1], (long long)y_strides4[2], (long long)y_strides4[3]};
-    for (int i = 0; i < 4; ++i) MVS_REQUIRE(ys[i] % 8 == 0, "%s: output strides must be multiples of 8 elements", name);
+    MVS_TRY(check_pads(name, pad_d, pad_h, pad_w));
+    long long ys[4];
+    MVS_TRY(copy_strides(name, y_strides4, ys));
     cudaStream_t st = (cudaStream_t)stream;
     // output channels per CTA: 32 while the filter (31 slots x 32 x K) and three slabs fit shared memory, else 16; the CTAs of
     // one launch share the channel groups (blockIdx % n_split)

@@ -20,6 +20,7 @@
 // Warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (one elected lane) + TMEM allocator, warps 2..5 = epilogue.
 #include "tc_common.cuh"
 #include <stdlib.h>
+#include <type_traits>
 
 using namespace mvsb200;
 
@@ -247,23 +248,36 @@ struct TilePlan {
     double score;
 };
 
-// pick the slab geometry: maximise useful rows per MMA row and per loaded row within the shared-memory budget
-TilePlan plan_tiles(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget) {
+// Slab geometry for MB 128-row blocks: BW voxels per line of which `halo` are halo columns, L = MB * 128 / BW output lines
+// plus `halo` halo lines, `slots` slabs in the ring next to the resident filter.  Maximises useful rows per MMA row and per
+// loaded row over BW = bw0, bw0 + bw_step, ... 256 within the shared-memory budget; the first BW wins a tie.  score <= 0:
+// nothing fits.
+TilePlan plan_slab(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget, int MB, int slots, int halo, int bw0,
+                   int bw_step) {
+    TilePlan best{};
+    best.score = -1.0;
+    for (int BW = bw0; BW <= 256; BW += bw_step) {
+        const int L = (MB * 128) / BW;
+        if (L < 1 || L + halo > 256) continue;
+        const int rows = MB * 128 + halo * BW + 2;
+        const int slab = ((rows * rowb) + 1023) / 1024 * 1024;
+        if (w_bytes_al + (size_t)slots * slab + 256 > smem_budget) continue;
+        const int tiles_x = (Wo + BW - 1 - halo) / (BW - halo), tiles_y = (Ho + L - 1) / L;
+        const double mma_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * MB * 128);
+        const double load_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * (L + halo) * BW);
+        const double score = mma_eff * (0.5 + 0.5 * load_eff);
+        if (score > best.score) best = TilePlan{BW, L, MB, tiles_x, tiles_y, slab, score};
+    }
+    return best;
+}
+
+// the best slab over MB = 1, 2, 4 blocks (the smaller MB wins a tie)
+TilePlan plan_tiles(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget, int slots, int halo, int bw0, int bw_step) {
     TilePlan best{};
     best.score = -1.0;
     for (int MB = 1; MB <= kMaxMB; MB *= 2) {
-        for (int BW = 10; BW <= 256; BW += 2) {
-            const int L = (MB * 128) / BW;
-            if (L < 1 || L + 2 > 256) continue;
-            const int rows = MB * 128 + 2 * BW + 2;
-            const int slab = ((rows * rowb) + 1023) / 1024 * 1024;
-            if (w_bytes_al + (size_t)kSlots3 * slab + 256 > smem_budget) continue;
-            const int tiles_x = (Wo + BW - 3) / (BW - 2), tiles_y = (Ho + L - 1) / L;
-            const double mma_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * MB * 128);
-            const double load_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * (L + 2) * BW);
-            const double score = mma_eff * (0.5 + 0.5 * load_eff);
-            if (score > best.score) best = TilePlan{BW, L, MB, tiles_x, tiles_y, slab, score};
-        }
+        const TilePlan tp = plan_slab(Ho, Wo, rowb, w_bytes_al, smem_budget, MB, slots, halo, bw0, bw_step);
+        if (tp.score > best.score) best = tp;
     }
     return best;
 }
@@ -274,34 +288,13 @@ int launch_conv(const void* x, const void* w, void* y, int B, int Di, int Hi, in
                 const long long* y_strides4, cudaStream_t st) {
     constexpr int ROWB = CIN * 2;
     constexpr size_t W_BYTES_AL = ((size_t)27 * NOUT * ROWB + 1023) / 1024 * 1024;
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "conv3d_s1: cuTensorMapEncodeTiled is not available from the driver");
     const size_t smem_budget = 227 * 1024 - 1024;       // 1024 for the manual alignment of the dynamic window
-    const TilePlan tp = plan_tiles(Ho, Wo, ROWB, W_BYTES_AL, smem_budget);
+    const TilePlan tp = plan_tiles(Ho, Wo, ROWB, W_BYTES_AL, smem_budget, kSlots3, 2, 10, 2);
     MVS_REQUIRE(tp.score > 0, "conv3d_s1: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
 
     CUtensorMap tm_x, tm_w;
-    {
-        const cuuint64_t dims[5] = {(cuuint64_t)CIN, (cuuint64_t)Wi, (cuuint64_t)Hi, (cuuint64_t)Di, (cuuint64_t)B};
-        const cuuint64_t strides[4] = {(cuuint64_t)ROWB, (cuuint64_t)ROWB * Wi, (cuuint64_t)ROWB * Wi * Hi,
-                                       (cuuint64_t)ROWB * Wi * Hi * Di};
-        const cuuint32_t box[5] = {(cuuint32_t)CIN, (cuuint32_t)tp.BW, (cuuint32_t)(tp.L + 2), 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1: cuTensorMapEncodeTiled(x) failed (%d)", (int)r);
-    }
-    {
-        const cuuint64_t dims[2] = {(cuuint64_t)CIN, (cuuint64_t)27 * n_rows};
-        const cuuint64_t strides[1] = {(cuuint64_t)ROWB};
-        const cuuint32_t box[2] = {(cuuint32_t)CIN, (cuuint32_t)NOUT};
-        const cuuint32_t es[2] = {1, 1};
-        CUresult r = enc(&tm_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1: cuTensorMapEncodeTiled(w) failed (%d)", (int)r);
-    }
+    MVS_TRY(encode_volume(&tm_x, x, CIN, CIN, Wi, Hi, Di, B, tp.BW, tp.L + 2, "conv3d_s1", "x"));
+    MVS_TRY(encode_filter(&tm_w, w, CIN, 27 * n_rows, NOUT, "conv3d_s1", "w"));
 
     ConvParams p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo;
@@ -316,25 +309,12 @@ int launch_conv(const void* x, const void* w, void* y, int B, int Di, int Hi, in
         p.y_sw = y_cs; p.y_sh = (long long)Wo * y_cs; p.y_sd = (long long)Ho * Wo * y_cs; p.y_sb = (long long)Do * Ho * Wo * y_cs;
     }
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
-    // depth runs: an item costs (planes + 2 halo planes + ~2 planes of pipeline fill); CTAs are persistent, one per SM,
-    // so pick the run length that minimises (items per CTA) x (cost per item)
+    // depth runs: an item costs its planes + 2 halo planes + ~2 planes of pipeline fill; one persistent CTA per SM
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= Do; ++nc) {
-        const int dc = (Do + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= Do) continue;           // would leave an empty run
-        const long items = tiles * nc * B;
-        const long cost = ((items + sms - 1) / sms) * (dc + 4);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (Do + best_chunks - 1) / best_chunks;
+    const int sms = sm_count();
+    const Runs runs = choose_runs(tiles, B, Do, sms, 4);
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     if (const char* e = getenv("MVSB200_CONV_DCHUNK")) {
         int v = atoi(e);
         if (v > 0) { p.dchunk = v < Do ? v : Do; p.nchunks = (Do + p.dchunk - 1) / p.dchunk; }
@@ -615,8 +595,6 @@ int launch_wgrad(const void* x, const void* gy, float* gw, int B, int Di, int Hi
     constexpr int ROWG = NCO * 2;
     constexpr int ROWX_BOX = CIN * 2;
     const int ROWX = cin_real * 2;
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "conv3d_s1_wgrad: cuTensorMapEncodeTiled is not available from the driver");
     const size_t smem_budget = 227 * 1024 - 1024;
     const WgPlan tp = plan_tiles_wgrad(Ho, Wo, ROWX_BOX, ROWG, smem_budget);
     MVS_REQUIRE(tp.score > 0, "conv3d_s1_wgrad: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NCO);
@@ -627,22 +605,9 @@ int launch_wgrad(const void* x, const void* gy, float* gw, int B, int Di, int Hi
         const cuuint64_t strides[4] = {(cuuint64_t)x_es * ROWX, (cuuint64_t)x_es * ROWX * Wx, (cuuint64_t)x_es * ROWX * Wx * Hx,
                                        (cuuint64_t)ROWX * Wx * Hx * Dx};
         const cuuint32_t box[5] = {(cuuint32_t)CIN, (cuuint32_t)tp.BW, (cuuint32_t)(tp.L + 2), 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWX_BOX), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1_wgrad: cuTensorMapEncodeTiled(x) failed (%d)", (int)r);
+        MVS_TRY(encode_tiled(&tm_x, x, 5, dims, strides, box, swizzle_for(ROWX_BOX), "conv3d_s1_wgrad", "x"));
     }
-    {
-        const cuuint64_t rowb = (cuuint64_t)cout * 2;
-        const cuuint64_t dims[5] = {(cuuint64_t)cout, (cuuint64_t)Wo, (cuuint64_t)Ho, (cuuint64_t)Do, (cuuint64_t)B};
-        const cuuint64_t strides[4] = {rowb, rowb * Wo, rowb * Wo * Ho, rowb * Wo * Ho * Do};
-        const cuuint32_t box[5] = {(cuuint32_t)NCO, (cuuint32_t)(tp.BW - 2), 1, 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        const CUtensorMapSwizzle sw = ROWG == 16 ? CU_TENSOR_MAP_SWIZZLE_NONE : swizzle_for(ROWG);
-        CUresult r = enc(&tm_g, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(gy), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1_wgrad: cuTensorMapEncodeTiled(gy) failed (%d)", (int)r);
-    }
+    MVS_TRY(encode_volume(&tm_g, gy, cout, NCO, Wo, Ho, Do, B, tp.BW - 2, 1, "conv3d_s1_wgrad", "gy"));
     WgradParams p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.off_d = off_d; p.off_h = off_h; p.off_w = off_w;
     p.BW = tp.BW; p.L = tp.L; p.tiles_x = tp.tiles_x; p.tiles_y = tp.tiles_y;
@@ -656,11 +621,7 @@ int launch_wgrad(const void* x, const void* gy, float* gw, int B, int Di, int Hi
     for (int t = 0; t < 27; ++t) p.tap_map[t] = tap_map ? tap_map[t] : t;
     p.gw = gw;
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
+    const int sms = sm_count();
     long walkers = sms / n_roles > 0 ? sms / n_roles : 1;          // CTAs that walk the items (each role has that many)
     {
         // every CTA ends with red.global.add of its whole accumulator set (up to 27 x CIN x NCO floats) onto the same addresses: on a
@@ -671,17 +632,9 @@ int launch_wgrad(const void* x, const void* gy, float* gw, int B, int Di, int Hi
         const long cap = potential / (kMinPlaneTiles > 0 ? kMinPlaneTiles : 1);
         if (cap < walkers) walkers = cap > 0 ? cap : 1;
     }
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= Do; ++nc) {
-        const int dc = (Do + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= Do) continue;
-        const long items = tiles * nc * B;
-        const long cost = ((items + walkers - 1) / walkers) * (dc + 4);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (Do + best_chunks - 1) / best_chunks;
+    const Runs runs = choose_runs(tiles, B, Do, walkers, 4);
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     p.n_items = (int)(tiles * p.nchunks * B);
     const dim3 grid((unsigned)((p.n_items < walkers ? p.n_items : walkers) * n_roles), 1, 1);
     const size_t smem = 1024 + (size_t)kSlots3 * tp.slab_bytes + 2 * (size_t)tp.gy_bytes + 256;
@@ -968,42 +921,19 @@ __global__ void s2_stats_finalize_kernel(const float* __restrict__ partials, int
     sums[t] = (float)acc;
 }
 
-static thread_local float* g_s2_stats = nullptr;    // set by mvsb200_conv3d_s2_fwd_stats around its launches
-static thread_local int g_s2_stats_cs = 0;
-static thread_local int g_s2_stats_blocks = 0;      // largest grid of those launches
-
-TilePlan plan_tiles_s2(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget) {
-    TilePlan best{};
-    best.score = -1.0;
-    for (int MB = 1; MB <= kMaxMB; MB *= 2) {
-        for (int BW = 9; BW <= 256; ++BW) {
-            const int L = (MB * 128) / BW;
-            if (L < 1 || L + 1 > 256) continue;
-            const int rows = MB * 128 + BW + 2;
-            const int slab = ((rows * rowb) + 1023) / 1024 * 1024;
-            if (w_bytes_al + (size_t)kS2Slots * slab + 256 > smem_budget) continue;
-            const int tiles_x = (Wo + BW - 2) / (BW - 1), tiles_y = (Ho + L - 1) / L;
-            const double mma_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * MB * 128);
-            const double load_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * (L + 1) * BW);
-            const double score = mma_eff * (0.5 + 0.5 * load_eff);
-            if (score > best.score) best = TilePlan{BW, L, MB, tiles_x, tiles_y, slab, score};
-        }
-    }
-    return best;
-}
-
+// stats: null, or the per-CTA statistics rows [grid][2][stats_cs] of the epilogue (ConvS2Params); the launch's grid size is
+// then raised into *n_blocks
 template <int CIN, int NOUT>
 int launch_conv_s2(const void* x, const void* w, void* y, int B, int Dx, int Hx, int Wx, int Do, int Ho, int Wo, int cout, int y_cs,
-                   int y_coff, int n_rows, int w_row0, int pad_d, int pad_h, int pad_w, cudaStream_t st, int cin_real = CIN) {
+                   int y_coff, int n_rows, int w_row0, int pad_d, int pad_h, int pad_w, cudaStream_t st, int cin_real, float* stats,
+                   int stats_cs, int* n_blocks) {
     // cin_real < CIN: voxel rows of x hold cin_real channels; the TMA box is CIN wide and the channels beyond the tensor's
     // extent arrive as zeros (out-of-bounds fill), so an 8-channel volume feeds the K = 16 MMA without a widened copy
     constexpr int ROWB = CIN * 2;
     const int rowx = cin_real * 2;
     constexpr size_t W_BYTES_AL = ((size_t)27 * NOUT * ROWB + 1023) / 1024 * 1024;
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "conv3d_s2: cuTensorMapEncodeTiled is not available from the driver");
     const size_t smem_budget = 227 * 1024 - 1024;
-    const TilePlan tp = plan_tiles_s2(Ho, Wo, ROWB, W_BYTES_AL, smem_budget);
+    const TilePlan tp = plan_tiles(Ho, Wo, ROWB, W_BYTES_AL, smem_budget, kS2Slots, 1, 9, 1);
     MVS_REQUIRE(tp.score > 0, "conv3d_s2: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
 
     CUtensorMap tm_x[4], tm_w;
@@ -1019,52 +949,27 @@ int launch_conv_s2(const void* x, const void* w, void* y, int B, int Dx, int Hx,
         const cuuint64_t strides[4] = {(cuuint64_t)2 * rowx, (cuuint64_t)2 * rowx * Wx, (cuuint64_t)rowx * Wx * Hx,
                                        (cuuint64_t)rowx * Wx * Hx * Dx};
         const cuuint32_t box[5] = {(cuuint32_t)CIN, (cuuint32_t)tp.BW, (cuuint32_t)(tp.L + 1), 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_x[c], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<char*>(base), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s2: cuTensorMapEncodeTiled(x, class %d) failed (%d)", c, (int)r);
+        MVS_TRY(encode_tiled(&tm_x[c], base, 5, dims, strides, box, swizzle_for(ROWB), "conv3d_s2", "x, class", c));
     }
-    {
-        const cuuint64_t dims[2] = {(cuuint64_t)CIN, (cuuint64_t)27 * n_rows};
-        const cuuint64_t strides[1] = {(cuuint64_t)ROWB};
-        const cuuint32_t box[2] = {(cuuint32_t)CIN, (cuuint32_t)NOUT};
-        const cuuint32_t es[2] = {1, 1};
-        CUresult r = enc(&tm_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s2: cuTensorMapEncodeTiled(w) failed (%d)", (int)r);
-    }
+    MVS_TRY(encode_filter(&tm_w, w, CIN, 27 * n_rows, NOUT, "conv3d_s2", "w"));
     ConvS2Params p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.pad_d = pad_d; p.pad_h = pad_h; p.pad_w = pad_w; p.Dx = Dx;
     p.BW = tp.BW; p.L = tp.L; p.MB = tp.MB; p.tiles_x = tp.tiles_x; p.tiles_y = tp.tiles_y;
     p.cout = cout; p.y_cs = y_cs; p.y_coff = y_coff; p.n_rows = n_rows; p.w_row0 = w_row0;
     p.slab_bytes = tp.slab_bytes;
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
-    p.stats = g_s2_stats;
-    p.stats_cs = g_s2_stats_cs;
+    p.stats = stats;
+    p.stats_cs = stats_cs;
     MVS_REQUIRE(p.stats == nullptr || (size_t)kS2Slots * tp.slab_bytes >= (size_t)4 * 2 * NOUT * sizeof(float), "conv3d_s2: slab ring too small for the statistics rows");
     MVS_REQUIRE(p.stats == nullptr || 2 * cout <= kTcThreads, "conv3d_s2: %d channels per launch with statistics", cout);
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= Do; ++nc) {
-        const int dc = (Do + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= Do) continue;
-        const long items = tiles * nc * B;
-        const long cost = ((items + sms - 1) / sms) * (dc + 1);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (Do + best_chunks - 1) / best_chunks;
+    const int sms = sm_count();
+    const Runs runs = choose_runs(tiles, B, Do, sms, 1);
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     p.n_items = (int)(tiles * p.nchunks * B);
     const dim3 grid((unsigned)(p.n_items < sms ? p.n_items : sms), 1, 1);
-    if ((int)grid.x > g_s2_stats_blocks) g_s2_stats_blocks = (int)grid.x;
+    if (n_blocks && (int)grid.x > *n_blocks) *n_blocks = (int)grid.x;
     const size_t smem = 1024 + W_BYTES_AL + (size_t)kS2Slots * tp.slab_bytes + 256;
     if (p.stats != nullptr) {
         // epilogue statistics: instantiated for the cost volume's 32 channels (the stacked branches, scripts/model.py:104-110)
@@ -1323,43 +1228,18 @@ conv3d_s1_kdn_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_cons
     }
 }
 
-TilePlan plan_tiles_mb(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget, int MB);
-
-static thread_local int g_kdn_planar = 0;        // set by mvsb200_conv2d_rows_fwd around its call of the kdn dispatch
-
-template <int CIN, int NOUT, int MB, bool AFF = false>
+// planar: KdnParams::planar
+template <int CIN, int NOUT, int MB, bool AFF>
 int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
                        int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, const TilePlan& tp, int slots,
-                       cudaStream_t st, int cin_real = CIN, const float* scale = nullptr, const float* shift = nullptr) {
+                       int planar, cudaStream_t st, int cin_real, const float* scale, const float* shift) {
     // cin_real < CIN: voxel rows of x hold cin_real channels; the TMA box is CIN wide, the channels beyond the tensor's extent
     // arrive as zeros (out-of-bounds fill) -- an 8-channel volume feeds the K = 16 MMA without a widened copy
     constexpr int ROWB = CIN * 2;
-    const int rowx = cin_real * 2;
     constexpr size_t W_BYTES_AL = ((size_t)27 * NOUT * ROWB + 1023) / 1024 * 1024;
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "conv3d_s1_kdn: cuTensorMapEncodeTiled is not available from the driver");
     CUtensorMap tm_x, tm_w;
-    {
-        const cuuint64_t dims[5] = {(cuuint64_t)cin_real, (cuuint64_t)Wi, (cuuint64_t)Hi, (cuuint64_t)Di, (cuuint64_t)B};
-        const cuuint64_t strides[4] = {(cuuint64_t)rowx, (cuuint64_t)rowx * Wi, (cuuint64_t)rowx * Wi * Hi,
-                                       (cuuint64_t)rowx * Wi * Hi * Di};
-        const cuuint32_t box[5] = {(cuuint32_t)CIN, (cuuint32_t)tp.BW, (cuuint32_t)(tp.L + 2), 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1_kdn: cuTensorMapEncodeTiled(x) failed (%d)", (int)r);
-    }
-    {
-        const cuuint64_t dims[2] = {(cuuint64_t)CIN, (cuuint64_t)27 * n_rows};
-        const cuuint64_t strides[1] = {(cuuint64_t)ROWB};
-        const cuuint32_t box[2] = {(cuuint32_t)CIN, (cuuint32_t)NOUT};
-        const cuuint32_t es[2] = {1, 1};
-        CUresult r = enc(&tm_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "conv3d_s1_kdn: cuTensorMapEncodeTiled(w) failed (%d)", (int)r);
-    }
+    MVS_TRY(encode_volume(&tm_x, x, cin_real, CIN, Wi, Hi, Di, B, tp.BW, tp.L + 2, "conv3d_s1_kdn", "x"));
+    MVS_TRY(encode_filter(&tm_w, w, CIN, 27 * n_rows, NOUT, "conv3d_s1_kdn", "w"));
     KdnParams kp;
     ConvParams& p = kp.c;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo;
@@ -1371,27 +1251,15 @@ int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int
     p.y_sw = y_cs; p.y_sh = (long long)Wo * y_cs; p.y_sd = (long long)Ho * Wo * y_cs; p.y_sb = (long long)Do * Ho * Wo * y_cs;
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
     kp.slots = slots;
-    kp.planar = g_kdn_planar;
+    kp.planar = planar;
     kp.scale = AFF ? scale + y_coff : nullptr;
     kp.shift = AFF ? shift + y_coff : nullptr;
-    const int halo = kp.planar ? 0 : 2;
+    const int halo = planar ? 0 : 2;
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= Do; ++nc) {
-        const int dc = (Do + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= Do) continue;
-        const long items = tiles * nc * B;
-        const long cost = ((items + sms - 1) / sms) * (dc + halo + 1);      // nd + 2 slabs per run (planar: nd) + pipeline fill
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (Do + best_chunks - 1) / best_chunks;
+    const int sms = sm_count();
+    const Runs runs = choose_runs(tiles, B, Do, sms, halo + 1);      // nd + 2 slabs per run (planar: nd) + pipeline fill
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     p.n_items = (int)(tiles * p.nchunks * B);
     const dim3 grid((unsigned)(p.n_items < sms ? p.n_items : sms), 1, 1);
     const size_t smem = 1024 + W_BYTES_AL + (size_t)slots * tp.slab_bytes + 256;
@@ -1401,10 +1269,10 @@ int launch_conv_kdn_mb(const void* x, const void* w, void* y, int B, int Di, int
     return MVSB200_OK;
 }
 
-template <int CIN, int NOUT, bool AFF = false>
+template <int CIN, int NOUT, bool AFF>
 int launch_conv_kdn(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
-                    int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, cudaStream_t st, int cin_real = CIN,
-                    const float* scale = nullptr, const float* shift = nullptr) {
+                    int y_cs, int y_coff, int n_rows, int w_row0, int off_d, int off_h, int off_w, int planar, cudaStream_t st,
+                    int cin_real, const float* scale, const float* shift) {
     constexpr int ROWB = CIN * 2;
     constexpr size_t W_BYTES_AL = ((size_t)27 * NOUT * ROWB + 1023) / 1024 * 1024;
     constexpr int MBMAX = 512 / (2 * 3 * NOUT) >= 4 ? 4 : (512 / (2 * 3 * NOUT) >= 2 ? 2 : 1);
@@ -1415,31 +1283,20 @@ int launch_conv_kdn(const void* x, const void* w, void* y, int B, int Di, int Hi
     int best_slots = 0;
     for (int MB = MBMAX; MB >= 1; MB /= 2) {
         for (int slots = 3; slots >= 2; --slots) {
-            // plan_tiles_mb budgets kSlots3 slabs: hand it the budget scaled to `slots`
-            TilePlan tp{};
-            tp.score = -1.0;
-            for (int BW = 6; BW <= 256; BW += 2) {
-                const int L = (MB * 128) / BW;
-                if (L < 1 || L + 2 > 256) continue;
-                const int rows = MB * 128 + 2 * BW + 2;
-                const int slab = ((rows * ROWB) + 1023) / 1024 * 1024;
-                if (W_BYTES_AL + (size_t)slots * slab + 256 > smem_budget) continue;
-                const int tiles_x = (Wo + BW - 3) / (BW - 2), tiles_y = (Ho + L - 1) / L;
-                const double mma_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * MB * 128);
-                const double load_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * (L + 2) * BW);
-                const double score = mma_eff * (0.5 + 0.5 * load_eff);
-                if (score > tp.score) tp = TilePlan{BW, L, MB, tiles_x, tiles_y, slab, score};
-            }
+            const TilePlan tp = plan_slab(Ho, Wo, ROWB, W_BYTES_AL, smem_budget, MB, slots, 2, 6, 2);
             if (tp.score > best.score * 1.02 || (best_slots == 0 && tp.score > 0)) { best = tp; best_slots = slots; }
             if (tp.score > 0) break;                      // a 3-deep ring fits for this MB: do not consider 2
         }
     }
     MVS_REQUIRE(best.score > 0, "conv3d_s1_kdn: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
-#define MVS_KDN(M) return launch_conv_kdn_mb<CIN, NOUT, M, AFF>(x, w, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, y_coff, n_rows, w_row0, off_d, off_h, off_w, best, best_slots, st, cin_real, scale, shift)
-    if (best.MB == 1) MVS_KDN(1);
-    if constexpr (MBMAX >= 2) { if (best.MB == 2) MVS_KDN(2); }
-    if constexpr (MBMAX >= 4) { if (best.MB == 4) MVS_KDN(4); }
-#undef MVS_KDN
+    auto run = [&](auto mb) {
+        return launch_conv_kdn_mb<CIN, NOUT, decltype(mb)::value, AFF>(x, w, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, y_coff, n_rows,
+                                                                      w_row0, off_d, off_h, off_w, best, best_slots, planar, st,
+                                                                      cin_real, scale, shift);
+    };
+    if (best.MB == 1) return run(std::integral_constant<int, 1>{});
+    if constexpr (MBMAX >= 2) { if (best.MB == 2) return run(std::integral_constant<int, 2>{}); }
+    if constexpr (MBMAX >= 4) { if (best.MB == 4) return run(std::integral_constant<int, 4>{}); }
     MVS_FAIL(MVSB200_E_UNSUPPORTED, "conv3d_s1_kdn: block count %d", best.MB);
 }
 
@@ -1783,37 +1640,15 @@ deconv3d_s2_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
     }
 }
 
-// slab geometry for a fixed number of 128-row blocks
-TilePlan plan_tiles_mb(int Ho, int Wo, int rowb, size_t w_bytes_al, size_t smem_budget, int MB) {
-    TilePlan best{};
-    best.score = -1.0;
-    for (int BW = 6; BW <= 256; BW += 2) {
-        const int L = (MB * 128) / BW;
-        if (L < 1 || L + 2 > 256) continue;
-        const int rows = MB * 128 + 2 * BW + 2;
-        const int slab = ((rows * rowb) + 1023) / 1024 * 1024;
-        if (w_bytes_al + (size_t)kSlots3 * slab + 256 > smem_budget) continue;
-        const int tiles_x = (Wo + BW - 3) / (BW - 2), tiles_y = (Ho + L - 1) / L;
-        const double mma_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * MB * 128);
-        const double load_eff = (double)Wo * Ho / ((double)tiles_x * tiles_y * (L + 2) * BW);
-        const double score = mma_eff * (0.5 + 0.5 * load_eff);
-        if (score > best.score) best = TilePlan{BW, L, MB, tiles_x, tiles_y, slab, score};
-    }
-    return best;
-}
-
 // EPI: win (host int[6]: lo_d, lo_h, lo_w, n_d, n_h, n_w) is the window of the Do x Ho x Wo canvas that is written, y / add
 // point at its origin; scale / shift / add as in DeconvParams.
 template <int CIN, int NOUT, bool EPI = false>
 int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int Hi, int Wi, int Do, int Ho, int Wo, int cout,
                      int n_rows, int pad_d, int pad_h, int pad_w, const long long* y_strides4, cudaStream_t st,
-                     float* stats = nullptr, int* n_blocks_out = nullptr, const int* win = nullptr, const float* scale = nullptr,
-                     const float* shift = nullptr, const void* add = nullptr) {
+                     float* stats, int* n_blocks_out, const int* win, const float* scale, const float* shift, const void* add) {
     constexpr int ROWB = CIN * 2;
     constexpr int MB = 512 / (16 * NOUT);
     constexpr size_t W_BYTES_AL = ((size_t)kDeconvSlots * NOUT * ROWB + 1023) / 1024 * 1024;
-    EncodeTiledFn enc = encode_fn();
-    MVS_REQUIRE(enc != nullptr, "deconv3d_s2: cuTensorMapEncodeTiled is not available from the driver");
     const size_t smem_budget = 227 * 1024 - 1024 - 1024;      // - the epilogue's statistics rows
     int Jd = (Do + 1) / 2, Jh = (Ho + 1) / 2, Jw = (Wo + 1) / 2;
     if (EPI) {
@@ -1821,31 +1656,12 @@ int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int H
         Jh = (win[1] + win[4] - 1) / 2 - win[1] / 2 + 1;
         Jw = (win[2] + win[5] - 1) / 2 - win[2] / 2 + 1;
     }
-    const TilePlan tp = plan_tiles_mb(Jh, Jw, ROWB, W_BYTES_AL, smem_budget, MB);
+    const TilePlan tp = plan_slab(Jh, Jw, ROWB, W_BYTES_AL, smem_budget, MB, kSlots3, 2, 6, 2);
     MVS_REQUIRE(tp.score > 0, "deconv3d_s2: no slab geometry fits shared memory (Cin=%d, N=%d)", CIN, NOUT);
 
     CUtensorMap tm_x, tm_w;
-    {
-        const cuuint64_t dims[5] = {(cuuint64_t)CIN, (cuuint64_t)Wi, (cuuint64_t)Hi, (cuuint64_t)Di, (cuuint64_t)B};
-        const cuuint64_t strides[4] = {(cuuint64_t)ROWB, (cuuint64_t)ROWB * Wi, (cuuint64_t)ROWB * Wi * Hi,
-                                       (cuuint64_t)ROWB * Wi * Hi * Di};
-        const cuuint32_t box[5] = {(cuuint32_t)CIN, (cuuint32_t)tp.BW, (cuuint32_t)(tp.L + 2), 1, 1};
-        const cuuint32_t es[5] = {1, 1, 1, 1, 1};
-        CUresult r = enc(&tm_x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void*>(x), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "deconv3d_s2: cuTensorMapEncodeTiled(x) failed (%d)", (int)r);
-    }
-    {
-        const cuuint64_t dims[2] = {(cuuint64_t)CIN, (cuuint64_t)28 * n_rows};      // 27 taps + the all-zero tap
-        const cuuint64_t strides[1] = {(cuuint64_t)ROWB};
-        const cuuint32_t box[2] = {(cuuint32_t)CIN, (cuuint32_t)NOUT};
-        const cuuint32_t es[2] = {1, 1};
-        CUresult r = enc(&tm_w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(w), dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(ROWB), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        MVS_REQUIRE(r == CUDA_SUCCESS, "deconv3d_s2: cuTensorMapEncodeTiled(w) failed (%d)", (int)r);
-    }
+    MVS_TRY(encode_volume(&tm_x, x, CIN, CIN, Wi, Hi, Di, B, tp.BW, tp.L + 2, "deconv3d_s2", "x"));
+    MVS_TRY(encode_filter(&tm_w, w, CIN, 28 * n_rows, NOUT, "deconv3d_s2", "w"));      // 27 taps + the all-zero tap
 
     DeconvParams p;
     p.B = B; p.Do = Do; p.Ho = Ho; p.Wo = Wo; p.Jd = Jd; p.Jh = Jh; p.Jw = Jw;
@@ -1858,29 +1674,17 @@ int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int H
     }
     p.BW = tp.BW; p.L = tp.L; p.MB = MB; p.tiles_x = tp.tiles_x; p.tiles_y = tp.tiles_y;
     p.cout = cout; p.n_rows = n_rows; p.slab_bytes = tp.slab_bytes;
-    { const int rc = build_deconv_wide(pad_d, pad_h, pad_w, NOUT, p.g); if (rc != MVSB200_OK) return rc; }
+    MVS_TRY(build_deconv_wide(pad_d, pad_h, pad_w, NOUT, p.g));
     MVS_REQUIRE(p.g.n_slots <= kDeconvSlots, "deconv3d_s2: %d filter slots", p.g.n_slots);
     p.y_sb = y_strides4[0]; p.y_sd = y_strides4[1]; p.y_sh = y_strides4[2]; p.y_sw = y_strides4[3];
     p.y = reinterpret_cast<__nv_bfloat16*>(y);
     p.wide_io = (cout % 16 == 0 && p.y_sb % 16 == 0 && p.y_sd % 16 == 0 && p.y_sh % 16 == 0 && p.y_sw % 16 == 0 && ((uintptr_t)y & 31u) == 0) ? 1 : 0;
 
     const long tiles = (long)tp.tiles_x * tp.tiles_y;
-    int sms = 148;
-    {
-        int dev = 0, nsm = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && nsm > 0) sms = nsm;
-    }
-    long best_cost = -1;
-    int best_chunks = 1;
-    for (int nc = 1; nc <= Jd; ++nc) {
-        const int dc = (Jd + nc - 1) / nc;
-        if ((long)(nc - 1) * dc >= Jd) continue;
-        const long items = tiles * nc * B;
-        const long cost = ((items + sms - 1) / sms) * (dc + 4);
-        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best_chunks = nc; }
-    }
-    p.nchunks = best_chunks;
-    p.dchunk = (Jd + best_chunks - 1) / best_chunks;
+    const int sms = sm_count();
+    const Runs runs = choose_runs(tiles, B, Jd, sms, 4);
+    p.nchunks = runs.nchunks;
+    p.dchunk = runs.chunk;
     p.n_items = (int)(tiles * p.nchunks * B);
     const dim3 grid((unsigned)(p.n_items < sms ? p.n_items : sms), 1, 1);
     const size_t smem = 1024 + W_BYTES_AL + (size_t)kSlots3 * tp.slab_bytes + 256 + 1024;
@@ -1892,35 +1696,56 @@ int launch_deconv_s2(const void* x, const void* w, void* y, int B, int Di, int H
     return MVSB200_OK;
 }
 
+// ---- entry points ---------------------------------------------------------------------------------------------
+// Channel dispatch: Ch<CI, N> is one instantiated pair of input channels and filter rows per launch; K is the kernel's
+// channel width (8-channel voxel rows run on the 16-channel kernel, whose TMA box reads the missing channels as zeros).
+template <int CI, int N>
+struct Ch { static constexpr int cin = CI, n = N, k = CI < 16 ? 16 : CI; };
+template <class... C>
+struct ChList {};
+using ConvChannels = ChList<Ch<16, 16>, Ch<16, 32>, Ch<32, 16>, Ch<32, 32>, Ch<64, 16>, Ch<64, 32>>;
+using KdnChannels = ChList<Ch<8, 16>, Ch<8, 32>, Ch<16, 16>, Ch<16, 32>, Ch<32, 16>, Ch<32, 32>, Ch<64, 16>, Ch<64, 32>>;
+using S2Channels = ChList<Ch<8, 16>, Ch<8, 32>, Ch<16, 16>, Ch<16, 32>, Ch<16, 48>, Ch<16, 64>, Ch<32, 16>, Ch<32, 32>, Ch<32, 48>,
+                          Ch<32, 64>, Ch<64, 16>, Ch<64, 32>>;
+using WgradChannels = ChList<Ch<16, 8>, Ch<16, 16>, Ch<16, 32>, Ch<32, 8>, Ch<32, 16>, Ch<32, 32>, Ch<64, 8>, Ch<64, 16>, Ch<64, 32>>;
+
+// runs f(C{}) for the listed pair C = (cin, n) and returns true with its result in rc; false if no pair is listed
+template <class... C, class F>
+bool dispatch(ChList<C...>, int cin, int n, int& rc, F&& f) {
+    return ((cin == C::cin && n == C::n && ((rc = f(C{})), true)) || ...);
+}
+
+// checks of the stride-1 forward entry points (conv3d_s1_fwd, conv3d_s1_fwd_ex and the kdn forms)
+int check_s1_fwd(const char* name, const void* x, const void* w, const void* y, int B, int Di, int Hi, int Wi, int Do, int Ho,
+                 int Wo, int cout, int y_cs, int n_rows) {
+    MVS_TRY(check_pointers(name, {x, w, y}));
+    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
+    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 64,
+                "%s: cout must be a multiple of 8 and n_rows a multiple of 16 <= 64 (cout=%d n_rows=%d)", name, cout, n_rows);
+    MVS_REQUIRE(y_cs >= cout && y_cs % 8 == 0, "%s: output channel stride %d", name, y_cs);
+    return MVSB200_OK;
+}
+
 }  // namespace
 
 static int conv3d_s1_dispatch(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin, int Do, int Ho,
                               int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w, unsigned tap_mask,
                               const long long* y_strides4, cudaStream_t st, const char* name) {
-    MVS_REQUIRE(x && w_packed && y, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "%s: pointers must be 16-byte aligned", name);
-    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
-    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 64,
-                "%s: cout must be a multiple of 8 and n_rows a multiple of 16 <= 64 (cout=%d n_rows=%d)", name, cout, n_rows);
-    MVS_REQUIRE(y_cs >= cout && y_cs % 8 == 0, "%s: output channel stride %d", name, y_cs);
+    MVS_TRY(check_s1_fwd(name, x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, n_rows));
     MVS_REQUIRE((tap_mask & 0x7ffffffu) != 0, "%s: empty tap mask", name);
     // N (filter rows per launch) is 16 or 32; a 64-row filter runs as two 32-row halves (all 27 taps of a 64 x 64
     // filter do not fit next to the slab ring; at N = 32 the tensor pipe is fed from shared memory at the same rate)
     for (int row0 = 0; row0 < n_rows && row0 < cout; row0 += 32) {
         const int nout = n_rows - row0 < 32 ? n_rows - row0 : 32;
         const int c_here = cout - row0 < nout ? cout - row0 : nout;
-        int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_CONV(CI, NO) \
-    rc = launch_conv<CI, NO>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, tap_mask, y_strides4, st)
-        if (Cin == 16 && nout == 16) MVS_CONV(16, 16);
-        else if (Cin == 16 && nout == 32) MVS_CONV(16, 32);
-        else if (Cin == 32 && nout == 16) MVS_CONV(32, 16);
-        else if (Cin == 32 && nout == 32) MVS_CONV(32, 32);
-        else if (Cin == 64 && nout == 16) MVS_CONV(64, 16);
-        else if (Cin == 64 && nout == 32) MVS_CONV(64, 32);
-        else MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
-#undef MVS_CONV
-        if (rc != MVSB200_OK) return rc;
+        int rc = MVSB200_OK;
+        if (!dispatch(ConvChannels{}, Cin, nout, rc, [&](auto c) {
+                using C = decltype(c);
+                return launch_conv<C::k, C::n>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h,
+                                               off_w, tap_mask, y_strides4, st);
+            }))
+            MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
+        MVS_TRY(rc);
     }
     return MVSB200_OK;
 }
@@ -1936,8 +1761,8 @@ extern "C" int mvsb200_conv3d_s1_fwd_ex(const void* x, const void* w_packed, voi
                                         int Do, int Ho, int Wo, int cout, int n_rows, int off_d, int off_h, int off_w,
                                         unsigned tap_mask, const int64_t* y_strides4, void* stream) {
     MVS_REQUIRE(y_strides4 != nullptr, "conv3d_s1_fwd_ex: null output strides");
-    const long long ys[4] = {(long long)y_strides4[0], (long long)y_strides4[1], (long long)y_strides4[2], (long long)y_strides4[3]};
-    for (int i = 0; i < 4; ++i) MVS_REQUIRE(ys[i] % 8 == 0, "conv3d_s1_fwd_ex: output strides must be multiples of 8 elements");
+    long long ys[4];
+    MVS_TRY(copy_strides("conv3d_s1_fwd_ex", y_strides4, ys));
     return conv3d_s1_dispatch(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, cout, n_rows, off_d, off_h, off_w, tap_mask, ys,
                               (cudaStream_t)stream, "conv3d_s1_fwd_ex");
 }
@@ -1985,100 +1810,101 @@ extern "C" int mvsb200_conv3d_s1_wgrad_ex(const void* x, const void* gy, float* 
     const int nco_max = Cin == 64 ? 16 : 32;
     const int nco = cout < nco_max ? cout : nco_max;
     for (int co0 = 0; co0 < cout; co0 += nco) {
-        int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_WG(CI, NC) rc = launch_wgrad<CI, NC>(x, gy, gw, B, Di, Hi, Wi, Do, Ho, Wo, cout, co0, off_d, off_h, off_w, st, 1, 0, 0, 0, kd_mask, \
-                                                 nullptr, 1, nullptr, nullptr, cin_real)
-        if (Cin == 16 && nco == 8) MVS_WG(16, 8);
-        else if (Cin == 16 && nco == 16) MVS_WG(16, 16);
-        else if (Cin == 16 && nco == 32) MVS_WG(16, 32);
-        else if (Cin == 32 && nco == 8) MVS_WG(32, 8);
-        else if (Cin == 32 && nco == 16) MVS_WG(32, 16);
-        else if (Cin == 32 && nco == 32) MVS_WG(32, 32);
-        else if (Cin == 64 && nco == 8) MVS_WG(64, 8);
-        else if (Cin == 64 && nco == 16) MVS_WG(64, 16);
-        else if (Cin == 64 && nco == 32) MVS_WG(64, 32);
-        else MVS_FAIL(MVSB200_E_UNSUPPORTED, "conv3d_s1_wgrad: unsupported channels Cin=%d cout=%d", Cin, cout);
-#undef MVS_WG
-        if (rc != MVSB200_OK) return rc;
+        int rc = MVSB200_OK;
+        if (!dispatch(WgradChannels{}, Cin, nco, rc, [&](auto c) {
+                using C = decltype(c);
+                return launch_wgrad<C::k, C::n>(x, gy, gw, B, Di, Hi, Wi, Do, Ho, Wo, cout, co0, off_d, off_h, off_w, st, 1, 0, 0, 0,
+                                                kd_mask, nullptr, 1, nullptr, nullptr, cin_real);
+            }))
+            MVS_FAIL(MVSB200_E_UNSUPPORTED, "conv3d_s1_wgrad: unsupported channels Cin=%d cout=%d", Cin, cout);
+        MVS_TRY(rc);
     }
     return MVSB200_OK;
 }
 
-extern "C" int mvsb200_conv3d_s2_fwd(const void* x, const void* w_packed, void* y, int B, int Dx, int Hx, int Wx, int Cin, int Do,
-                                     int Ho, int Wo, int cout, int y_cs, int n_rows, int pad_d, int pad_h, int pad_w, void* stream) {
-    MVS_REQUIRE(x && w_packed && y, "conv3d_s2_fwd: null pointer");
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "conv3d_s2_fwd: pointers must be 16-byte aligned");
-    MVS_REQUIRE(B >= 1 && Dx >= 1 && Hx >= 2 && Wx >= 2 && Do >= 1 && Ho >= 1 && Wo >= 1, "conv3d_s2_fwd: bad shape");
-    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 128, "conv3d_s2_fwd: cout %d / n_rows %d", cout, n_rows);
-    MVS_REQUIRE(y_cs >= cout && y_cs % 8 == 0, "conv3d_s2_fwd: output channel stride %d", y_cs);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "conv3d_s2_fwd: pad must be 1 or 2 per axis");
-    cudaStream_t st = (cudaStream_t)stream;
+// the stride-2 forward in launches of up to 64 filter rows.  stats: null, or the workspace of mvsb200_conv3d_s2_fwd_stats,
+// whose rows the launches' epilogues fill; the largest grid of the launches is then raised into *n_blocks.
+static int conv3d_s2_fwd_rows(const void* x, const void* w_packed, void* y, int B, int Dx, int Hx, int Wx, int Cin, int Do, int Ho,
+                              int Wo, int cout, int y_cs, int n_rows, int pad_d, int pad_h, int pad_w, float* stats, int* n_blocks,
+                              cudaStream_t st) {
+    const char* name = "conv3d_s2_fwd";
+    MVS_TRY(check_pointers(name, {x, w_packed, y}));
+    MVS_REQUIRE(B >= 1 && Dx >= 1 && Hx >= 2 && Wx >= 2 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
+    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 128, "%s: cout %d / n_rows %d", name, cout,
+                n_rows);
+    MVS_REQUIRE(y_cs >= cout && y_cs % 8 == 0, "%s: output channel stride %d", name, y_cs);
+    MVS_TRY(check_pads(name, pad_d, pad_h, pad_w));
     // filter rows per launch: up to 64 (27 x 64 x Cin taps resident in shared memory), then 48 / 32 / 16
     for (int row0 = 0; row0 < n_rows && row0 < cout;) {
         const int left = n_rows - row0;
         const int nmax = Cin == 64 ? 32 : 64;
         const int nout = left >= nmax ? nmax : left;
         const int c_here = cout - row0 < nout ? cout - row0 : nout;
-        int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_S2(CI, NO) rc = launch_conv_s2<CI, NO>(x, w_packed, y, B, Dx, Hx, Wx, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, pad_d, pad_h, pad_w, st)
-        if (Cin == 8 && nout == 16) rc = launch_conv_s2<16, 16>(x, w_packed, y, B, Dx, Hx, Wx, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, pad_d, pad_h, pad_w, st, 8);
-        else if (Cin == 8 && nout == 32) rc = launch_conv_s2<16, 32>(x, w_packed, y, B, Dx, Hx, Wx, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, pad_d, pad_h, pad_w, st, 8);
-        else if (Cin == 16 && nout == 16) MVS_S2(16, 16);
-        else if (Cin == 16 && nout == 32) MVS_S2(16, 32);
-        else if (Cin == 16 && nout == 48) MVS_S2(16, 48);
-        else if (Cin == 16 && nout == 64) MVS_S2(16, 64);
-        else if (Cin == 32 && nout == 16) MVS_S2(32, 16);
-        else if (Cin == 32 && nout == 32) MVS_S2(32, 32);
-        else if (Cin == 32 && nout == 48) MVS_S2(32, 48);
-        else if (Cin == 32 && nout == 64) MVS_S2(32, 64);
-        else if (Cin == 64 && nout == 16) MVS_S2(64, 16);
-        else if (Cin == 64 && nout == 32) MVS_S2(64, 32);
-        else MVS_FAIL(MVSB200_E_UNSUPPORTED, "conv3d_s2_fwd: unsupported channels Cin=%d rows=%d", Cin, nout);
-#undef MVS_S2
-        if (rc != MVSB200_OK) return rc;
+        int rc = MVSB200_OK;
+        if (!dispatch(S2Channels{}, Cin, nout, rc, [&](auto c) {
+                using C = decltype(c);
+                return launch_conv_s2<C::k, C::n>(x, w_packed, y, B, Dx, Hx, Wx, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, pad_d,
+                                                  pad_h, pad_w, st, Cin, stats, cout, n_blocks);
+            }))
+            MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d rows=%d", name, Cin, nout);
+        MVS_TRY(rc);
         row0 += nout;
     }
     return MVSB200_OK;
 }
 
-/* 2D convolution 3x3 / padding 1 of N maps stacked as channel-last rows [N, H, W, Cin] -> [N, H, W, y_cs] (SURVEY §8 rows f1 / f2;
- * scripts/model.py:22-65, :129-152): conv3d_s1_kdn_kernel in its planar mode.  w_packed is the kdn operand [9 (kh,kw)][3][n_rows][Cin]
- * of which only the middle row block of every in-plane tap is read. */
-extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
-                                         int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
-                                         void* stream);
-extern "C" int mvsb200_conv2d_rows_fwd(const void* x, const void* w_packed, void* y, int N, int H, int W, int Cin, int cout, int y_cs,
-                                       int n_rows, void* stream) {
-    g_kdn_planar = 1;
-    const int rc = mvsb200_conv3d_s1_fwd_kdn(x, w_packed, y, 1, N, H, W, Cin, N, H, W, cout, y_cs, n_rows, 0, -1, -1, stream);
-    g_kdn_planar = 0;
-    return rc;
+extern "C" int mvsb200_conv3d_s2_fwd(const void* x, const void* w_packed, void* y, int B, int Dx, int Hx, int Wx, int Cin, int Do,
+                                     int Ho, int Wo, int cout, int y_cs, int n_rows, int pad_d, int pad_h, int pad_w, void* stream) {
+    return conv3d_s2_fwd_rows(x, w_packed, y, B, Dx, Hx, Wx, Cin, Do, Ho, Wo, cout, y_cs, n_rows, pad_d, pad_h, pad_w, nullptr, nullptr,
+                              (cudaStream_t)stream);
 }
 
 /* mvsb200_conv3d_s2_fwd that also leaves sums[2][cout] = (sum, sum of squares) of its outputs per channel, accumulated in the
  * kernels' epilogues (fp32 accumulators) and combined in fixed order: the box BatchNorm that follows needs no statistics pass.
  * workspace: at least (SM count) * 2 * cout floats. */
-extern "C" int mvsb200_conv3d_s2_fwd(const void* x, const void* w_packed, void* y, int B, int Dx, int Hx, int Wx, int Cin, int Do,
-                                     int Ho, int Wo, int cout, int y_cs, int n_rows, int pad_d, int pad_h, int pad_w, void* stream);
 extern "C" int mvsb200_conv3d_s2_fwd_stats(const void* x, const void* w_packed, void* y, int B, int Dx, int Hx, int Wx, int Cin, int Do,
                                            int Ho, int Wo, int cout, int y_cs, int n_rows, int pad_d, int pad_h, int pad_w,
                                            float* workspace, float* sums, void* stream) {
     MVS_REQUIRE(workspace && sums, "conv3d_s2_fwd_stats: null statistics buffers");
     cudaStream_t st = (cudaStream_t)stream;
-    int sms = 148;
-    {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-    }
-    MVS_CUDA(cudaMemsetAsync(workspace, 0, (size_t)sms * 2 * cout * sizeof(float), st));      // launches may differ in grid size
-    g_s2_stats = workspace; g_s2_stats_cs = cout; g_s2_stats_blocks = 0;
-    const int rc = mvsb200_conv3d_s2_fwd(x, w_packed, y, B, Dx, Hx, Wx, Cin, Do, Ho, Wo, cout, y_cs, n_rows, pad_d, pad_h, pad_w, stream);
-    const int n_blocks = g_s2_stats_blocks;
-    g_s2_stats = nullptr; g_s2_stats_cs = 0; g_s2_stats_blocks = 0;
-    if (rc != MVSB200_OK) return rc;
+    MVS_CUDA(cudaMemsetAsync(workspace, 0, (size_t)sm_count() * 2 * cout * sizeof(float), st));      // launches may differ in grid size
+    int n_blocks = 0;
+    MVS_TRY(conv3d_s2_fwd_rows(x, w_packed, y, B, Dx, Hx, Wx, Cin, Do, Ho, Wo, cout, y_cs, n_rows, pad_d, pad_h, pad_w, workspace,
+                               &n_blocks, st));
     s2_stats_finalize_kernel<<<(2 * cout + 127) / 128, 128, 0, st>>>(workspace, n_blocks, cout, sums);
     MVS_CHECK_LAUNCH("s2_stats_finalize");
     return MVSB200_OK;
+}
+
+// one body for mvsb200_deconv3d_s2_fwd(_stats) (EPI = false: win, scale, shift and add null) and mvsb200_deconv3d_s2_fwd_affine
+// (EPI = true, stats null; its caller has checked win, scale and shift for null)
+template <bool EPI>
+static int deconv3d_s2_fwd_body(const char* name, const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
+                                int Do, int Ho, int Wo, int cout, int n_rows, int pad_d, int pad_h, int pad_w,
+                                const int64_t* y_strides4, float* stats, int* n_blocks_host, const int* win, const float* scale,
+                                const float* shift, const void* add, void* stream) {
+    MVS_TRY(check_pointers(name, {x, w_packed, y}, {y_strides4}));
+    MVS_REQUIRE(add == nullptr || aligned16(add), "%s: pointers must be 16-byte aligned", name);
+    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
+    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && (n_rows == 16 || n_rows == 32),
+                "%s: cout must be a multiple of 8 and n_rows 16 or 32 (cout=%d n_rows=%d)", name, cout, n_rows);
+    MVS_TRY(check_pads(name, pad_d, pad_h, pad_w));
+    if (EPI) {
+        const int ext[3] = {Do, Ho, Wo};
+        for (int a = 0; a < 3; ++a)
+            MVS_REQUIRE(win[a] >= 0 && win[3 + a] >= 1 && win[a] + win[3 + a] <= ext[a],
+                        "%s: window [%d, %d) outside the canvas extent %d (axis %d)", name, win[a], win[a] + win[3 + a], ext[a], a);
+    }
+    long long ys[4];
+    MVS_TRY(copy_strides(name, y_strides4, ys));
+    int rc = MVSB200_OK;
+    if (!dispatch(ConvChannels{}, Cin, n_rows, rc, [&](auto c) {
+            using C = decltype(c);
+            return launch_deconv_s2<C::k, C::n, EPI>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, n_rows, pad_d, pad_h, pad_w, ys,
+                                                     (cudaStream_t)stream, stats, n_blocks_host, win, scale, shift, add);
+        }))
+        MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
+    return rc;
 }
 
 /* stats (may be NULL): [n_blocks][2][cout] fp32 per-CTA sums of the stored values and of their squares over the written canvas,
@@ -2087,26 +1913,8 @@ extern "C" int mvsb200_conv3d_s2_fwd_stats(const void* x, const void* w_packed, 
 extern "C" int mvsb200_deconv3d_s2_fwd_stats(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
                                              int Do, int Ho, int Wo, int cout, int n_rows, int pad_d, int pad_h, int pad_w,
                                              const int64_t* y_strides4, float* stats, int* n_blocks_host, void* stream) {
-    MVS_REQUIRE(x && w_packed && y && y_strides4, "deconv3d_s2_fwd: null pointer");
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "deconv3d_s2_fwd: pointers must be 16-byte aligned");
-    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "deconv3d_s2_fwd: bad shape");
-    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && (n_rows == 16 || n_rows == 32),
-                "deconv3d_s2_fwd: cout must be a multiple of 8 and n_rows 16 or 32 (cout=%d n_rows=%d)", cout, n_rows);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "deconv3d_s2_fwd: pad must be 1 or 2 per axis");
-    const long long ys[4] = {(long long)y_strides4[0], (long long)y_strides4[1], (long long)y_strides4[2], (long long)y_strides4[3]};
-    for (int i = 0; i < 4; ++i) MVS_REQUIRE(ys[i] % 8 == 0, "deconv3d_s2_fwd: output strides must be multiples of 8 elements");
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_DC(CI, NO) rc = launch_deconv_s2<CI, NO>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, n_rows, pad_d, pad_h, pad_w, ys, st, stats, n_blocks_host)
-    if (Cin == 16 && n_rows == 16) MVS_DC(16, 16);
-    else if (Cin == 16 && n_rows == 32) MVS_DC(16, 32);
-    else if (Cin == 32 && n_rows == 16) MVS_DC(32, 16);
-    else if (Cin == 32 && n_rows == 32) MVS_DC(32, 32);
-    else if (Cin == 64 && n_rows == 16) MVS_DC(64, 16);
-    else if (Cin == 64 && n_rows == 32) MVS_DC(64, 32);
-    else MVS_FAIL(MVSB200_E_UNSUPPORTED, "deconv3d_s2_fwd: unsupported channels Cin=%d n_rows=%d", Cin, n_rows);
-#undef MVS_DC
-    return rc;
+    return deconv3d_s2_fwd_body<false>("deconv3d_s2_fwd", x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, n_rows, pad_d, pad_h,
+                                       pad_w, y_strides4, stats, n_blocks_host, nullptr, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int mvsb200_deconv3d_s2_fwd(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
@@ -2123,64 +1931,30 @@ extern "C" int mvsb200_deconv3d_s2_fwd_affine(const void* x, const void* w_packe
                                               const int* window6_host, const int64_t* y_strides4, const float* scale, const float* shift,
                                               const void* add, void* stream) {
     const char* name = "deconv3d_s2_fwd_affine";
-    MVS_REQUIRE(x && w_packed && y && y_strides4 && window6_host && scale && shift, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y) && (add == nullptr || aligned16(add)),
-                "%s: pointers must be 16-byte aligned", name);
-    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
-    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && (n_rows == 16 || n_rows == 32),
-                "%s: cout must be a multiple of 8 and n_rows 16 or 32 (cout=%d n_rows=%d)", name, cout, n_rows);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
-    const int* wn = window6_host;
-    const int ext[3] = {Do, Ho, Wo};
-    for (int a = 0; a < 3; ++a)
-        MVS_REQUIRE(wn[a] >= 0 && wn[3 + a] >= 1 && wn[a] + wn[3 + a] <= ext[a], "%s: window [%d, %d) outside the canvas extent %d (axis %d)",
-                    name, wn[a], wn[a] + wn[3 + a], ext[a], a);
-    const long long ys[4] = {(long long)y_strides4[0], (long long)y_strides4[1], (long long)y_strides4[2], (long long)y_strides4[3]};
-    for (int i = 0; i < 4; ++i) MVS_REQUIRE(ys[i] % 8 == 0, "%s: output strides must be multiples of 8 elements", name);
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_DC(CI, NO) rc = launch_deconv_s2<CI, NO, true>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, n_rows, pad_d, pad_h, pad_w, ys, st, \
-                                                          nullptr, nullptr, wn, scale, shift, add)
-    if (Cin == 16 && n_rows == 16) MVS_DC(16, 16);
-    else if (Cin == 16 && n_rows == 32) MVS_DC(16, 32);
-    else if (Cin == 32 && n_rows == 16) MVS_DC(32, 16);
-    else if (Cin == 32 && n_rows == 32) MVS_DC(32, 32);
-    else if (Cin == 64 && n_rows == 16) MVS_DC(64, 16);
-    else if (Cin == 64 && n_rows == 32) MVS_DC(64, 32);
-    else MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
-#undef MVS_DC
-    return rc;
+    MVS_TRY(check_pointers(name, {}, {window6_host, scale, shift}));
+    return deconv3d_s2_fwd_body<true>(name, x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, n_rows, pad_d, pad_h, pad_w,
+                                      y_strides4, nullptr, nullptr, window6_host, scale, shift, add, stream);
 }
 
 /* Same convolution as mvsb200_conv3d_s1_fwd with the depth tap folded into the MMA N extent (conv3d_s1_kdn_kernel).
- * w_packed: [9 (kh,kw)][3 (kd)][n_rows][Cin] bf16. */
+ * w_packed: [9 (kh,kw)][3 (kd)][n_rows][Cin] bf16.  planar: KdnParams::planar. */
 template <bool AFF>
 static int kdn_dispatch(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin, int Do, int Ho, int Wo,
-                        int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w, void* stream, const char* name,
-                        const float* scale = nullptr, const float* shift = nullptr) {
-    MVS_REQUIRE(x && w_packed && y, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(x) && aligned16(w_packed) && aligned16(y), "%s: pointers must be 16-byte aligned", name);
-    MVS_REQUIRE(B >= 1 && B <= 65535 && Di >= 1 && Hi >= 1 && Wi >= 1 && Do >= 1 && Ho >= 1 && Wo >= 1, "%s: bad shape", name);
-    MVS_REQUIRE(cout >= 8 && cout % 8 == 0 && cout <= n_rows && n_rows % 16 == 0 && n_rows <= 64,
-                "%s: cout must be a multiple of 8 and n_rows a multiple of 16 <= 64 (cout=%d n_rows=%d)", name, cout, n_rows);
-    MVS_REQUIRE(y_cs >= cout && y_cs % 8 == 0, "%s: output channel stride %d", name, y_cs);
+                        int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w, int planar, void* stream, const char* name,
+                        const float* scale, const float* shift) {
+    MVS_TRY(check_s1_fwd(name, x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, cout, y_cs, n_rows));
     cudaStream_t st = (cudaStream_t)stream;
     for (int row0 = 0; row0 < n_rows && row0 < cout; row0 += 32) {
         const int nout = n_rows - row0 < 32 ? n_rows - row0 : 32;
         const int c_here = cout - row0 < nout ? cout - row0 : nout;
-        int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_CONV(CI, NO) rc = launch_conv_kdn<CI, NO, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, CI, scale, shift)
-        if (Cin == 8 && nout == 16) rc = launch_conv_kdn<16, 16, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8, scale, shift);
-        else if (Cin == 8 && nout == 32) rc = launch_conv_kdn<16, 32, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d, off_h, off_w, st, 8, scale, shift);
-        else if (Cin == 16 && nout == 16) MVS_CONV(16, 16);
-        else if (Cin == 16 && nout == 32) MVS_CONV(16, 32);
-        else if (Cin == 32 && nout == 16) MVS_CONV(32, 16);
-        else if (Cin == 32 && nout == 32) MVS_CONV(32, 32);
-        else if (Cin == 64 && nout == 16) MVS_CONV(64, 16);
-        else if (Cin == 64 && nout == 32) MVS_CONV(64, 32);
-        else MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
-#undef MVS_CONV
-        if (rc != MVSB200_OK) return rc;
+        int rc = MVSB200_OK;
+        if (!dispatch(KdnChannels{}, Cin, nout, rc, [&](auto c) {
+                using C = decltype(c);
+                return launch_conv_kdn<C::k, C::n, AFF>(x, w_packed, y, B, Di, Hi, Wi, Do, Ho, Wo, c_here, y_cs, row0, n_rows, row0, off_d,
+                                                        off_h, off_w, planar, st, Cin, scale, shift);
+            }))
+            MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels Cin=%d n_rows=%d", name, Cin, n_rows);
+        MVS_TRY(rc);
     }
     return MVSB200_OK;
 }
@@ -2188,8 +1962,17 @@ static int kdn_dispatch(const void* x, const void* w_packed, void* y, int B, int
 extern "C" int mvsb200_conv3d_s1_fwd_kdn(const void* x, const void* w_packed, void* y, int B, int Di, int Hi, int Wi, int Cin,
                                          int Do, int Ho, int Wo, int cout, int y_cs, int n_rows, int off_d, int off_h, int off_w,
                                          void* stream) {
-    return kdn_dispatch<false>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, stream,
-                               "conv3d_s1_fwd_kdn");
+    return kdn_dispatch<false>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, 0, stream,
+                               "conv3d_s1_fwd_kdn", nullptr, nullptr);
+}
+
+/* 2D convolution 3x3 / padding 1 of N maps stacked as channel-last rows [N, H, W, Cin] -> [N, H, W, y_cs] (SURVEY §8 rows f1 / f2;
+ * scripts/model.py:22-65, :129-152): conv3d_s1_kdn_kernel in its planar mode.  w_packed is the kdn operand [9 (kh,kw)][3][n_rows][Cin]
+ * of which only the middle row block of every in-plane tap is read. */
+extern "C" int mvsb200_conv2d_rows_fwd(const void* x, const void* w_packed, void* y, int N, int H, int W, int Cin, int cout, int y_cs,
+                                       int n_rows, void* stream) {
+    return kdn_dispatch<false>(x, w_packed, y, 1, N, H, W, Cin, N, H, W, cout, y_cs, n_rows, 0, -1, -1, 1, stream, "conv3d_s1_fwd_kdn",
+                               nullptr, nullptr);
 }
 
 /* mvsb200_conv3d_s1_fwd_kdn (planar = 0) or mvsb200_conv2d_rows_fwd (planar = 1, B = 1, Di = Do = maps) with eval-mode BatchNorm +
@@ -2200,11 +1983,8 @@ extern "C" int mvsb200_conv3d_s1_fwd_kdn_affine(const void* x, const void* w_pac
     const char* name = "conv3d_s1_fwd_kdn_affine";
     MVS_REQUIRE(scale && shift, "%s: null scale / shift", name);
     MVS_REQUIRE(planar == 0 || (planar == 1 && B == 1 && Di == Do && off_d == 0), "%s: planar mode takes B = 1, Di = Do, off_d = 0", name);
-    g_kdn_planar = planar;
-    const int rc = kdn_dispatch<true>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, stream, name,
-                                      scale, shift);
-    g_kdn_planar = 0;
-    return rc;
+    return kdn_dispatch<true>(x, w_packed, y, B, Di, Hi, Wi, Cin, Do, Ho, Wo, cout, y_cs, n_rows, off_d, off_h, off_w, planar, stream, name,
+                              scale, shift);
 }
 
 /* Weight gradient of the STRIDE-2 layers on the same kernel:  gw[k][cb][cs] = sum_o big(2o - pad + k)[cb] * small(o)[cs]
@@ -2216,12 +1996,11 @@ extern "C" int mvsb200_conv3d_s1_fwd_kdn_affine(const void* x, const void* w_pac
 extern "C" int mvsb200_conv3d_s2_wgrad(const void* big, const void* small, float* gw, int B, int Db, int Hb, int Wb, int Cb,
                                        int Ds, int Hs, int Ws, int Cs, int pad_d, int pad_h, int pad_w, void* stream) {
     const char* name = "conv3d_s2_wgrad";
-    MVS_REQUIRE(big && small && gw, "%s: null pointer", name);
-    MVS_REQUIRE(aligned16(big) && aligned16(small) && aligned16(gw), "%s: pointers must be 16-byte aligned", name);
+    MVS_TRY(check_pointers(name, {big, small, gw}));
     MVS_REQUIRE(B >= 1 && Db >= 1 && Hb >= 1 && Wb >= 1 && Ds >= 1 && Hs >= 1 && Ws >= 1, "%s: bad shape", name);
     MVS_REQUIRE(Cb == 16 || Cb == 32 || Cb == 64, "%s: the strided operand must have 16, 32 or 64 channels (got %d)", name, Cb);
     MVS_REQUIRE(Cs >= 8 && Cs % 8 == 0, "%s: the dense operand needs a multiple of 8 channels (got %d)", name, Cs);
-    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
+    MVS_TRY(check_pads(name, pad_d, pad_h, pad_w));
     cudaStream_t st = (cudaStream_t)stream;
     MVS_CUDA(cudaMemsetAsync(gw, 0, (size_t)27 * Cb * Cs * sizeof(float), st));
     const int pads[3] = {pad_d, pad_h, pad_w};
@@ -2260,19 +2039,14 @@ extern "C" int mvsb200_conv3d_s2_wgrad(const void* big, const void* small, float
         for (int co0 = 0; co0 < Cs;) {
             const int left = Cs - co0;
             const int nco = left >= nco_max ? nco_max : (left >= 16 ? 16 : 8);
-            int rc = MVSB200_E_UNSUPPORTED;
-#define MVS_WG(CI, NC) rc = launch_wgrad<CI, NC>(base, small, gw, B, sub[0], sub[1], sub[2], Ds, Hs, Ws, Cs, co0, -1, -1, -1, st, 2, Db, Hb, Wb, kd_mask, tap_map)
-            if (Cb == 16 && nco == 8) MVS_WG(16, 8);
-            else if (Cb == 16 && nco == 16) MVS_WG(16, 16);
-            else if (Cb == 16 && nco == 32) MVS_WG(16, 32);
-            else if (Cb == 32 && nco == 8) MVS_WG(32, 8);
-            else if (Cb == 32 && nco == 16) MVS_WG(32, 16);
-            else if (Cb == 32 && nco == 32) MVS_WG(32, 32);
-            else if (Cb == 64 && nco == 8) MVS_WG(64, 8);
-            else if (Cb == 64 && nco == 16) MVS_WG(64, 16);
-            else MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels %d / %d", name, Cb, nco);
-#undef MVS_WG
-            if (rc != MVSB200_OK) return rc;
+            int rc = MVSB200_OK;
+            if (!dispatch(WgradChannels{}, Cb, nco, rc, [&](auto c) {
+                    using C = decltype(c);
+                    return launch_wgrad<C::k, C::n>(base, small, gw, B, sub[0], sub[1], sub[2], Ds, Hs, Ws, Cs, co0, -1, -1, -1, st, 2, Db,
+                                                    Hb, Wb, kd_mask, tap_map);
+                }))
+                MVS_FAIL(MVSB200_E_UNSUPPORTED, "%s: unsupported channels %d / %d", name, Cb, nco);
+            MVS_TRY(rc);
             co0 += nco;
         }
     }

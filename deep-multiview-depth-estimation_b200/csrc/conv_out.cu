@@ -455,11 +455,7 @@ extern "C" int mvsb200_conv_out_wgrad(const void* z, const float* glogits, float
         // taken from the device's SM count.  One CTA per SM would leave half of every SM to the streaming kernels the side
         // stream's weight gradient runs beside (mvs_b200/ops.py, wgrad_fork), but measured slower in the cfg2 step: 15.97
         // against 15.57 ms (profiles/r07_wgrad_overlap.md)
-        int sms = 148;
-        {
-            int dev = 0, n = 0;
-            if (cudaGetDevice(&dev) == cudaSuccess && cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) sms = n;
-        }
+        const int sms = sm_count();
         const long cap = (long)kWgMarchCtasPerSm * sms < kWgBlocks ? (long)kWgMarchCtasPerSm * sms : kWgBlocks;
         const int grid = (int)(items < cap ? items : cap);
         conv_out_wgrad_march_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>((const uint32_t*)z, glogits, workspace, B, D, h, w, tiles_x,

@@ -1,8 +1,9 @@
-// tcgen05 / TMA / mbarrier PTX wrappers, UMMA shared-memory descriptors and the tensor-map encoder shared by the tensor-core
-// convolution kernels of libmvs_b200.so (conv3d_tc.cu, conv3d_s2_bwd.cu).  sm_100a only.
+// tcgen05 / TMA / mbarrier PTX wrappers, UMMA shared-memory descriptors, the tensor-map encoder and the host-side launch
+// helpers shared by the tensor-core convolution kernels of libmvs_b200.so (conv3d_tc.cu, conv3d_s2_bwd.cu).  sm_100a only.
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
+#include <initializer_list>
 
 namespace {
 
@@ -148,8 +149,83 @@ EncodeTiledFn encode_fn() {
     return fn;
 }
 
+// swizzle of a box whose rows are rowb bytes (one swizzle span); 16-byte rows are not swizzled
 CUtensorMapSwizzle swizzle_for(int rowb) {
-    return rowb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (rowb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+    return rowb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                       : (rowb == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : (rowb == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE));
+}
+
+// bf16 tensor map of `rank` dims (innermost first), rank - 1 byte strides and a box in elements; L2 128-byte promotion,
+// elements outside the tensor read as zeros.  Errors name the launcher and the operand: `what`, followed by `index` if it
+// is not negative.
+int encode_tiled(CUtensorMap* map, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
+                 const cuuint32_t* box, CUtensorMapSwizzle swizzle, const char* name, const char* what, int index = -1) {
+    EncodeTiledFn enc = encode_fn();
+    MVS_REQUIRE(enc != nullptr, "%s: cuTensorMapEncodeTiled is not available from the driver", name);
+    const cuuint32_t es[5] = {1, 1, 1, 1, 1};
+    const CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, es,
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS && index >= 0) MVS_FAIL(MVSB200_E_BADARG, "%s: cuTensorMapEncodeTiled(%s %d) failed (%d)", name, what, index, (int)r);
+    MVS_REQUIRE(r == CUDA_SUCCESS, "%s: cuTensorMapEncodeTiled(%s) failed (%d)", name, what, (int)r);
+    return MVSB200_OK;
+}
+
+// dense channel-last volume [B][D][H][W][C] read in boxes of box_c channels x box_w voxels x box_h lines of one plane (a box
+// wider than C reads the missing channels as zeros)
+int encode_volume(CUtensorMap* map, const void* base, int C, int box_c, int W, int H, int D, int B, int box_w, int box_h,
+                  const char* name, const char* what, int index = -1) {
+    const cuuint64_t row = (cuuint64_t)C * 2;
+    const cuuint64_t dims[5] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)D, (cuuint64_t)B};
+    const cuuint64_t strides[4] = {row, row * W, row * W * H, row * W * H * D};
+    const cuuint32_t box[5] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_h, 1, 1};
+    return encode_tiled(map, base, 5, dims, strides, box, swizzle_for(2 * box_c), name, what, index);
+}
+
+// packed filter: `rows` rows of C channels, read box_rows rows at a time
+int encode_filter(CUtensorMap* map, const void* base, int C, int rows, int box_rows, const char* name, const char* what,
+                  int index = -1) {
+    const cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)C * 2};
+    const cuuint32_t box[2] = {(cuuint32_t)C, (cuuint32_t)box_rows};
+    return encode_tiled(map, base, 2, dims, strides, box, swizzle_for(2 * C), name, what, index);
+}
+
+// Split `extent` planes (or lines) into runs for persistent CTAs: `walkers` CTAs take the tiles * runs * B items in turn and
+// an item costs its run length + `overhead` (halo planes, pipeline fill).  Picks the run count with the least
+// (items per walker) x (cost per item); a run count that would leave a run empty is skipped.
+struct Runs { int nchunks, chunk; };
+Runs choose_runs(long tiles, int B, int extent, long walkers, int overhead) {
+    long best_cost = -1;
+    int best = 1;
+    for (int nc = 1; nc <= extent; ++nc) {
+        const int dc = (extent + nc - 1) / nc;
+        if ((long)(nc - 1) * dc >= extent) continue;
+        const long items = tiles * nc * B;
+        const long cost = ((items + walkers - 1) / walkers) * (dc + overhead);
+        if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = nc; }
+    }
+    return Runs{best, (extent + best - 1) / best};
+}
+
+// argument checks shared by the convolution entry points; `name` starts the message.  Pointers in `aligned` must be
+// non-null and 16-byte aligned, those in `present` non-null.
+int check_pointers(const char* name, std::initializer_list<const void*> aligned, std::initializer_list<const void*> present = {}) {
+    for (const void* p : aligned) MVS_REQUIRE(p, "%s: null pointer", name);
+    for (const void* p : present) MVS_REQUIRE(p, "%s: null pointer", name);
+    for (const void* p : aligned) MVS_REQUIRE(::mvsb200::aligned16(p), "%s: pointers must be 16-byte aligned", name);
+    return MVSB200_OK;
+}
+int check_pads(const char* name, int pad_d, int pad_h, int pad_w) {
+    MVS_REQUIRE(pad_d >= 1 && pad_d <= 2 && pad_h >= 1 && pad_h <= 2 && pad_w >= 1 && pad_w <= 2, "%s: pad must be 1 or 2 per axis", name);
+    return MVSB200_OK;
+}
+// output voxel-row strides (b, d, h, w) in elements, each a multiple of 8
+int copy_strides(const char* name, const int64_t* s, long long ys[4]) {
+    for (int i = 0; i < 4; ++i) {
+        ys[i] = (long long)s[i];
+        MVS_REQUIRE(ys[i] % 8 == 0, "%s: output strides must be multiples of 8 elements", name);
+    }
+    return MVSB200_OK;
 }
 
 // 32-byte global loads / stores (sm_100: ld/st.global.v8.b32): one instruction per 16-channel bf16 piece of a voxel row
